@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W                       # our arm
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                                # CPU arm (C oracle port)
+    python bench.py ... --dump-outputs DIR                              # also write the last step's Gt values
 
 A "step" is one pass of the hot path (Miller loop + final exponentiation) over one batch of
 2^LOG2 synthetic (G1,G2) pairs per GPU (weak scaling).  `value` times the kernels with inputs
@@ -44,6 +45,9 @@ MACS_PRODUCT_PAIR = (FP_MULS_MILLER + 3 * FP_MULS_MILLER_EXTRA_PAIR) * MACS_PER_
 IO_BYTES_PER_PAIRING = 288 + 576
 NOMINAL_WIDE_PEAK = 148 * 4 * 8 * 1.965e9     # one IMAD.WIDE per 4 cycles per scheduler: 148 SM x 4 x 8 lanes x max clock
 EXECUTED_PROFILE = os.path.join(ROOT, "profiles", "executed_work.json")
+# --dump-outputs: at most 2^15 Gt values (2^15 x 144 limbs x 8 bytes = 37.7 MB), rows above that drawn with a fixed seed
+DUMP_ROWS = 1 << 15
+DUMP_SEED = 0xD0D0
 
 
 def hbm_peak():
@@ -86,7 +90,15 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the sub-records of the other BASELINE configs")
     ap.add_argument("--config5-log2", type=int, default=24, help="total pairings of the config5 sub-record (N > 1)")
     ap.add_argument("--ref-seconds", type=float, default=None, help="--impl reference: CPU seconds per step (default: bounded by the step count)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the Gt values of the last step (rank 0's batch) to DIR/gt.npy: float64 (k, 144), "
+                         "each Fp12 as 144 little-endian 32-bit limbs; batches above 2^15 pairings are sampled with a fixed seed")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ CPU arm
@@ -288,6 +300,8 @@ def run_ours(args):
     launches = eng.launch_count - launches0
     clocks = sampler.stop() if sampler else None
     assert int(err.item()) == 0, "non-canonical synthetic input?"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)        # before the records below reuse `out`
     max_ms = sharding.max_over_ranks(total_ms, world, dev)
     value = sharding.whole_job_rate(n, args.steps, world, max_ms)
 
@@ -311,30 +325,28 @@ def run_ours(args):
 
     e2e_step()                      # warm-up (allocates the pipeline buffers)
     barrier()
-    e2e_steps = max(1, args.steps)
     t0 = time.perf_counter()
-    for _ in range(e2e_steps):
+    for _ in range(args.steps):
         e2e_step()
     barrier()
     e2e_dt = time.perf_counter() - t0
-    e2e_value = sharding.whole_job_rate(e2e_n, e2e_steps, world, 1e3 * sharding.max_over_ranks(e2e_dt, world, dev))
+    e2e_value = sharding.whole_job_rate(e2e_n, args.steps, world, 1e3 * sharding.max_over_ranks(e2e_dt, world, dev))
     # the e2e result must equal the device-resident result (same inputs)
     same = bool(torch.equal(h_out[:4096], out[:4096].cpu()))
     del h_g1, h_g2, h_out, n_g1, n_g2, n_out
 
-    sub_steps = max(1, min(args.steps, 5))
     extra_launches0 = eng.launch_count
     configs, product, config5, strong = None, None, None, None
     if not args.no_configs:
-        product = bench_product(eng, z, sharding, torch, dist, world, rank, dev, st, n, SEED, g1, g2, out, err, sub_steps, barrier)
+        product = bench_product(eng, z, sharding, torch, dist, world, rank, dev, st, n, SEED, g1, g2, out, err, args.steps, barrier)
         if world == 1:
-            configs = bench_configs(eng, z, torch, np, dev, st, n, g1, g2, out, err, peak, sub_steps, timed_ms)
+            configs = bench_configs(eng, z, torch, np, dev, st, n, g1, g2, out, err, peak, args.steps, timed_ms)
         else:
             del g1, g2, i1, i2, out
             torch.cuda.empty_cache()
             config5 = bench_sliced(eng, z, sharding, torch, dist, world, rank, dev, st, 1 << args.config5_log2, 0xC5C5, 1, barrier,
                                    with_product=True)
-            strong = bench_sliced(eng, z, sharding, torch, dist, world, rank, dev, st, 1 << args.log2_batch, SEED, sub_steps, barrier,
+            strong = bench_sliced(eng, z, sharding, torch, dist, world, rank, dev, st, 1 << args.log2_batch, SEED, args.steps, barrier,
                                   with_product=False)
             strong["single_gpu_reference"] = "value of the N=1 line of the same sweep (same 2^%d pairings on one GPU)" % args.log2_batch
 
@@ -377,7 +389,7 @@ def run_ours(args):
                                  "achieved_gbs": pairs_per_s_kernel * IO_BYTES_PER_PAIRING / 1e9, "peak_gbs": hbm_peak(),
                                  "note": "HBM is three orders of magnitude away from binding (SURVEY 8d)"}},
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": e2e_n * 288, "d2h_bytes_per_step": e2e_n * 576,
-                    "steps": e2e_steps, "matches_device_path": same},
+                    "steps": args.steps, "matches_device_path": same},
             "gpu_launches": launches,
             "gpu_launches_subrecords": eng.launch_count - extra_launches0,
             "clocks": clocks,
@@ -397,6 +409,26 @@ def run_ours(args):
     eng.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_rows(n: int):
+    """Rows of an n-pairing batch that --dump-outputs writes: all of them up to DUMP_ROWS, else DUMP_ROWS rows drawn
+    without replacement by a fixed seed, in increasing order, so that every build dumps the same rows."""
+    import numpy as np
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+
+
+def dump_outputs(path, out):
+    """DIR/gt.npy: the rows dump_rows() picks from `out` (the (n, 72) int64 Gt tensor of the timed path), each Fp12 as
+    144 little-endian 32-bit limbs in float64, which holds them exactly."""
+    import numpy as np
+    import torch
+    rows = torch.from_numpy(dump_rows(out.shape[0])).to(out.device)
+    gt = out.index_select(0, rows).cpu().numpy().view("<u4").astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "gt.npy"), gt)
 
 
 def _rate_record(units, ms, unit, macs_per_unit=None, peak=None, **extra):

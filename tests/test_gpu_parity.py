@@ -515,7 +515,7 @@ def test_default_stream_ordering_and_device_restored(engine, coracle):
 def _all_devices_engine():
     import zkvm_pairings_b200 as z
     if z.device_count() < 2:
-        pytest.skip("needs >= 2 CUDA devices (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 CUDA devices")
     return z.PairingEngine()
 
 
