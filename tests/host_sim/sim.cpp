@@ -16,6 +16,7 @@
 #include <thread>
 
 #include "../../zkvm_pairings_b200/csrc/ops.cuh"
+#include "../device_harness/bodies.cuh"
 
 namespace zkp {
 thread_local int zkp_sim_par = 0;
@@ -218,6 +219,13 @@ int sim_vertex_check(int what) {
         }
     });
     return bad.load();
+}
+// the bodies of tests/device_harness/bodies.cuh on raw representatives, n elements of BODY_U64 u64: the same
+// computation as the device harness (harness_run), representative for representative
+void sim_body(int body, const uint64_t *in, uint64_t *out, size_t n) {
+    run_pair([&]() {
+        for (size_t i = 0; i < n; i++) body_one(body, in + i * BODY_U64, out + i * BODY_U64, true);
+    });
 }
 // wide MACs executed by both lanes since the last call (boundary conversions included)
 uint64_t sim_take_mac_count() { return g_macs.exchange(0); }

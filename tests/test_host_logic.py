@@ -127,7 +127,8 @@ def sim():
     defs = os.environ.get("ZKP_SIM_DEFINES", "").split()
     so = os.path.join(d, "libzkpair_sim%s.so" % ("_" + re.sub(r"\W+", "_", "".join(defs)) if defs else ""))
     src = [os.path.join(d, "sim.cpp")] + [os.path.join(ROOT, "zkvm_pairings_b200", "csrc", f)
-                                          for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh")]
+                                          for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh")] + \
+        [os.path.join(ROOT, "tests", "device_harness", "bodies.cuh")]
     if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared"] + defs + ["-o", so, src[0]])
     return ctypes.CDLL(so)
@@ -338,7 +339,8 @@ def _sim_variant(defs):
     d = os.path.join(ROOT, "tests", "host_sim")
     so = os.path.join(d, "libzkpair_sim_%s.so" % re.sub(r"\W+", "_", "".join(defs)))
     src = [os.path.join(d, "sim.cpp")] + [os.path.join(ROOT, "zkvm_pairings_b200", "csrc", f)
-                                          for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh")]
+                                          for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh")] + \
+        [os.path.join(ROOT, "tests", "device_harness", "bodies.cuh")]
     if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):
         subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared"] + list(defs) + ["-o", so, src[0]])
     return ctypes.CDLL(so)
