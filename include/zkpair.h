@@ -266,6 +266,50 @@ int32_t zkp_g1_add_batch(zkp_ctx *ctx, const uint64_t *a_xy, const uint8_t *a_in
 int32_t zkp_g2_add_batch(zkp_ctx *ctx, const uint64_t *a_xy, const uint8_t *a_inf, const uint64_t *b_xy, const uint8_t *b_inf,
                          size_t n, uint64_t *out_xy, uint8_t *out_flag);
 
+/* ---- Groth16 verification (one verdict per proof) ----------------------------------------------
+ * Verifying key: alpha in G1; beta, gamma, delta in G2; IC_0 .. IC_l in G1 (l = n_public).  Proof: A in G1,
+ * B in G2, C in G1.  Public inputs: x_1 .. x_l, each an Fr as four little-endian u64 limbs.  A proof is
+ * accepted iff A, B, C are canonical, on their curves and in the prime-order subgroups (G1Affine::is_valid /
+ * G2Affine::is_valid), every x_j < r, and e(A, B) = e(alpha, beta) e(L, gamma) e(C, delta) with
+ * L = IC_0 + sum_j x_j IC_j -- the Groth16 equation, evaluated as the prepared 4-pair check
+ * e(A,B) e(alpha,-beta) e(L,-gamma) e(C,-delta) == 1.  A proof point at infinity is a valid group element.
+ *
+ * Malformed proofs are PER-PROOF rejections (a status byte), not call errors: the call returns ZKP_OK and the
+ * other proofs are unaffected -- unlike the ZKP_ERR_NONCANONICAL convention of the other entry points. */
+#define ZKP_G16_VALID 0       /* all checks pass and the equation holds */
+#define ZKP_G16_INVALID 1     /* well formed, the equation fails */
+#define ZKP_G16_BAD_POINT 2   /* A, B or C has a limb >= p, is off its curve or is not torsion free (precedes 3) */
+#define ZKP_G16_BAD_INPUT 3   /* some x_j >= r */
+#define ZKP_GROTH16_PROOF_U64 48   /* A.x|A.y | B.x.c0|B.x.c1|B.y.c0|B.y.c1 | C.x|C.y */
+/* Public inputs per key.  The key keeps a fixed-base window table per IC_j on every device of its context: 32 x 255
+ * affine points, 765 KiB per input, so 200 MB per device at the bound (and as much again while it is built). */
+#define ZKP_GROTH16_MAX_PUBLIC 256
+
+typedef struct zkp_groth16_vk zkp_groth16_vk;
+
+/* Validates every key point on the GPU and builds the resident key on every device of ctx: the prepared tables of
+ * -beta, -gamma, -delta and the window tables of IC_1 .. IC_l.  ic_g1 holds n_public + 1 points, ic_inf their
+ * is_infinity flags or NULL (an identity IC_j is allowed and contributes nothing).  alpha, beta, gamma, delta have no
+ * infinity flag: the identity is not a valid key point.  A limb >= p gives ZKP_ERR_NONCANONICAL; an off-curve or
+ * non-subgroup point or n_public outside 0 .. ZKP_GROTH16_MAX_PUBLIC gives ZKP_ERR_INVALID_ARG, the message naming
+ * the point.  The key belongs to ctx: other contexts reject it, and it must be destroyed before ctx. */
+int32_t zkp_groth16_vk_create(zkp_ctx *ctx, const uint64_t *alpha_g1, const uint64_t *beta_g2, const uint64_t *gamma_g2,
+                              const uint64_t *delta_g2, const uint64_t *ic_g1, const uint8_t *ic_inf, int32_t n_public,
+                              zkp_groth16_vk **out);
+void zkp_groth16_vk_destroy(zkp_groth16_vk *vk);
+/* n proofs (n x ZKP_GROTH16_PROOF_U64 u64), proof_inf = n x 3 flags (A, B, C) or NULL, public_inputs = n x n_public
+ * x 4 u64 (may be NULL when n_public = 0) -> out_status[i] = ZKP_G16_*.  Sharded over the context's devices in
+ * contiguous slices, double-buffered chunks of at most 2^18 proofs and 64 MB of public inputs. */
+int32_t zkp_groth16_verify_batch(zkp_ctx *ctx, const zkp_groth16_vk *vk, const uint64_t *proofs, const uint8_t *proof_inf,
+                                 const uint64_t *public_inputs, size_t n, uint8_t *out_status);
+/* Bytes of d_scratch zkp_groth16_verify_dev needs for n proofs (the assembled pairs, Gt outputs and is_one). */
+size_t zkp_groth16_scratch_bytes(size_t n);
+/* Device-resident form on device `dev` of the key's context; asynchronous, same buffer layouts; d_scratch
+ * 16-byte aligned. */
+int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *vk, const uint64_t *d_proofs,
+                               const uint8_t *d_proof_inf, const uint64_t *d_public_inputs, size_t n, uint8_t *d_status,
+                               void *d_scratch, void *stream);
+
 /* ---- measurement helpers -------------------------------------------------------------------- */
 
 /* Integer-multiply roofline probe: runs independent IMAD.WIDE.U32 (kind 0), IMAD lo (kind 1) or

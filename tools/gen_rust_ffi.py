@@ -8,6 +8,8 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TYPES = [
     (r"^zkp_ctx \*\*$", "*mut *mut ZkpCtx"), (r"^const zkp_ctx \*$", "*const ZkpCtx"), (r"^zkp_ctx \*$", "*mut ZkpCtx"),
+    (r"^zkp_groth16_vk \*\*$", "*mut *mut ZkpGroth16Vk"), (r"^const zkp_groth16_vk \*$", "*const ZkpGroth16Vk"),
+    (r"^zkp_groth16_vk \*$", "*mut ZkpGroth16Vk"),
     (r"^const uint64_t \*$", "*const u64"), (r"^uint64_t \*$", "*mut u64"), (r"^const uint8_t \*$", "*const u8"),
     (r"^uint8_t \*$", "*mut u8"), (r"^const uint32_t \*$", "*const u32"), (r"^uint32_t \*$", "*mut u32"), (r"^uint32_t$", "u32"), (r"^const void \*$", "*const c_void"),
     (r"^void \*$", "*mut c_void"), (r"^const int \*$", "*const c_int"), (r"^double \*$", "*mut f64"),

@@ -26,6 +26,7 @@
 
 #include "../../include/zkpair.h"
 #include "fe_scratch.cuh"   // ops.cuh + the context-owned helper objects of the final exponentiation
+#include "groth16.cuh"
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -123,6 +124,53 @@ k_group_op(int gop, const uint64_t *__restrict__ pts, const uint8_t *__restrict_
         if (gop <= GOP_G2_CHECK) flag[i] = f;
         if (bad && err) atomicOr(err, 1u);
     }
+}
+
+// ---- Groth16 verification front end (groth16.cuh)
+
+// the verifying key's -beta, -gamma, -delta: negated here, then the prepared line tables of k_g2_prepare
+__global__ void __launch_bounds__(ZKP_TPB, ZKP_MIN_BLOCKS)
+k_g16_neg_prepare(const uint64_t *__restrict__ g2, Fp *__restrict__ out, size_t n) {
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= n) return;
+    bool bad = false;
+    G2A q;
+    load_g2(q, g2 + 24 * i, bad);
+    q.y = fp2_neg(q.y);
+    g2_prepare(q, out + i * (ZKP_LINE_STEPS * 3 * 2) + lane_par());
+}
+
+// one THREAD per (IC_j, window): Fp-level work only, no lane exchange.  ic = IC_0 .. IC_l (canonical);
+// scratch: 2 * 255 Fp per thread
+__global__ void __launch_bounds__(ZKP_TPB)
+k_g16_window_tables(const uint64_t *__restrict__ ic, const uint8_t *__restrict__ ic_inf, int n_public, Fp *__restrict__ tables,
+                    Fp *__restrict__ scratch) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (size_t)n_public * ZKP_G16_WINDOWS) return;
+    int j = (int)(t / ZKP_G16_WINDOWS), w = (int)(t % ZKP_G16_WINDOWS);
+    if (ic_inf[j + 1]) return;
+    Fp *zs = scratch + t * 2 * ZKP_G16_DIGITS;
+    groth16_window_table(ic + 12 * (j + 1), w, tables + (size_t)j * ZKP_G16_TABLE_FP + (size_t)w * ZKP_G16_DIGITS * 2, zs,
+                         zs + ZKP_G16_DIGITS);
+}
+
+__global__ void __launch_bounds__(ZKP_TPB, ZKP_MIN_BLOCKS)
+k_groth16_prepare(G16Key vk, const uint64_t *__restrict__ proofs, const uint8_t *__restrict__ proof_inf, const uint64_t *__restrict__ x,
+                  size_t n, uint64_t *__restrict__ g1, uint8_t *__restrict__ g1inf, uint64_t *__restrict__ g2,
+                  uint8_t *__restrict__ g2inf, uint8_t *__restrict__ status) {
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= n) return;
+    uint8_t s = groth16_prepare_one(vk, proofs + 48 * i, proof_inf ? proof_inf + 3 * i : nullptr, x + (size_t)vk.n_public * 4 * i,
+                                    g1 + 48 * i, g1inf + 4 * i, g2 + 24 * i, g2inf + i);
+    if (lane_par() == 0) status[i] = s;
+}
+
+// the verdict: a front-end rejection stands, otherwise the equation decides
+__global__ void k_groth16_verdict(const uint8_t *__restrict__ is_one, uint8_t *__restrict__ status, size_t n) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint8_t s = status[i];
+    status[i] = s ? s : (is_one[i] ? ZKP_G16_VALID : ZKP_G16_INVALID);
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -387,6 +435,69 @@ static cudaError_t launch_product(zkp_ctx *ctx, const uint64_t *d_in, size_t n, 
     return cudaGetLastError();
 }
 
+// ---- Groth16 verification: resident verifying key and the per-batch launch sequence
+
+static inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+struct G16Dev {   // one device's copy of a verifying key, in one allocation
+    int id = 0;
+    void *mem = nullptr;
+    const Fp *prep = nullptr;   // prepared tables of -beta, -gamma, -delta
+    G16Key key = {};
+};
+struct zkp_groth16_vk {
+    zkp_ctx *ctx = nullptr;
+    int n_public = 0;
+    std::vector<G16Dev> devs;   // one per device of ctx, same order
+};
+
+// proofs per host pipeline chunk: at most 2^18, and at most 64 MB of public inputs (2^21 scalars)
+static size_t g16_chunk(int n_public) {
+    size_t c = n_public > 8 ? ((size_t)ZKP_CHUNK * 8) / (size_t)n_public : (size_t)ZKP_CHUNK;
+    return c ? c : 1;
+}
+
+// scratch of one batch of n proofs: assembled pairs [A, alpha, L, C] x [B], the Gt outputs and is_one
+struct G16Scratch {
+    uint64_t *g1, *g2, *gt;
+    uint8_t *g1inf, *g2inf, *is_one;
+};
+static size_t g16_layout(size_t n, void *base, G16Scratch *s) {
+    const size_t sz[6] = {n * 4 * 96, n * 192, n * 576, n * 4, n, n};
+    size_t off[6], o = 0;
+    for (int i = 0; i < 6; i++) {
+        off[i] = o;
+        o += align256(sz[i]);
+    }
+    if (s) {
+        uint8_t *b = (uint8_t *)base;
+        s->g1 = (uint64_t *)(b + off[0]);
+        s->g2 = (uint64_t *)(b + off[1]);
+        s->gt = (uint64_t *)(b + off[2]);
+        s->g1inf = b + off[3];
+        s->g2inf = b + off[4];
+        s->is_one = b + off[5];
+    }
+    return o;
+}
+
+// front end -> prepared 4-pair check (k = 4, the last kf = 3 pairs from the key's tables) -> verdict
+static cudaError_t launch_groth16(zkp_ctx *ctx, DevState &d, const G16Dev &k, const uint64_t *proofs, const uint8_t *proof_inf,
+                                  const uint64_t *x, size_t n, uint8_t *status, void *scratch, uint32_t *err, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    G16Scratch s;
+    g16_layout(n, scratch, &s);
+    k_groth16_prepare<<<grid_for(n), ZKP_TPB, 0, st>>>(k.key, proofs, proof_inf, x, n, s.g1, s.g1inf, s.g2, s.g2inf, status);
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, s.g2, s.g2inf, n, 4, nullptr, s.gt, s.is_one, err, st, k.prep, nullptr, 3);
+    if (e != cudaSuccess) return e;
+    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
+    ctx->launches++;
+    return cudaGetLastError();
+}
+
 extern "C" {
 
 const char *zkp_last_error(void) { return g_err.c_str(); }
@@ -620,7 +731,7 @@ static void slice_of(size_t n, size_t ndev, size_t d, size_t &lo, size_t &hi) {
 }
 
 struct HostJob {
-    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product
+    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16
     const uint64_t *pts = nullptr, *scalars = nullptr;   // group op inputs (inf in g1inf, outputs in out / flags)
     const uint64_t *tab = nullptr;                       // prepared G2 line tables shared by all checks (kf of them)
     const uint8_t *tabinf = nullptr;
@@ -632,6 +743,7 @@ struct HostJob {
     int k = 1, op = 0;
     int miller_mode = 1;   // mode 64: 1 = SURVEY 9.1 line scaling (the Miller product is returned), 5 = free scaling (only Gt is)
     uint64_t seed = 0, first = 0;
+    const zkp_groth16_vk *vk = nullptr;   // mode 80 = Groth16 verification (proofs in pts, their flags in g1inf, inputs in scalars)
 };
 
 // Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
@@ -650,7 +762,7 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
     CUS(cudaStreamSynchronize(d.stream[0]));
     int na = 0, nb = 0, nr = 0;
     if (j.mode == 16) tower_op_shape(j.op, na, nb, nr);
-    size_t chunk = ZKP_CHUNK;
+    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : ZKP_CHUNK;
     int s = 0;
     cudaStream_t st = nullptr;
     d.pend[0].clear();   // (a job that failed half-way leaves nothing behind for the next one)
@@ -786,6 +898,27 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
                                    (uint64_t *)B[B_OUT].p + 72 * nc4, nullptr, d.d_err, st));
             }
             CUS(launch_product(ctx, (const uint64_t *)B[B_OUT].p, ne, (uint64_t *)B[B_IN].p, (uint64_t *)d.partial.p + 72 * ci, d.d_err, st));
+        } else if (j.mode == 80) {
+            const G16Dev &kd = j.vk->devs[&d - ctx->devs.data()];
+            const size_t np = (size_t)j.vk->n_public;
+            const uint8_t *dpi = nullptr;
+            const uint64_t *dx = nullptr;
+            CUS(B[B_G1].ensure(cn * 384));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(B[B_OUT].ensure(g16_layout(cn, nullptr, nullptr)));
+            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 48, cn * 384));
+            if (j.g1inf) {
+                CUS(B[B_G1INF].ensure(cn * 3));
+                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 3, cn * 3));
+                dpi = (const uint8_t *)B[B_G1INF].p;
+            }
+            if (np) {
+                CUS(B[B_IN].ensure(cn * np * 32));
+                CUS(h2d(B_IN, B[B_IN].p, j.scalars + c0 * np * 4, cn * np * 32));
+                dx = (const uint64_t *)B[B_IN].p;
+            }
+            CUS(launch_groth16(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, dx, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
         } else {
             size_t np = cn * (size_t)j.k, p0 = c0 * (size_t)j.k;
             size_t nq = cn * (size_t)(j.k - j.kf), q0 = c0 * (size_t)(j.k - j.kf);   // per-check G2 points
@@ -1162,6 +1295,137 @@ int32_t zkp_multi_miller_product(zkp_ctx *ctx, const uint64_t *g1, const uint8_t
     if (out_miller_product) CU(cudaMemcpyAsync(out_miller_product, prod, 576, cudaMemcpyDeviceToHost, d0.stream[0]));
     if (out_gt) CU(cudaMemcpyAsync(out_gt, gt, 576, cudaMemcpyDeviceToHost, d0.stream[0]));
     CU(cudaStreamSynchronize(d0.stream[0]));
+    return ZKP_OK;
+}
+
+// ---- Groth16 verification
+static const char *g16_point_error(uint8_t st) { return st == ZKP_POINT_NOT_ON_CURVE ? "is not on the curve" : "is not torsion free"; }
+
+int32_t zkp_groth16_vk_create(zkp_ctx *ctx, const uint64_t *alpha_g1, const uint64_t *beta_g2, const uint64_t *gamma_g2,
+                              const uint64_t *delta_g2, const uint64_t *ic_g1, const uint8_t *ic_inf, int32_t n_public,
+                              zkp_groth16_vk **out) {
+    if (!out) return fail(ZKP_ERR_INVALID_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (!alpha_g1 || !beta_g2 || !gamma_g2 || !delta_g2 || !ic_g1) return fail(ZKP_ERR_INVALID_ARG, "NULL verifying-key point");
+    if (n_public < 0 || n_public > ZKP_GROTH16_MAX_PUBLIC)
+        return fail(ZKP_ERR_INVALID_ARG, "n_public out of range (0 .. ZKP_GROTH16_MAX_PUBLIC)");
+    const size_t nic = (size_t)n_public + 1;
+    // every key point is validated on the GPU: alpha and IC_0 .. IC_l (G1), beta, gamma, delta (G2)
+    std::vector<uint64_t> g1(12 * (nic + 1)), g2(72);
+    std::vector<uint8_t> g1inf(nic + 1, 0), st1(nic + 1), st2(3);
+    memcpy(g1.data(), alpha_g1, 96);
+    memcpy(g1.data() + 12, ic_g1, 96 * nic);
+    if (ic_inf) memcpy(g1inf.data() + 1, ic_inf, nic);
+    memcpy(g2.data(), beta_g2, 192);
+    memcpy(g2.data() + 24, gamma_g2, 192);
+    memcpy(g2.data() + 48, delta_g2, 192);
+    int32_t rc = zkp_g1_check_batch(ctx, g1.data(), g1inf.data(), nic + 1, st1.data());
+    if (rc == ZKP_OK) rc = zkp_g2_check_batch(ctx, g2.data(), nullptr, 3, st2.data());
+    if (rc != ZKP_OK) return rc;
+    if (st1[0]) return fail(ZKP_ERR_INVALID_ARG, std::string("alpha_g1 ") + g16_point_error(st1[0]));
+    static const char *g2names[3] = {"beta_g2", "gamma_g2", "delta_g2"};
+    for (int i = 0; i < 3; i++)
+        if (st2[i]) return fail(ZKP_ERR_INVALID_ARG, std::string(g2names[i]) + " " + g16_point_error(st2[i]));
+    for (size_t j = 0; j < nic; j++)
+        if (st1[j + 1]) return fail(ZKP_ERR_INVALID_ARG, "ic_g1[" + std::to_string(j) + "] " + g16_point_error(st1[j + 1]));
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    zkp_groth16_vk *vk = new zkp_groth16_vk();
+    vk->ctx = ctx;
+    vk->n_public = n_public;
+    vk->devs.resize(ctx->devs.size());
+    const size_t prep_b = align256(3 * (size_t)ZKP_G2_PREPARED_U64 * 8), tab_b = (size_t)n_public * ZKP_G16_TABLE_FP * sizeof(Fp);
+    const size_t tmp_ic = align256(96 * nic), tmp_g2 = align256(192 * 3);
+    const size_t tmp_b = tmp_ic + tmp_g2 + (size_t)n_public * ZKP_G16_WINDOWS * 2 * ZKP_G16_DIGITS * sizeof(Fp);
+    cudaError_t e = cudaSuccess;
+    for (size_t di = 0; di < ctx->devs.size() && e == cudaSuccess; di++) {
+        DevState &d = ctx->devs[di];
+        G16Dev &k = vk->devs[di];
+        k.id = d.id;
+        void *tmp = nullptr;
+        e = cudaSetDevice(d.id);
+        // resident layout: prepared tables | alpha | IC_0 | IC flags | window tables
+        if (e == cudaSuccess) e = cudaMalloc(&k.mem, prep_b + 256 + 256 + align256(nic) + tab_b);
+        if (e == cudaSuccess) e = cudaMalloc(&tmp, tmp_b);
+        if (e == cudaSuccess) {
+            uint8_t *m = (uint8_t *)k.mem, *t = (uint8_t *)tmp;
+            k.prep = (const Fp *)m;
+            k.key.alpha = (const uint64_t *)(m + prep_b);
+            k.key.ic0 = (const uint64_t *)(m + prep_b + 256);
+            k.key.ic_inf = m + prep_b + 512;
+            k.key.tables = (const Fp *)(m + prep_b + 512 + align256(nic));
+            k.key.n_public = n_public;
+            cudaStream_t st = d.stream[0];
+            e = cudaMemcpyAsync((void *)k.key.alpha, alpha_g1, 96, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync((void *)k.key.ic0, ic_g1, 96, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync((void *)k.key.ic_inf, g1inf.data() + 1, nic, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(t, ic_g1, 96 * nic, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(t + tmp_ic, g2.data(), 192 * 3, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) {
+                k_g16_neg_prepare<<<grid_for(3), ZKP_TPB, 0, st>>>((const uint64_t *)(t + tmp_ic), (Fp *)k.prep, 3);
+                ctx->launches++;
+                e = cudaGetLastError();
+            }
+            if (e == cudaSuccess && n_public) {
+                unsigned threads = (unsigned)n_public * ZKP_G16_WINDOWS;
+                k_g16_window_tables<<<(threads + ZKP_TPB - 1) / ZKP_TPB, ZKP_TPB, 0, st>>>(
+                    (const uint64_t *)t, k.key.ic_inf, n_public, (Fp *)k.key.tables, (Fp *)(t + tmp_ic + tmp_g2));
+                ctx->launches++;
+                e = cudaGetLastError();
+            }
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        }
+        if (tmp) cudaFree(tmp);
+    }
+    if (e != cudaSuccess) {
+        std::string msg = std::string("verifying key setup failed: ") + cudaGetErrorString(e);
+        zkp_groth16_vk_destroy(vk);
+        return fail(ZKP_ERR_CUDA, msg);
+    }
+    *out = vk;
+    return ZKP_OK;
+}
+
+void zkp_groth16_vk_destroy(zkp_groth16_vk *vk) {
+    if (!vk) return;
+    DeviceGuard guard;
+    for (G16Dev &k : vk->devs) {
+        if (!k.mem) continue;
+        cudaSetDevice(k.id);
+        cudaFree(k.mem);
+    }
+    delete vk;
+}
+
+size_t zkp_groth16_scratch_bytes(size_t n) { return g16_layout(n, nullptr, nullptr); }
+
+int32_t zkp_groth16_verify_batch(zkp_ctx *ctx, const zkp_groth16_vk *vk, const uint64_t *proofs, const uint8_t *proof_inf,
+                                 const uint64_t *public_inputs, size_t n, uint8_t *out_status) {
+    if (!ctx || !vk) return fail(ZKP_ERR_INVALID_ARG, "ctx or vk is NULL");
+    if (vk->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the verifying key belongs to another context");
+    if (n && (!proofs || !out_status || (vk->n_public && !public_inputs))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 80; j.vk = vk; j.pts = proofs; j.g1inf = proof_inf; j.scalars = public_inputs; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *vk, const uint64_t *d_proofs,
+                               const uint8_t *d_proof_inf, const uint64_t *d_public_inputs, size_t n, uint8_t *d_status,
+                               void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc) return rc;
+    if (!vk) return fail(ZKP_ERR_INVALID_ARG, "vk is NULL");
+    if (vk->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the verifying key belongs to another context");
+    if (n && (!d_proofs || !d_status || !d_scratch || (vk->n_public && !d_public_inputs))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if ((uintptr_t)d_scratch & 15) return fail(ZKP_ERR_INVALID_ARG, "d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
+    CU(launch_groth16(ctx, d, vk->devs[dev], d_proofs, d_proof_inf, d_public_inputs, n, d_status, d_scratch, nullptr, st));
     return ZKP_OK;
 }
 

@@ -10,6 +10,7 @@ No CPU fallback: constructing an engine without libzkpair.so or without a CUDA d
 from __future__ import annotations
 
 import ctypes
+import weakref
 from typing import Optional, Sequence
 
 import numpy as np
@@ -32,6 +33,11 @@ _BINARY = {"add", "sub", "mul"}
 
 MODE_MILLER, MODE_FINAL_EXP, MODE_PAIRING = 1, 2, 3
 MODE_MILLER_FOR_FINAL_EXP = 5   # Miller loop whose output only feeds a final exponentiation (free line scaling, cheaper)
+
+# per-proof verdicts of groth16_verify_batch / groth16_verify_dev (include/zkpair.h ZKP_G16_*)
+G16_VALID, G16_INVALID, G16_BAD_POINT, G16_BAD_INPUT = 0, 1, 2, 3
+GROTH16_PROOF_U64 = 48
+GROTH16_MAX_PUBLIC = 256
 
 
 class ZkpError(RuntimeError):
@@ -75,11 +81,44 @@ def _dptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+class Groth16VerifyingKey:
+    """A verifying key resident on every device of one engine (PairingEngine.groth16_prepare_vk).  It holds a
+    reference to its engine, so the engine's context outlives it; ``close()`` (or leaving a ``with`` block)
+    frees the device memory."""
+
+    def __init__(self, engine: "PairingEngine", handle: ctypes.c_void_p, n_public: int):
+        self.engine, self._vk, self.n_public = engine, handle, n_public
+
+    @property
+    def handle(self):
+        if not self._vk:
+            raise ValueError("the verifying key is closed")
+        return self._vk
+
+    def close(self):
+        if getattr(self, "_vk", None):
+            self.engine._lib.zkp_groth16_vk_destroy(self._vk)
+            self._vk = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
 class PairingEngine:
     """One C-ABI context: a set of CUDA devices with their streams and scratch buffers."""
 
     def __init__(self, devices: Optional[Sequence[int]] = None):
         self._lib = _lib.load()
+        self._vks = weakref.WeakSet()   # verifying keys of this context: freed before the context is
         self._ctx = ctypes.c_void_p()
         if devices is None:
             arr, n = None, 0
@@ -99,6 +138,8 @@ class PairingEngine:
         raise ZkpError(rc, msg)
 
     def close(self):
+        for vk in list(getattr(self, "_vks", ())):
+            vk.close()
         if getattr(self, "_ctx", None):
             self._lib.zkp_ctx_destroy(self._ctx)
             self._ctx = None
@@ -283,6 +324,42 @@ class PairingEngine:
         self._check(self._lib.zkp_multi_pairing_prepared_dev(self._ctx, dev, _dptr(g1), _dptr(g1_inf), _dptr(g2), _dptr(g2_inf), n_checks,
                                                              pairs_per_check, _dptr(d_tables), _dptr(tables_inf), prepared_pairs,
                                                              _dptr(out), _dptr(is_one), _dptr(err), ctypes.c_void_p(stream)))
+
+    # ------------------------------------------------------------------ Groth16 verification
+    def groth16_prepare_vk(self, alpha, beta, gamma, delta, ic, ic_inf=None) -> Groth16VerifyingKey:
+        """Verifying key (alpha (12,), beta/gamma/delta (24,), ic (n_public + 1, 12)) -> a key validated and resident on
+        the GPU.  Raises NonCanonicalError for a limb >= p, ZkpError (INVALID_ARG) for an invalid point."""
+        a = np.ascontiguousarray(alpha, dtype=np.uint64).reshape(12)
+        b, g, d = (np.ascontiguousarray(v, dtype=np.uint64).reshape(24) for v in (beta, gamma, delta))
+        ic = np.ascontiguousarray(ic, dtype=np.uint64).reshape(-1, 12)
+        n_public = ic.shape[0] - 1
+        ii = _np8(ic_inf, ic.shape[0])
+        h = ctypes.c_void_p()
+        self._check(self._lib.zkp_groth16_vk_create(self._ctx, _ptr(a), _ptr(b), _ptr(g), _ptr(d), _ptr(ic), _ptr(ii), n_public,
+                                                    ctypes.byref(h)))
+        vk = Groth16VerifyingKey(self, h, n_public)
+        self._vks.add(vk)
+        return vk
+
+    def groth16_verify_batch(self, vk: Groth16VerifyingKey, proofs, public_inputs, proof_inf=None):
+        """proofs (n, 48) = A | B | C, public_inputs (n, n_public, 4) Fr limbs, proof_inf (n, 3) or None ->
+        uint8 (n,) verdicts G16_*."""
+        pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(-1, GROTH16_PROOF_U64)
+        n = pr.shape[0]
+        x = np.ascontiguousarray(public_inputs, dtype=np.uint64).reshape(n, vk.n_public * 4)
+        pi = None if proof_inf is None else _np8(proof_inf, 3 * n)
+        st = np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_groth16_verify_batch(self._ctx, vk.handle, _ptr(pr), _ptr(pi), _ptr(x), n, _ptr(st)))
+        return st
+
+    def groth16_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_groth16_scratch_bytes(n))
+
+    def groth16_verify_dev(self, vk: Groth16VerifyingKey, d_proofs, d_public_inputs, n: int, d_status, d_scratch, d_proof_inf=None,
+                           stream: int = 0, dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_scratch holds groth16_scratch_bytes(n) bytes."""
+        self._check(self._lib.zkp_groth16_verify_dev(self._ctx, dev, vk.handle, _dptr(d_proofs), _dptr(d_proof_inf), _dptr(d_public_inputs),
+                                                     n, _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ byte (de)serialisation (SURVEY 8f)
     def fp_from_bytes_batch(self, data):

@@ -106,3 +106,61 @@ def groth16_checks(engine, n_checks: int, seed: int = 0x6716, corrupt_every: int
     g2[:, 1:] = fixed[None]
     return {"g1": g1.reshape(-1, 12), "g2": g2.reshape(-1, 24), "g2_var": np.ascontiguousarray(gB), "fixed": fixed,
             "expect_one": ~corrupt, "pairs_per_check": 4, "prepared_pairs": 3}
+
+
+def _fr_matrix(vals) -> np.ndarray:
+    """Python ints (< 2^256) -> (n, 4) little-endian u64 limbs, vectorised over 64-bit slices."""
+    vals = list(vals)
+    m = np.empty((len(vals), 4), dtype=np.uint64)
+    for k in range(4):
+        m[:, k] = np.array([(v >> (64 * k)) & 0xFFFFFFFFFFFFFFFF for v in vals], dtype=np.uint64)
+    return m
+
+
+def groth16_proofs(engine, n: int, n_public: int, seed: int = 0x6716, corrupt_every: int = 100, corrupt_at: int = 7):
+    """Groth16 verifying key, proofs and public inputs with known verdicts, from the trapdoor construction.
+
+    Seeded alpha, beta, gamma, delta and u_0 .. u_l give the key alpha G1, beta G2, gamma G2, delta G2 and
+    IC_j = u_j G1.  Per proof: random a, b and full-width inputs x_j < r, l = u_0 + sum_j x_j u_j and
+    c = (a b - alpha beta - l gamma) / delta mod r; A = a G1, B = b G2, C = c G1 (engine.g1_mul_batch /
+    g2_mul_batch).  The verifier sees only the equation, so these proofs exercise it as a prover's would.  A seeded
+    1 % is corrupted as x_1 + 1 (C + G1 when there is no public input), so the expected verdicts are known without
+    running a pairing.  Returns a dict:
+        alpha (12,), beta / gamma / delta (24,), ic (l + 1, 12)      the verifying key
+        proofs (n, 48) A | B | C, inputs (n, l, 4)                  what the verifier receives
+        l (n, 4) the discrete log of the L the verifier derives    expect (n,) uint8 ZKP_G16_VALID / ZKP_G16_INVALID
+    """
+    import random
+    rng = random.Random(seed)
+    n, lp = int(n), int(n_public)
+    alpha, beta, gamma, delta = (rng.randrange(1, R_ORDER) for _ in range(4))
+    u = [rng.randrange(1, R_ORDER) for _ in range(lp + 1)]
+    g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
+    k1, _ = engine.g1_mul_batch(np.tile(g1gen, (lp + 2, 1)), _fr_matrix([alpha] + u))
+    k2, _ = engine.g2_mul_batch(np.tile(g2gen, (3, 1)), _fr_matrix([beta, gamma, delta]))
+    corrupt = np.zeros(n, dtype=bool)
+    if corrupt_every:
+        corrupt[corrupt_at % corrupt_every::corrupt_every] = True
+    a = [rng.randrange(1, R_ORDER) for _ in range(n)]
+    b = [rng.randrange(1, R_ORDER) for _ in range(n)]
+    x = [[rng.randrange(R_ORDER) for _ in range(lp)] for _ in range(n)]
+    ab_ = alpha * beta
+    dinv = pow(delta, -1, R_ORDER)
+    ls, cs = [], []
+    for i in range(n):
+        l = (u[0] + sum(xj * uj for xj, uj in zip(x[i], u[1:]))) % R_ORDER
+        c = (a[i] * b[i] - ab_ - l * gamma) * dinv % R_ORDER
+        if corrupt[i] and lp:
+            x[i][0] = (x[i][0] + 1) % R_ORDER
+            l = (l + u[1]) % R_ORDER
+        elif corrupt[i]:
+            c = (c + 1) % R_ORDER
+        ls.append(l)
+        cs.append(c)
+    gA, _ = engine.g1_mul_batch(np.tile(g1gen, (n, 1)), _fr_matrix(a))
+    gB, _ = engine.g2_mul_batch(np.tile(g2gen, (n, 1)), _fr_matrix(b))
+    gC, _ = engine.g1_mul_batch(np.tile(g1gen, (n, 1)), _fr_matrix(cs))
+    inputs = _fr_matrix([v for row in x for v in row]).reshape(n, lp, 4)
+    return {"alpha": k1[0], "beta": k2[0], "gamma": k2[1], "delta": k2[2], "ic": k1[1:],
+            "proofs": np.concatenate([gA, gB, gC], axis=1), "inputs": inputs, "l": _fr_matrix(ls),
+            "expect": corrupt.astype(np.uint8)}
