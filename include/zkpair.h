@@ -310,6 +310,40 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
                                const uint8_t *d_proof_inf, const uint64_t *d_public_inputs, size_t n, uint8_t *d_status,
                                void *d_scratch, void *stream);
 
+/* ---- KZG point-evaluation verification (one verdict per proof) ----------------------------------
+ * EIP-4844's verify_kzg_proof(C, z, y, pi) on the library's limb boundary.  Setup: [tau]G2.  Proof: commitment C in
+ * G1, evaluation point z and claimed value y (each an Fr as four little-endian u64 limbs), opening proof pi in G1.
+ * A proof is accepted iff C and pi are canonical, on the curve and torsion free (G1Affine::is_valid), z < r, y < r
+ * and e(C - [y]G1, G2) = e(pi, [tau]G2 - [z]G2), evaluated as the prepared 2-pair check
+ * e(C + [z]pi - [y]G1, G2) e(pi, -[tau]G2) == 1 (G1, G2 the standard generators).  C or pi at infinity is a valid
+ * group element.  As for Groth16, malformed proofs are per-proof rejections and the call returns ZKP_OK. */
+#define ZKP_KZG_VALID 0        /* all checks pass and the equation holds */
+#define ZKP_KZG_INVALID 1      /* well formed, the equation fails */
+#define ZKP_KZG_BAD_POINT 2    /* C or pi has a limb >= p, is off the curve or is not torsion free (precedes 3) */
+#define ZKP_KZG_BAD_SCALAR 3   /* z >= r or y >= r */
+#define ZKP_KZG_PROOF_U64 24   /* C.x|C.y | pi.x|pi.y */
+
+typedef struct zkp_kzg_setup zkp_kzg_setup;
+
+/* Validates [tau]G2 on the GPU and builds the resident setup on every device of ctx: the prepared tables of G2 and
+ * -[tau]G2 and a fixed-base window table of G1 (32 x 255 affine points, 765 KiB).  There is no infinity flag: the
+ * identity is not a valid setup.  A limb >= p gives ZKP_ERR_NONCANONICAL; an off-curve or non-subgroup point gives
+ * ZKP_ERR_INVALID_ARG, the message naming tau_g2.  The setup belongs to ctx: other contexts reject it, and it must be
+ * destroyed before ctx. */
+int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup **out);
+void zkp_kzg_setup_destroy(zkp_kzg_setup *s);
+/* n proofs (n x ZKP_KZG_PROOF_U64 u64), proof_inf = n x 2 flags (C, pi) or NULL, zy = n x 8 u64 (z | y) ->
+ * out_status[i] = ZKP_KZG_*.  Sharded over the context's devices in contiguous slices, double-buffered chunks of at
+ * most 2^18 proofs. */
+int32_t zkp_kzg_verify_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *proofs, const uint8_t *proof_inf,
+                             const uint64_t *zy, size_t n, uint8_t *out_status);
+/* Bytes of d_scratch zkp_kzg_verify_dev needs for n proofs (the pairs [P, pi], their flags, Gt outputs and is_one). */
+size_t zkp_kzg_scratch_bytes(size_t n);
+/* Device-resident form on device `dev` of the setup's context; asynchronous, same buffer layouts; d_scratch
+ * 16-byte aligned; stream NULL = the legacy default stream. */
+int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
+                           const uint64_t *d_zy, size_t n, uint8_t *d_status, void *d_scratch, void *stream);
+
 /* ---- measurement helpers -------------------------------------------------------------------- */
 
 /* Integer-multiply roofline probe: runs independent IMAD.WIDE.U32 (kind 0), IMAD lo (kind 1) or

@@ -10,6 +10,8 @@ TYPES = [
     (r"^zkp_ctx \*\*$", "*mut *mut ZkpCtx"), (r"^const zkp_ctx \*$", "*const ZkpCtx"), (r"^zkp_ctx \*$", "*mut ZkpCtx"),
     (r"^zkp_groth16_vk \*\*$", "*mut *mut ZkpGroth16Vk"), (r"^const zkp_groth16_vk \*$", "*const ZkpGroth16Vk"),
     (r"^zkp_groth16_vk \*$", "*mut ZkpGroth16Vk"),
+    (r"^zkp_kzg_setup \*\*$", "*mut *mut ZkpKzgSetup"), (r"^const zkp_kzg_setup \*$", "*const ZkpKzgSetup"),
+    (r"^zkp_kzg_setup \*$", "*mut ZkpKzgSetup"),
     (r"^const uint64_t \*$", "*const u64"), (r"^uint64_t \*$", "*mut u64"), (r"^const uint8_t \*$", "*const u8"),
     (r"^uint8_t \*$", "*mut u8"), (r"^const uint32_t \*$", "*const u32"), (r"^uint32_t \*$", "*mut u32"), (r"^uint32_t$", "u32"), (r"^const void \*$", "*const c_void"),
     (r"^void \*$", "*mut c_void"), (r"^const int \*$", "*const c_int"), (r"^double \*$", "*mut f64"),

@@ -27,6 +27,7 @@
 #include "../../include/zkpair.h"
 #include "fe_scratch.cuh"   // ops.cuh + the context-owned helper objects of the final exponentiation
 #include "groth16.cuh"
+#include "kzg.cuh"
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -171,6 +172,26 @@ __global__ void k_groth16_verdict(const uint8_t *__restrict__ is_one, uint8_t *_
     if (i >= n) return;
     uint8_t s = status[i];
     status[i] = s ? s : (is_one[i] ? ZKP_G16_VALID : ZKP_G16_INVALID);
+}
+
+// ---- KZG point-evaluation verification front end (kzg.cuh)
+
+// the canonical G1 generator at g1 (x|y) and G2 generator at g2 (x.c0|x.c1|y.c0|y.c1): one lane pair
+__global__ void k_kzg_generators(uint64_t *__restrict__ g1, uint64_t *__restrict__ g2) {
+    if (threadIdx.x >= 2) return;
+    store_fp(g1 + 6 * lane_par(), fp_const(ZKP_G1_GEN + ZKP_NL * lane_par()), nullptr);
+    store_fp2(g2, fp2_const(ZKP_G2_GEN), nullptr);
+    store_fp2(g2 + 12, fp2_const(ZKP_G2_GEN + 2 * ZKP_NL), nullptr);
+}
+
+__global__ void __launch_bounds__(ZKP_TPB, ZKP_MIN_BLOCKS)
+k_kzg_prepare(const Fp *__restrict__ g1_table, const uint64_t *__restrict__ proofs, const uint8_t *__restrict__ proof_inf,
+              const uint64_t *__restrict__ zy, size_t n, uint64_t *__restrict__ g1, uint8_t *__restrict__ g1inf,
+              uint8_t *__restrict__ status) {
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= n) return;
+    uint8_t s = kzg_prepare_one(g1_table, proofs + 24 * i, proof_inf ? proof_inf + 2 * i : nullptr, zy + 8 * i, g1 + 24 * i, g1inf + 2 * i);
+    if (lane_par() == 0) status[i] = s;
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -498,6 +519,58 @@ static cudaError_t launch_groth16(zkp_ctx *ctx, DevState &d, const G16Dev &k, co
     return cudaGetLastError();
 }
 
+// ---- KZG point-evaluation verification: resident setup and the per-batch launch sequence
+
+struct KzgDev {   // one device's copy of a setup, in one allocation
+    int id = 0;
+    void *mem = nullptr;
+    const Fp *prep = nullptr;    // prepared tables of G2 and -[tau]G2
+    const Fp *table = nullptr;   // window table of G1 (ZKP_G16_TABLE_FP)
+};
+struct zkp_kzg_setup {
+    zkp_ctx *ctx = nullptr;
+    std::vector<KzgDev> devs;   // one per device of ctx, same order
+};
+
+// scratch of one batch of n proofs: assembled pairs [P, pi], their flags, the Gt outputs and is_one
+struct KzgScratch {
+    uint64_t *g1, *gt;
+    uint8_t *g1inf, *is_one;
+};
+static size_t kzg_layout(size_t n, void *base, KzgScratch *s) {
+    const size_t sz[4] = {n * 2 * 96, n * 576, n * 2, n};
+    size_t off[4], o = 0;
+    for (int i = 0; i < 4; i++) {
+        off[i] = o;
+        o += align256(sz[i]);
+    }
+    if (s) {
+        uint8_t *b = (uint8_t *)base;
+        s->g1 = (uint64_t *)(b + off[0]);
+        s->gt = (uint64_t *)(b + off[1]);
+        s->g1inf = b + off[2];
+        s->is_one = b + off[3];
+    }
+    return o;
+}
+
+// front end -> prepared 2-pair check (k = kf = 2: both G2 points from the setup's tables) -> verdict
+static cudaError_t launch_kzg(zkp_ctx *ctx, DevState &d, const KzgDev &k, const uint64_t *proofs, const uint8_t *proof_inf,
+                              const uint64_t *zy, size_t n, uint8_t *status, void *scratch, uint32_t *err, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    KzgScratch s;
+    kzg_layout(n, scratch, &s);
+    k_kzg_prepare<<<grid_for(n), ZKP_TPB, 0, st>>>(k.table, proofs, proof_inf, zy, n, s.g1, s.g1inf, status);
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, nullptr, nullptr, n, 2, nullptr, s.gt, s.is_one, err, st, k.prep, nullptr, 2);
+    if (e != cudaSuccess) return e;
+    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
+    ctx->launches++;
+    return cudaGetLastError();
+}
+
 extern "C" {
 
 const char *zkp_last_error(void) { return g_err.c_str(); }
@@ -731,7 +804,7 @@ static void slice_of(size_t n, size_t ndev, size_t d, size_t &lo, size_t &hi) {
 }
 
 struct HostJob {
-    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16
+    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16 ; 96 = KZG
     const uint64_t *pts = nullptr, *scalars = nullptr;   // group op inputs (inf in g1inf, outputs in out / flags)
     const uint64_t *tab = nullptr;                       // prepared G2 line tables shared by all checks (kf of them)
     const uint8_t *tabinf = nullptr;
@@ -744,6 +817,7 @@ struct HostJob {
     int miller_mode = 1;   // mode 64: 1 = SURVEY 9.1 line scaling (the Miller product is returned), 5 = free scaling (only Gt is)
     uint64_t seed = 0, first = 0;
     const zkp_groth16_vk *vk = nullptr;   // mode 80 = Groth16 verification (proofs in pts, their flags in g1inf, inputs in scalars)
+    const zkp_kzg_setup *kzg = nullptr;   // mode 96 = KZG verification (proofs in pts, their flags in g1inf, z | y in scalars)
 };
 
 // Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
@@ -918,6 +992,23 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
                 dx = (const uint64_t *)B[B_IN].p;
             }
             CUS(launch_groth16(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, dx, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
+        } else if (j.mode == 96) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            const uint8_t *dpi = nullptr;
+            CUS(B[B_G1].ensure(cn * 192));
+            CUS(B[B_IN].ensure(cn * 64));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(B[B_OUT].ensure(kzg_layout(cn, nullptr, nullptr)));
+            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 24, cn * 192));
+            CUS(h2d(B_IN, B[B_IN].p, j.scalars + c0 * 8, cn * 64));
+            if (j.g1inf) {
+                CUS(B[B_G1INF].ensure(cn * 2));
+                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 2, cn * 2));
+                dpi = (const uint8_t *)B[B_G1INF].p;
+            }
+            CUS(launch_kzg(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, (const uint64_t *)B[B_IN].p, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p,
+                           d.d_err, st));
             CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
         } else {
             size_t np = cn * (size_t)j.k, p0 = c0 * (size_t)j.k;
@@ -1426,6 +1517,107 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
     CU(cudaSetDevice(d.id));
     cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
     CU(launch_groth16(ctx, d, vk->devs[dev], d_proofs, d_proof_inf, d_public_inputs, n, d_status, d_scratch, nullptr, st));
+    return ZKP_OK;
+}
+
+// ---- KZG point-evaluation verification
+
+int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup **out) {
+    if (!out) return fail(ZKP_ERR_INVALID_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (!tau_g2) return fail(ZKP_ERR_INVALID_ARG, "tau_g2 is NULL");
+    uint8_t st2 = 0;
+    int32_t rc = zkp_g2_check_batch(ctx, tau_g2, nullptr, 1, &st2);   // validated on the GPU
+    if (rc != ZKP_OK) return rc;
+    if (st2) return fail(ZKP_ERR_INVALID_ARG, std::string("tau_g2 ") + g16_point_error(st2));
+
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    zkp_kzg_setup *s = new zkp_kzg_setup();
+    s->ctx = ctx;
+    s->devs.resize(ctx->devs.size());
+    const size_t prep_b = align256(2 * (size_t)ZKP_G2_PREPARED_U64 * 8), tab_b = (size_t)ZKP_G16_TABLE_FP * sizeof(Fp);
+    // temporary layout: IC_0 = 0 | IC_1 = G1 (the window-table kernel's key layout, one table) | their two flags | G2 |
+    // tau_g2 | the window-table kernel's scratch
+    const size_t t_inf = 256, t_g2 = 512, t_tau = 768, t_ws = 1024;
+    const size_t tmp_b = t_ws + (size_t)ZKP_G16_WINDOWS * 2 * ZKP_G16_DIGITS * sizeof(Fp);
+    cudaError_t e = cudaSuccess;
+    for (size_t di = 0; di < ctx->devs.size() && e == cudaSuccess; di++) {
+        DevState &d = ctx->devs[di];
+        KzgDev &k = s->devs[di];
+        k.id = d.id;
+        void *tmp = nullptr;
+        e = cudaSetDevice(d.id);
+        // resident layout: prepared tables of G2, -[tau]G2 | window table of G1
+        if (e == cudaSuccess) e = cudaMalloc(&k.mem, prep_b + tab_b);
+        if (e == cudaSuccess) e = cudaMalloc(&tmp, tmp_b);
+        if (e == cudaSuccess) {
+            uint8_t *m = (uint8_t *)k.mem, *t = (uint8_t *)tmp;
+            k.prep = (const Fp *)m;
+            k.table = (const Fp *)(m + prep_b);
+            cudaStream_t st = d.stream[0];
+            e = cudaMemsetAsync(t, 0, t_g2, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(t + t_tau, tau_g2, 192, cudaMemcpyHostToDevice, st);
+            if (e == cudaSuccess) {
+                k_kzg_generators<<<1, 32, 0, st>>>((uint64_t *)t + 12, (uint64_t *)(t + t_g2));
+                k_g2_prepare<<<grid_for(1), ZKP_TPB, 0, st>>>((const uint64_t *)(t + t_g2), (Fp *)k.prep, nullptr, 1);
+                k_g16_neg_prepare<<<grid_for(1), ZKP_TPB, 0, st>>>((const uint64_t *)(t + t_tau),
+                                                                   (Fp *)(m + (size_t)ZKP_G2_PREPARED_U64 * 8), 1);
+                k_g16_window_tables<<<1, ZKP_TPB, 0, st>>>((const uint64_t *)t, t + t_inf, 1, (Fp *)k.table, (Fp *)(t + t_ws));
+                ctx->launches += 4;
+                e = cudaGetLastError();
+            }
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        }
+        if (tmp) cudaFree(tmp);
+    }
+    if (e != cudaSuccess) {
+        std::string msg = std::string("KZG setup failed: ") + cudaGetErrorString(e);
+        zkp_kzg_setup_destroy(s);
+        return fail(ZKP_ERR_CUDA, msg);
+    }
+    *out = s;
+    return ZKP_OK;
+}
+
+void zkp_kzg_setup_destroy(zkp_kzg_setup *s) {
+    if (!s) return;
+    DeviceGuard guard;
+    for (KzgDev &k : s->devs) {
+        if (!k.mem) continue;
+        cudaSetDevice(k.id);
+        cudaFree(k.mem);
+    }
+    delete s;
+}
+
+size_t zkp_kzg_scratch_bytes(size_t n) { return kzg_layout(n, nullptr, nullptr); }
+
+int32_t zkp_kzg_verify_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *proofs, const uint8_t *proof_inf, const uint64_t *zy,
+                             size_t n, uint8_t *out_status) {
+    if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (n && (!proofs || !zy || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 96; j.kzg = s; j.pts = proofs; j.g1inf = proof_inf; j.scalars = zy; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
+                           const uint64_t *d_zy, size_t n, uint8_t *d_status, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc) return rc;
+    if (!s) return fail(ZKP_ERR_INVALID_ARG, "setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (n && (!d_proofs || !d_zy || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if ((uintptr_t)d_scratch & 15) return fail(ZKP_ERR_INVALID_ARG, "d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
+    CU(launch_kzg(ctx, d, s->devs[dev], d_proofs, d_proof_inf, d_zy, n, d_status, d_scratch, nullptr, st));
     return ZKP_OK;
 }
 

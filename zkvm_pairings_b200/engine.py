@@ -38,6 +38,9 @@ MODE_MILLER_FOR_FINAL_EXP = 5   # Miller loop whose output only feeds a final ex
 G16_VALID, G16_INVALID, G16_BAD_POINT, G16_BAD_INPUT = 0, 1, 2, 3
 GROTH16_PROOF_U64 = 48
 GROTH16_MAX_PUBLIC = 256
+# per-proof verdicts of kzg_verify_batch / kzg_verify_dev (include/zkpair.h ZKP_KZG_*)
+KZG_VALID, KZG_INVALID, KZG_BAD_POINT, KZG_BAD_SCALAR = 0, 1, 2, 3
+KZG_PROOF_U64 = 24
 
 
 class ZkpError(RuntimeError):
@@ -81,24 +84,27 @@ def _dptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class Groth16VerifyingKey:
-    """A verifying key resident on every device of one engine (PairingEngine.groth16_prepare_vk).  It holds a
-    reference to its engine, so the engine's context outlives it; ``close()`` (or leaving a ``with`` block)
-    frees the device memory."""
+class _ContextObject:
+    """Device memory that belongs to one engine's context (a C handle freed by ``_destroy``).  It holds a reference
+    to its engine, so the engine's context outlives it; ``close()`` (or leaving a ``with`` block) frees the device
+    memory, and the engine closes it first when the engine itself is closed."""
+    _destroy = ""
+    _what = ""
 
-    def __init__(self, engine: "PairingEngine", handle: ctypes.c_void_p, n_public: int):
-        self.engine, self._vk, self.n_public = engine, handle, n_public
+    def __init__(self, engine: "PairingEngine", handle: ctypes.c_void_p):
+        self.engine, self._h = engine, handle
+        engine._resident.add(self)
 
     @property
     def handle(self):
-        if not self._vk:
-            raise ValueError("the verifying key is closed")
-        return self._vk
+        if not self._h:
+            raise ValueError("the %s is closed" % self._what)
+        return self._h
 
     def close(self):
-        if getattr(self, "_vk", None):
-            self.engine._lib.zkp_groth16_vk_destroy(self._vk)
-            self._vk = None
+        if getattr(self, "_h", None):
+            getattr(self.engine._lib, self._destroy)(self._h)
+            self._h = None
 
     def __del__(self):
         try:
@@ -113,12 +119,28 @@ class Groth16VerifyingKey:
         self.close()
 
 
+class Groth16VerifyingKey(_ContextObject):
+    """A verifying key resident on every device of one engine (PairingEngine.groth16_prepare_vk)."""
+    _destroy = "zkp_groth16_vk_destroy"
+    _what = "verifying key"
+
+    def __init__(self, engine: "PairingEngine", handle: ctypes.c_void_p, n_public: int):
+        super().__init__(engine, handle)
+        self.n_public = n_public
+
+
+class KzgSetup(_ContextObject):
+    """A KZG setup ([tau]G2) resident on every device of one engine (PairingEngine.kzg_setup)."""
+    _destroy = "zkp_kzg_setup_destroy"
+    _what = "KZG setup"
+
+
 class PairingEngine:
     """One C-ABI context: a set of CUDA devices with their streams and scratch buffers."""
 
     def __init__(self, devices: Optional[Sequence[int]] = None):
         self._lib = _lib.load()
-        self._vks = weakref.WeakSet()   # verifying keys of this context: freed before the context is
+        self._resident = weakref.WeakSet()   # verifying keys and KZG setups of this context: freed before the context is
         self._ctx = ctypes.c_void_p()
         if devices is None:
             arr, n = None, 0
@@ -138,8 +160,8 @@ class PairingEngine:
         raise ZkpError(rc, msg)
 
     def close(self):
-        for vk in list(getattr(self, "_vks", ())):
-            vk.close()
+        for obj in list(getattr(self, "_resident", ())):
+            obj.close()
         if getattr(self, "_ctx", None):
             self._lib.zkp_ctx_destroy(self._ctx)
             self._ctx = None
@@ -337,9 +359,7 @@ class PairingEngine:
         h = ctypes.c_void_p()
         self._check(self._lib.zkp_groth16_vk_create(self._ctx, _ptr(a), _ptr(b), _ptr(g), _ptr(d), _ptr(ic), _ptr(ii), n_public,
                                                     ctypes.byref(h)))
-        vk = Groth16VerifyingKey(self, h, n_public)
-        self._vks.add(vk)
-        return vk
+        return Groth16VerifyingKey(self, h, n_public)
 
     def groth16_verify_batch(self, vk: Groth16VerifyingKey, proofs, public_inputs, proof_inf=None):
         """proofs (n, 48) = A | B | C, public_inputs (n, n_public, 4) Fr limbs, proof_inf (n, 3) or None ->
@@ -360,6 +380,34 @@ class PairingEngine:
         """Asynchronous form on device-resident torch tensors; d_scratch holds groth16_scratch_bytes(n) bytes."""
         self._check(self._lib.zkp_groth16_verify_dev(self._ctx, dev, vk.handle, _dptr(d_proofs), _dptr(d_proof_inf), _dptr(d_public_inputs),
                                                      n, _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
+    # ------------------------------------------------------------------ KZG point-evaluation verification
+    def kzg_setup(self, tau_g2) -> KzgSetup:
+        """[tau]G2 (24,) -> a setup validated and resident on the GPU.  Raises NonCanonicalError for a limb >= p,
+        ZkpError (INVALID_ARG) for an off-curve or non-subgroup point."""
+        t = np.ascontiguousarray(tau_g2, dtype=np.uint64).reshape(24)
+        h = ctypes.c_void_p()
+        self._check(self._lib.zkp_kzg_setup_create(self._ctx, _ptr(t), ctypes.byref(h)))
+        return KzgSetup(self, h)
+
+    def kzg_verify_batch(self, setup: KzgSetup, proofs, zy, proof_inf=None):
+        """proofs (n, 24) = C | pi, zy (n, 8) = z | y Fr limbs, proof_inf (n, 2) or None -> uint8 (n,) verdicts KZG_*."""
+        pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(-1, KZG_PROOF_U64)
+        n = pr.shape[0]
+        s = np.ascontiguousarray(zy, dtype=np.uint64).reshape(n, 8)
+        pi = None if proof_inf is None else _np8(proof_inf, 2 * n)
+        st = np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_verify_batch(self._ctx, setup.handle, _ptr(pr), _ptr(pi), _ptr(s), n, _ptr(st)))
+        return st
+
+    def kzg_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_kzg_scratch_bytes(n))
+
+    def kzg_verify_dev(self, setup: KzgSetup, d_proofs, d_zy, n: int, d_status, d_scratch, d_proof_inf=None, stream: int = 0,
+                       dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_scratch holds kzg_scratch_bytes(n) bytes."""
+        self._check(self._lib.zkp_kzg_verify_dev(self._ctx, dev, setup.handle, _dptr(d_proofs), _dptr(d_proof_inf), _dptr(d_zy), n,
+                                                 _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ byte (de)serialisation (SURVEY 8f)
     def fp_from_bytes_batch(self, data):

@@ -164,3 +164,36 @@ def groth16_proofs(engine, n: int, n_public: int, seed: int = 0x6716, corrupt_ev
     return {"alpha": k1[0], "beta": k2[0], "gamma": k2[1], "delta": k2[2], "ic": k1[1:],
             "proofs": np.concatenate([gA, gB, gC], axis=1), "inputs": inputs, "l": _fr_matrix(ls),
             "expect": corrupt.astype(np.uint8)}
+
+
+def kzg_proofs(engine, n: int, seed: int = 0x4844, corrupt_every: int = 100, corrupt_at: int = 7):
+    """KZG point-evaluation setup and proofs with known verdicts, from the trapdoor construction.
+
+    A seeded tau gives the setup [tau]G2.  Per proof: random z, y and q < r, pi = q G1 and C = (y + q (tau - z)) G1
+    (engine.g1_mul_batch), so C - y G1 = q (tau - z) G1 opens the committed polynomial at z to y.  A seeded 1 % of the
+    claimed values is corrupted as y + 1 mod r, so the expected verdicts are known without running a pairing.
+    Returns a dict:
+        tau_g2 (24,)                                  the setup
+        proofs (n, 24) C | pi, zy (n, 8) z | y          what the verifier receives
+        p (n, 4) the discrete log of P = C + z pi - y G1 the verifier derives
+        expect (n,) uint8 ZKP_KZG_VALID / ZKP_KZG_INVALID
+    """
+    import random
+    rng = random.Random(seed)
+    n = int(n)
+    tau = rng.randrange(1, R_ORDER)
+    g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
+    tg, _ = engine.g2_mul_batch(g2gen[None], _fr_matrix([tau]))
+    corrupt = np.zeros(n, dtype=bool)
+    if corrupt_every:
+        corrupt[corrupt_at % corrupt_every::corrupt_every] = True
+    z = [rng.randrange(R_ORDER) for _ in range(n)]
+    y = [rng.randrange(R_ORDER) for _ in range(n)]
+    q = [rng.randrange(1, R_ORDER) for _ in range(n)]
+    c = [(yi + qi * (tau - zi)) % R_ORDER for zi, yi, qi in zip(z, y, q)]
+    y = [(yi + 1) % R_ORDER if bad else yi for yi, bad in zip(y, corrupt)]
+    p = [(ci - yi + zi * qi) % R_ORDER for ci, yi, zi, qi in zip(c, y, z, q)]
+    pts, _ = engine.g1_mul_batch(np.tile(g1gen, (2 * n, 1)), _fr_matrix(c + q))
+    return {"tau_g2": tg[0], "proofs": np.concatenate([pts[:n], pts[n:]], axis=1),
+            "zy": np.concatenate([_fr_matrix(z), _fr_matrix(y)], axis=1), "p": _fr_matrix(p),
+            "expect": corrupt.astype(np.uint8)}
