@@ -326,7 +326,8 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
 typedef struct zkp_kzg_setup zkp_kzg_setup;
 
 /* Validates [tau]G2 on the GPU and builds the resident setup on every device of ctx: the prepared tables of G2 and
- * -[tau]G2 and a fixed-base window table of G1 (32 x 255 affine points, 765 KiB).  There is no infinity flag: the
+ * -[tau]G2, a fixed-base window table of G1 (32 x 255 affine points, 765 KiB) and the 4096-point evaluation domain of
+ * zkp_kzg_verify_blob_batch (128 KiB).  There is no infinity flag: the
  * identity is not a valid setup.  A limb >= p gives ZKP_ERR_NONCANONICAL; an off-curve or non-subgroup point gives
  * ZKP_ERR_INVALID_ARG, the message naming tau_g2.  The setup belongs to ctx: other contexts reject it, and it must be
  * destroyed before ctx. */
@@ -343,6 +344,32 @@ size_t zkp_kzg_scratch_bytes(size_t n);
  * 16-byte aligned; stream NULL = the legacy default stream. */
 int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
                            const uint64_t *d_zy, size_t n, uint8_t *d_status, void *d_scratch, void *stream);
+
+/* ---- EIP-4844 blob verification (one verdict per blob) -------------------------------------------
+ * verify_blob_kzg_proof(blob, C, pi) of the consensus specs (deneb polynomial-commitments.md) on the GPU: z is the
+ * Fiat-Shamir challenge SHA-256(b"FSBLOBVERIFY_V1_" | 4096 as 16 big-endian bytes | blob | compressed C) mod r, y the
+ * blob's polynomial (its 4096 big-endian elements are the values at the bit-reversed roots of unity of order 4096)
+ * evaluated at z, and the verdict is that of zkp_kzg_verify_batch for (C, z, y, pi).  C and pi cross the boundary as
+ * affine limbs with infinity flags, as for zkp_kzg_verify_batch; the compressed encoding of C that the transcript
+ * hashes is derived on the device.  Verdicts are ZKP_KZG_*; z and y are derived here, so ZKP_KZG_BAD_SCALAR means
+ * that some blob element is >= r (ZKP_KZG_BAD_POINT takes precedence).  The call returns ZKP_OK for malformed blobs
+ * and proofs.  A blob is 128 KiB: the host path streams double-buffered chunks of at most 2^14 blobs (2 GiB) per
+ * device, so a large batch takes up to 2 x 2 GiB of device buffers per device, and pageable blobs are staged through up
+ * to 2 x 2 GiB of pinned memory per device (smaller batches take proportionally less). */
+#define ZKP_BLOB_FIELD_ELEMENTS 4096
+#define ZKP_BLOB_BYTES (32 * ZKP_BLOB_FIELD_ELEMENTS)
+/* n blobs (n x ZKP_BLOB_BYTES), proofs / proof_inf exactly as zkp_kzg_verify_batch (C | pi) -> out_status[i] = ZKP_KZG_*.
+ * out_zy (optional, n x 8 u64) receives the derived z | y; for a blob with an element >= r it holds r | 0, so
+ * zkp_kzg_verify_batch(proofs, out_zy) reproduces out_status in every slot. */
+int32_t zkp_kzg_verify_blob_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *proofs,
+                                  const uint8_t *proof_inf, size_t n, uint8_t *out_status, uint64_t *out_zy);
+/* Bytes of d_scratch zkp_kzg_verify_blob_dev needs for n blobs (z | y, then zkp_kzg_scratch_bytes(n)). */
+size_t zkp_kzg_blob_scratch_bytes(size_t n);
+/* Device-resident form on device `dev` of the setup's context; asynchronous, same buffer layouts; d_blobs and d_scratch
+ * 16-byte aligned; d_out_zy optional; stream NULL = the legacy default stream. */
+int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_proofs,
+                                const uint8_t *d_proof_inf, size_t n, uint8_t *d_status, uint64_t *d_out_zy, void *d_scratch,
+                                void *stream);
 
 /* ---- measurement helpers -------------------------------------------------------------------- */
 

@@ -28,6 +28,7 @@
 #include "fe_scratch.cuh"   // ops.cuh + the context-owned helper objects of the final exponentiation
 #include "groth16.cuh"
 #include "kzg.cuh"
+#include "blob.cuh"
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -192,6 +193,60 @@ k_kzg_prepare(const Fp *__restrict__ g1_table, const uint64_t *__restrict__ proo
     if (i >= n) return;
     uint8_t s = kzg_prepare_one(g1_table, proofs + 24 * i, proof_inf ? proof_inf + 2 * i : nullptr, zy + 8 * i, g1 + 24 * i, g1inf + 2 * i);
     if (lane_par() == 0) status[i] = s;
+}
+
+// ---- EIP-4844 blob verification front end (blob.cuh)
+
+#ifndef ZKP_BLOB_CHALLENGE_TPB
+#define ZKP_BLOB_CHALLENGE_TPB 32   // one thread per blob: small blocks spread a small batch over more SMs
+#endif
+
+// the setup's domain table roots_brp (Montgomery), one thread per entry
+__global__ void k_blob_domain(Fr *__restrict__ roots) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < ZKP_BLOB_N) roots[i] = blob_root(i);
+}
+
+// z of every blob (canonical, zy[8 i .. 8 i + 4)): one thread per blob, 2050 dependent SHA-256 compressions
+__global__ void __launch_bounds__(ZKP_BLOB_CHALLENGE_TPB)
+k_blob_challenge(const uint8_t *__restrict__ blobs, const uint64_t *__restrict__ proofs, const uint8_t *__restrict__ proof_inf, size_t n,
+                 uint64_t *__restrict__ zy) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint32_t digest[8];
+    blob_challenge_one(blobs + i * ZKP_BLOB_BYTES_, proofs + 24 * i, proof_inf ? proof_inf[2 * i] : 0, digest, zy + 8 * i);
+}
+
+// y = p(z) of every blob (zy[8 i + 4 .. 8 i + 8)), or z = r, y = 0 for a blob with an element >= r: one block per blob,
+// thread t owning elements t + 256 k (a warp's 32-byte loads are contiguous); one inversion per blob
+__global__ void __launch_bounds__(ZKP_BLOB_TPB)
+k_blob_eval(const uint8_t *__restrict__ blobs, const Fr *__restrict__ roots, uint64_t *__restrict__ zy) {
+    __shared__ BlobShared sh;
+    const int t = threadIdx.x;
+    const uint8_t *blob = blobs + (size_t)blockIdx.x * ZKP_BLOB_BYTES_;
+    uint64_t *o = zy + 8 * (size_t)blockIdx.x;
+    const Fr zm = blob_z_mont(o);
+    BlobLane ln;
+    if (t == 0) blob_eval_init(sh);
+    blob_eval_prefix(t, roots, zm, sh, ln);
+    __syncthreads();
+    for (int w = ZKP_BLOB_TPB / 2; w >= 1; w >>= 1) {
+        if (t < w) blob_tree_mul(sh.tree, w + t);
+        __syncthreads();
+    }
+    if (t == 0) blob_tree_invert_root(sh.tree);
+    __syncthreads();
+    for (int w = 1; w < ZKP_BLOB_TPB; w <<= 1) {
+        if (t < w) blob_tree_inv(sh.tree, w + t);
+        __syncthreads();
+    }
+    blob_eval_terms(t, blob, roots, zm, sh, ln);
+    __syncthreads();
+    for (int w = ZKP_BLOB_TPB / 2; w >= 1; w >>= 1) {
+        if (t < w) blob_tree_add(sh.tree, w + t);
+        __syncthreads();
+    }
+    if (t == 0) blob_eval_finish(sh, zm, o);
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -526,6 +581,7 @@ struct KzgDev {   // one device's copy of a setup, in one allocation
     void *mem = nullptr;
     const Fp *prep = nullptr;    // prepared tables of G2 and -[tau]G2
     const Fp *table = nullptr;   // window table of G1 (ZKP_G16_TABLE_FP)
+    const Fr *roots = nullptr;   // the blob domain roots_brp (ZKP_BLOB_N Fr, Montgomery)
 };
 struct zkp_kzg_setup {
     zkp_ctx *ctx = nullptr;
@@ -569,6 +625,34 @@ static cudaError_t launch_kzg(zkp_ctx *ctx, DevState &d, const KzgDev &k, const 
     k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
     ctx->launches++;
     return cudaGetLastError();
+}
+
+// ---- EIP-4844 blob verification: z by k_blob_challenge, y by k_blob_eval, then the point-evaluation check
+
+#ifndef ZKP_BLOB_CHUNK
+// blobs per host pipeline chunk: 2 GiB of blobs per buffer set.  Measured at 2^15 blobs (profiles/r3c_kzg_blob_chunk.txt,
+// B200 at 1000 W), chunks of 2^10 .. 2^14 blobs: 42 / 71 / 108 / 146 / 171 k blobs/s from pinned and 31 / 44 / 56 / 64 /
+// 69 k blobs/s from pageable memory; every launch sequence pays the fixed latency of the transcript (4.3 ms).
+#define ZKP_BLOB_CHUNK (1u << 14)
+#endif
+
+// scratch of one batch of n blobs: z | y (n x 64 bytes), then the point-evaluation scratch
+static size_t blob_zy_bytes(size_t n) { return align256(n * 64); }
+extern "C" size_t zkp_kzg_blob_scratch_bytes(size_t n) { return blob_zy_bytes(n) + kzg_layout(n, nullptr, nullptr); }
+
+// zy = the caller's z | y buffer, or NULL for the one in scratch
+static cudaError_t launch_kzg_blob(zkp_ctx *ctx, DevState &d, const KzgDev &k, const uint8_t *blobs, const uint64_t *proofs,
+                                   const uint8_t *proof_inf, size_t n, uint8_t *status, uint64_t *zy, void *scratch, uint32_t *err,
+                                   cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    if (!zy) zy = (uint64_t *)scratch;
+    k_blob_challenge<<<(unsigned)((n + ZKP_BLOB_CHALLENGE_TPB - 1) / ZKP_BLOB_CHALLENGE_TPB), ZKP_BLOB_CHALLENGE_TPB, 0, st>>>(
+        blobs, proofs, proof_inf, n, zy);
+    k_blob_eval<<<(unsigned)n, ZKP_BLOB_TPB, 0, st>>>(blobs, k.roots, zy);
+    ctx->launches += 2;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    return launch_kzg(ctx, d, k, proofs, proof_inf, zy, n, status, (uint8_t *)scratch + blob_zy_bytes(n), err, st);
 }
 
 extern "C" {
@@ -804,7 +888,7 @@ static void slice_of(size_t n, size_t ndev, size_t d, size_t &lo, size_t &hi) {
 }
 
 struct HostJob {
-    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16 ; 96 = KZG
+    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16 ; 96 = KZG ; 112 = KZG blobs
     const uint64_t *pts = nullptr, *scalars = nullptr;   // group op inputs (inf in g1inf, outputs in out / flags)
     const uint64_t *tab = nullptr;                       // prepared G2 line tables shared by all checks (kf of them)
     const uint8_t *tabinf = nullptr;
@@ -818,6 +902,7 @@ struct HostJob {
     uint64_t seed = 0, first = 0;
     const zkp_groth16_vk *vk = nullptr;   // mode 80 = Groth16 verification (proofs in pts, their flags in g1inf, inputs in scalars)
     const zkp_kzg_setup *kzg = nullptr;   // mode 96 = KZG verification (proofs in pts, their flags in g1inf, z | y in scalars)
+    const uint8_t *blobs = nullptr;       // mode 112 = KZG blob verification (setup in kzg, proofs in pts, flags in g1inf, z | y out in out)
 };
 
 // Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
@@ -836,7 +921,7 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
     CUS(cudaStreamSynchronize(d.stream[0]));
     int na = 0, nb = 0, nr = 0;
     if (j.mode == 16) tower_op_shape(j.op, na, nb, nr);
-    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : ZKP_CHUNK;
+    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : j.mode == 112 ? (size_t)ZKP_BLOB_CHUNK : (size_t)ZKP_CHUNK;
     int s = 0;
     cudaStream_t st = nullptr;
     d.pend[0].clear();   // (a job that failed half-way leaves nothing behind for the next one)
@@ -993,6 +1078,24 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
             }
             CUS(launch_groth16(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, dx, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
             CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
+        } else if (j.mode == 112) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            const uint8_t *dpi = nullptr;
+            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
+            CUS(B[B_G1].ensure(cn * 192));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(B[B_OUT].ensure(zkp_kzg_blob_scratch_bytes(cn)));
+            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
+            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 24, cn * 192));
+            if (j.g1inf) {
+                CUS(B[B_G1INF].ensure(cn * 2));
+                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 2, cn * 2));
+                dpi = (const uint8_t *)B[B_G1INF].p;
+            }
+            CUS(launch_kzg_blob(ctx, d, kd, (const uint8_t *)B[B_IN].p, (const uint64_t *)B[B_G1].p, dpi, cn, (uint8_t *)B[B_FLAG].p, nullptr,
+                                B[B_OUT].p, d.d_err, st));
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
+            if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, B[B_OUT].p, cn * 64));   // z | y, first in the scratch
         } else if (j.mode == 96) {
             const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
             const uint8_t *dpi = nullptr;
@@ -1537,7 +1640,8 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
     zkp_kzg_setup *s = new zkp_kzg_setup();
     s->ctx = ctx;
     s->devs.resize(ctx->devs.size());
-    const size_t prep_b = align256(2 * (size_t)ZKP_G2_PREPARED_U64 * 8), tab_b = (size_t)ZKP_G16_TABLE_FP * sizeof(Fp);
+    const size_t prep_b = align256(2 * (size_t)ZKP_G2_PREPARED_U64 * 8), tab_b = align256((size_t)ZKP_G16_TABLE_FP * sizeof(Fp));
+    const size_t roots_b = (size_t)ZKP_BLOB_N * sizeof(Fr);
     // temporary layout: IC_0 = 0 | IC_1 = G1 (the window-table kernel's key layout, one table) | their two flags | G2 |
     // tau_g2 | the window-table kernel's scratch
     const size_t t_inf = 256, t_g2 = 512, t_tau = 768, t_ws = 1024;
@@ -1549,13 +1653,14 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
         k.id = d.id;
         void *tmp = nullptr;
         e = cudaSetDevice(d.id);
-        // resident layout: prepared tables of G2, -[tau]G2 | window table of G1
-        if (e == cudaSuccess) e = cudaMalloc(&k.mem, prep_b + tab_b);
+        // resident layout: prepared tables of G2, -[tau]G2 | window table of G1 | blob domain roots_brp
+        if (e == cudaSuccess) e = cudaMalloc(&k.mem, prep_b + tab_b + roots_b);
         if (e == cudaSuccess) e = cudaMalloc(&tmp, tmp_b);
         if (e == cudaSuccess) {
             uint8_t *m = (uint8_t *)k.mem, *t = (uint8_t *)tmp;
             k.prep = (const Fp *)m;
             k.table = (const Fp *)(m + prep_b);
+            k.roots = (const Fr *)(m + prep_b + tab_b);
             cudaStream_t st = d.stream[0];
             e = cudaMemsetAsync(t, 0, t_g2, st);
             if (e == cudaSuccess) e = cudaMemcpyAsync(t + t_tau, tau_g2, 192, cudaMemcpyHostToDevice, st);
@@ -1565,7 +1670,8 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
                 k_g16_neg_prepare<<<grid_for(1), ZKP_TPB, 0, st>>>((const uint64_t *)(t + t_tau),
                                                                    (Fp *)(m + (size_t)ZKP_G2_PREPARED_U64 * 8), 1);
                 k_g16_window_tables<<<1, ZKP_TPB, 0, st>>>((const uint64_t *)t, t + t_inf, 1, (Fp *)k.table, (Fp *)(t + t_ws));
-                ctx->launches += 4;
+                k_blob_domain<<<ZKP_BLOB_N / 128, 128, 0, st>>>((Fr *)k.roots);
+                ctx->launches += 5;
                 e = cudaGetLastError();
             }
             if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -1618,6 +1724,35 @@ int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, co
     CU(cudaSetDevice(d.id));
     cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
     CU(launch_kzg(ctx, d, s->devs[dev], d_proofs, d_proof_inf, d_zy, n, d_status, d_scratch, nullptr, st));
+    return ZKP_OK;
+}
+
+// ---- EIP-4844 blob verification
+
+int32_t zkp_kzg_verify_blob_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *proofs,
+                                  const uint8_t *proof_inf, size_t n, uint8_t *out_status, uint64_t *out_zy) {
+    if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (n && (!blobs || !proofs || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 112; j.kzg = s; j.blobs = blobs; j.pts = proofs; j.g1inf = proof_inf; j.flags = out_status; j.out = out_zy;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_proofs,
+                                const uint8_t *d_proof_inf, size_t n, uint8_t *d_status, uint64_t *d_out_zy, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc) return rc;
+    if (!s) return fail(ZKP_ERR_INVALID_ARG, "setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (n && (!d_blobs || !d_proofs || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
+    CU(launch_kzg_blob(ctx, d, s->devs[dev], d_blobs, d_proofs, d_proof_inf, n, d_status, d_out_zy, d_scratch, nullptr, st));
     return ZKP_OK;
 }
 

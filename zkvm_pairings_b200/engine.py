@@ -41,6 +41,7 @@ GROTH16_MAX_PUBLIC = 256
 # per-proof verdicts of kzg_verify_batch / kzg_verify_dev (include/zkpair.h ZKP_KZG_*)
 KZG_VALID, KZG_INVALID, KZG_BAD_POINT, KZG_BAD_SCALAR = 0, 1, 2, 3
 KZG_PROOF_U64 = 24
+BLOB_BYTES = 32 * 4096   # one EIP-4844 blob: 4096 big-endian field elements (include/zkpair.h ZKP_BLOB_BYTES)
 
 
 class ZkpError(RuntimeError):
@@ -408,6 +409,29 @@ class PairingEngine:
         """Asynchronous form on device-resident torch tensors; d_scratch holds kzg_scratch_bytes(n) bytes."""
         self._check(self._lib.zkp_kzg_verify_dev(self._ctx, dev, setup.handle, _dptr(d_proofs), _dptr(d_proof_inf), _dptr(d_zy), n,
                                                  _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
+    # ------------------------------------------------------------------ EIP-4844 blob verification
+    def kzg_verify_blob_batch(self, setup: KzgSetup, blobs, proofs, proof_inf=None, return_zy: bool = False):
+        """blobs (n, BLOB_BYTES) uint8, proofs (n, 24) = C | pi, proof_inf (n, 2) or None -> uint8 (n,) verdicts KZG_*
+        (verify_blob_kzg_proof); with return_zy also the derived z | y (n, 8) (r | 0 for a blob with an element >= r)."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(n, KZG_PROOF_U64)
+        pi = None if proof_inf is None else _np8(proof_inf, 2 * n)
+        st = np.zeros(n, np.uint8)
+        zy = np.zeros((n, 8), np.uint64) if return_zy else None
+        self._check(self._lib.zkp_kzg_verify_blob_batch(self._ctx, setup.handle, _ptr(b), _ptr(pr), _ptr(pi), n, _ptr(st), _ptr(zy)))
+        return (st, zy) if return_zy else st
+
+    def kzg_blob_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_kzg_blob_scratch_bytes(n))
+
+    def kzg_verify_blob_dev(self, setup: KzgSetup, d_blobs, d_proofs, n: int, d_status, d_scratch, d_proof_inf=None, d_out_zy=None,
+                            stream: int = 0, dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_scratch holds kzg_blob_scratch_bytes(n) bytes, d_blobs
+        and d_scratch 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_verify_blob_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), _dptr(d_proofs), _dptr(d_proof_inf), n,
+                                                      _dptr(d_status), _dptr(d_out_zy), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ byte (de)serialisation (SURVEY 8f)
     def fp_from_bytes_batch(self, data):

@@ -197,3 +197,99 @@ def kzg_proofs(engine, n: int, seed: int = 0x4844, corrupt_every: int = 100, cor
     return {"tau_g2": tg[0], "proofs": np.concatenate([pts[:n], pts[n:]], axis=1),
             "zy": np.concatenate([_fr_matrix(z), _fr_matrix(y)], axis=1), "p": _fr_matrix(p),
             "expect": corrupt.astype(np.uint8)}
+
+
+BLOB_N = 4096                # EIP-4844 FIELD_ELEMENTS_PER_BLOB
+BLOB_BYTES = 32 * BLOB_N
+P_BASE = 0x1a0111ea397fe69a4b1ba7b6434bacd764774b84f38512bf6730d2a0f6b0f6241eabfffeb153ffffb9feffffffffaaab
+
+
+def blob_domain():
+    """roots_brp: the 4096th roots of unity of Fr (generator 7^((r - 1) / 4096)) in bit-reversed order."""
+    w = pow(7, (R_ORDER - 1) // BLOB_N, R_ORDER)
+    roots = [1] * BLOB_N
+    for i in range(1, BLOB_N):
+        roots[i] = roots[i - 1] * w % R_ORDER
+    return [roots[int(format(i, "012b")[::-1], 2)] for i in range(BLOB_N)]
+
+
+def _batch_inv(vals):
+    pre, acc = [], 1
+    for v in vals:
+        pre.append(acc)
+        acc = acc * v % R_ORDER
+    inv, out = pow(acc, -1, R_ORDER), [0] * len(vals)
+    for i in range(len(vals) - 1, -1, -1):
+        out[i] = inv * pre[i] % R_ORDER
+        inv = inv * vals[i] % R_ORDER
+    return out
+
+
+def blob_eval(poly, z, roots):
+    """The blob's polynomial (values at roots) at z, barycentric (the value itself when z is a root)."""
+    if z in roots:
+        return poly[roots.index(z)]
+    inv = _batch_inv([(z - w) % R_ORDER for w in roots])
+    s = sum(p * w % R_ORDER * i for p, w, i in zip(poly, roots, inv)) % R_ORDER
+    return s * (pow(z, BLOB_N, R_ORDER) - 1) * pow(BLOB_N, -1, R_ORDER) % R_ORDER
+
+
+def g1_compressed(xy, inf=False) -> bytes:
+    """The 48-byte compressed encoding of a G1 point given as canonical limbs x | y (12 u64)."""
+    if inf:
+        return b"\xc0" + bytes(47)
+    x = sum(int(v) << (64 * k) for k, v in enumerate(xy[:6]))
+    y = sum(int(v) << (64 * k) for k, v in enumerate(xy[6:12]))
+    b = bytearray(x.to_bytes(48, "big"))
+    b[0] |= 0x80 | (0x20 if y > (P_BASE - 1) // 2 else 0)
+    return bytes(b)
+
+
+def blob_challenge(blob: bytes, c48: bytes) -> int:
+    """compute_challenge: SHA-256 of the Fiat-Shamir transcript as a big-endian integer mod r."""
+    import hashlib
+    data = b"FSBLOBVERIFY_V1_" + BLOB_N.to_bytes(16, "big") + blob + c48
+    return int.from_bytes(hashlib.sha256(data).digest(), "big") % R_ORDER
+
+
+def kzg_blob_proofs(engine, n: int, seed: int = 0x4844, distinct: int = 64, corrupt_every: int = 100, corrupt_at: int = 7):
+    """EIP-4844 blobs, commitments and proofs with known verdicts, from the trapdoor construction.
+
+    A seeded tau gives the setup [tau]G2.  Per distinct blob: random elements p_i < r, c = p(tau) from the Lagrange
+    coefficients at tau, C = c G1 (engine.g1_mul_batch), z from the transcript of the blob and C, y = p(z), and
+    pi = q G1 with q = (c - y) / (tau - z).  Python costs about 10 ms per distinct blob, so at most `distinct` blobs
+    are built and tiled over the n slots.  A seeded 1 % of the slots gets pi = (q + 1) G1, so the expected verdicts are
+    known without running a pairing.  Returns a dict:
+        tau_g2 (24,)                                    the setup
+        blobs (n, BLOB_BYTES) uint8, proofs (n, 24) C | pi   what the verifier receives
+        zy (n, 8) the z | y the verifier derives         expect (n,) uint8 ZKP_KZG_VALID / ZKP_KZG_INVALID
+    """
+    import random
+    rng = random.Random(seed)
+    n = int(n)
+    m = max(1, min(n, int(distinct)))
+    tau = rng.randrange(1, R_ORDER)
+    roots = blob_domain()
+    g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
+    tg, _ = engine.g2_mul_batch(g2gen[None], _fr_matrix([tau]))
+    scale = (pow(tau, BLOB_N, R_ORDER) - 1) * pow(BLOB_N, -1, R_ORDER) % R_ORDER
+    lag = [scale * w % R_ORDER * i % R_ORDER for w, i in zip(roots, _batch_inv([(tau - w) % R_ORDER for w in roots]))]
+    polys = [[rng.randrange(R_ORDER) for _ in range(BLOB_N)] for _ in range(m)]
+    blobs = np.frombuffer(b"".join(v.to_bytes(32, "big") for p in polys for v in p), dtype=np.uint8).reshape(m, BLOB_BYTES)
+    cs = [sum(p * l for p, l in zip(poly, lag)) % R_ORDER for poly in polys]
+    cpts, cinf = engine.g1_mul_batch(np.tile(g1gen, (m, 1)), _fr_matrix(cs))
+    zs, ys, qs = [], [], []
+    for k in range(m):
+        z = blob_challenge(blobs[k].tobytes(), g1_compressed(cpts[k], cinf[k]))
+        y = blob_eval(polys[k], z, roots)
+        zs.append(z)
+        ys.append(y)
+        qs.append((cs[k] - y) * pow((tau - z) % R_ORDER, -1, R_ORDER) % R_ORDER)
+    corrupt = np.zeros(n, dtype=bool)
+    if corrupt_every:
+        corrupt[corrupt_at % corrupt_every::corrupt_every] = True
+    idx = np.arange(n) % m
+    pis, _ = engine.g1_mul_batch(np.tile(g1gen, (n, 1)), _fr_matrix([(qs[k] + int(b)) % R_ORDER for k, b in zip(idx, corrupt)]))
+    zy = np.concatenate([_fr_matrix(zs), _fr_matrix(ys)], axis=1)
+    return {"tau_g2": tg[0], "blobs": blobs[idx], "proofs": np.concatenate([cpts[idx], pis], axis=1), "zy": zy[idx],
+            "expect": corrupt.astype(np.uint8)}
