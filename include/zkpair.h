@@ -371,6 +371,54 @@ int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *
                                 const uint8_t *d_proof_inf, size_t n, uint8_t *d_status, uint64_t *d_out_zy, void *d_scratch,
                                 void *stream);
 
+/* ---- EIP-4844 commitments and proofs (one status per blob) ---------------------------------------
+ * blob_to_kzg_commitment, compute_kzg_proof and compute_blob_kzg_proof of the consensus specs (deneb
+ * polynomial-commitments.md) on the GPU.  A commitment is C = sum_i p_i L_brp(i) over the blob's elements p_i and the
+ * setup's Lagrange points in bit-reversed order; a proof is pi = sum_i q_i L_brp(i) over the quotient
+ * q_i = (p_i - y) / (omega_i - z) of compute_kzg_proof_impl (for z = omega_m, q_m is compute_quotient_eval_within_domain
+ * and y = p_m).  Points leave as canonical affine limbs x|y with an infinity flag; the identity is (0, 1) with the flag
+ * set.  Statuses are ZKP_KZG_*: ZKP_KZG_VALID (0) when the point was computed, ZKP_KZG_BAD_SCALAR when a blob element
+ * (or z) is >= r, ZKP_KZG_BAD_POINT when the commitment given to compute_blob_kzg_proof is non-canonical, off the curve
+ * or not torsion free (precedes BAD_SCALAR).  A rejected slot holds zero limbs with its flag set (and y = 0); the call
+ * returns ZKP_OK.  The host path streams double-buffered chunks of at most 2^14 blobs per device, like
+ * zkp_kzg_verify_blob_batch; a proof chunk also holds its 4096 quotient scalars per blob (128 KiB), so a large proof
+ * batch takes up to 2 x 4 GiB of device buffers per device (commitments 2 x 2 GiB), plus the resident setup. */
+
+/* zkp_kzg_setup_create plus the 4096 G1 Lagrange points of the trusted setup, g1_lagrange = 4096 x 12 u64 (canonical
+ * x|y, no infinity flags) in the natural order of the setup file, L_k = [l_k(tau)]G1 at omega^k; the library applies
+ * the bit-reversal permutation itself.  Every point is validated on the GPU (a limb >= p gives ZKP_ERR_NONCANONICAL; an
+ * off-curve or non-subgroup point ZKP_ERR_INVALID_ARG, the message naming its index), and the points are checked
+ * against tau_g2 with one MSM and one pairing check: sum_k L_k = G1 and e(sum_k omega^k L_k, G2) = e(G1, [tau]G2).
+ * A mismatch (a wrong order, a wrong tau, a truncated file) gives ZKP_ERR_INVALID_ARG "g1_lagrange is inconsistent
+ * with tau_g2".  The setup verifies exactly as one from zkp_kzg_setup_create; it also holds, on every device of ctx,
+ * signed-digit window tables of the Lagrange points: 4096 x 32 windows x 128 affine points, 1 610 612 736 bytes
+ * (1.5 GiB) per device on top of the verifier's 1.0 MiB.  Creation takes about 400 MiB of temporary device memory. */
+int32_t zkp_kzg_setup_create_prover(zkp_ctx *ctx, const uint64_t *tau_g2, const uint64_t *g1_lagrange, zkp_kzg_setup **out);
+/* n blobs (n x ZKP_BLOB_BYTES) -> commitments out_c (n x 12 u64), out_c_inf (n), out_status (n).  The prover calls fail
+ * with ZKP_ERR_INVALID_ARG on a setup made without Lagrange points. */
+int32_t zkp_kzg_blob_to_commitment_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint64_t *out_c,
+                                         uint8_t *out_c_inf, uint8_t *out_status);
+/* n blobs and evaluation points z (n x 4 u64, Fr limbs) -> proofs (n x 12 u64, flags), y = p(z) (n x 4 u64) and statuses. */
+int32_t zkp_kzg_compute_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *z, size_t n,
+                                    uint64_t *out_proof, uint8_t *out_proof_inf, uint64_t *out_y, uint8_t *out_status);
+/* n blobs and their commitments (n x 12 u64, commitment_inf n flags or NULL) -> proofs (n x 12 u64, flags) and statuses;
+ * z is the transcript's challenge, as in zkp_kzg_verify_blob_batch.  out_zy (optional, n x 8 u64) receives z | y in the
+ * convention of zkp_kzg_verify_blob_batch. */
+int32_t zkp_kzg_compute_blob_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *commitments,
+                                         const uint8_t *commitment_inf, size_t n, uint64_t *out_proof, uint8_t *out_proof_inf,
+                                         uint8_t *out_status, uint64_t *out_zy);
+/* Bytes of d_scratch the two proof _dev forms need for n blobs (the quotient rows, then z | y); commitments need none. */
+size_t zkp_kzg_prover_scratch_bytes(size_t n);
+/* Device-resident forms on device `dev` of the setup's context; asynchronous, same buffer layouts; d_blobs and
+ * d_scratch 16-byte aligned; stream NULL = the legacy default stream. */
+int32_t zkp_kzg_blob_to_commitment_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
+                                       uint64_t *d_c, uint8_t *d_c_inf, uint8_t *d_status, void *stream);
+int32_t zkp_kzg_compute_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_z, size_t n,
+                                  uint64_t *d_proof, uint8_t *d_proof_inf, uint64_t *d_y, uint8_t *d_status, void *d_scratch, void *stream);
+int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_commitments,
+                                       const uint8_t *d_commitment_inf, size_t n, uint64_t *d_proof, uint8_t *d_proof_inf, uint8_t *d_status,
+                                       uint64_t *d_out_zy, void *d_scratch, void *stream);
+
 /* ---- measurement helpers -------------------------------------------------------------------- */
 
 /* Integer-multiply roofline probe: runs independent IMAD.WIDE.U32 (kind 0), IMAD lo (kind 1) or

@@ -76,6 +76,19 @@ SYMBOLS = {
     "zkp_kzg_blob_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
     "zkp_kzg_verify_blob_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t,
                                                  c_u8p, c_u64p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_kzg_setup_create_prover": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u64p, ctypes.POINTER(ctypes.c_void_p)]),
+    "zkp_kzg_blob_to_commitment_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u64p, c_u8p, c_u8p]),
+    "zkp_kzg_compute_proof_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p, c_u64p,
+                                                     c_u8p]),
+    "zkp_kzg_compute_blob_proof_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t, c_u64p,
+                                                          c_u8p, c_u8p, c_u64p]),
+    "zkp_kzg_prover_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
+    "zkp_kzg_blob_to_commitment_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u64p, c_u8p,
+                                                        c_u8p, ctypes.c_void_p]),
+    "zkp_kzg_compute_proof_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p,
+                                                   c_u8p, c_u64p, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_kzg_compute_blob_proof_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t,
+                                                        c_u64p, c_u8p, c_u8p, c_u64p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_imad_peak": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(ctypes.c_double)]),
     "zkp_launch_count": (ctypes.c_uint64, [ctypes.c_void_p]),
     "zkp_set_kernel_timing": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32]),

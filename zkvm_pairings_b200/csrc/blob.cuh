@@ -211,8 +211,11 @@ ZKP_HD void blob_tree_inv(Fr *tr, int k) {
 }
 // Step 5, thread t: back-substitution from its leaf, 1/d_i = acc * pre[k - 1], acc *= d_i, and its partial sum of
 // p_i omega_i / (z - omega_i), which replaces its leaf.  p_i enters canonical and omega_i and 1/d_i Montgomery, so
-// each product p_i omega_i (1/d_i) comes out canonical: the conversion of p_i costs nothing.
-ZKP_HD void blob_eval_terms(int t, const uint8_t *blob, const Fr *roots, const Fr &zm, BlobShared &sh, const BlobLane &ln) {
+// each product p_i omega_i (1/d_i) comes out canonical: the conversion of p_i costs nothing.  ROW: 1/d_i is also
+// stored at row[i] (the prover's quotient, kzg_prove.cuh).
+template <bool ROW = false>
+ZKP_HD void blob_eval_terms(int t, const uint8_t *blob, const Fr *roots, const Fr &zm, BlobShared &sh, const BlobLane &ln,
+                            Fr *row = nullptr) {
     Fr acc = sh.tree[ZKP_BLOB_TPB + t], sum = fr_zero();
     bool bad = false;
 #pragma unroll
@@ -227,6 +230,7 @@ ZKP_HD void blob_eval_terms(int t, const uint8_t *blob, const Fr *roots, const F
             sh.pj = p;
         }
         const Fr inv = k ? fr_mul(acc, ln.pre[k - 1]) : acc;
+        if (ROW) row[i] = inv;
         if (k) acc = fr_mul(acc, fr_select(fr_is_zero(d), fr_one(), d));
         sum = fr_add(sum, fr_mul(fr_mul(p, w), inv));
     }

@@ -48,11 +48,12 @@ ZKP_NOINLINE void jac_add(Jac<O> &r, const Jac<O> &p, const Jac<O> &q) {
     r.x = x3; r.y = y3; r.z = z3;
 }
 
-// Window table of ONE (IC_j, window w), built by one thread: entry d - 1 = d 2^(8w) IC_j for d = 1..255,
-// affine.  A Jacobian chain P, 2P, .., 255P from P = 2^(8w) IC_j (8w doublings, one inversion), then
-// Montgomery's trick over the chain's Z.  IC_j is a validated subgroup point, so no entry is the
-// identity (d 2^(8w) < r is never a multiple of the prime r).  zs / pre: scratch of 255 Fp each.
-ZKP_HD void groth16_window_table(const uint64_t *ic_xy, int w, Fp *out, Fp *zs, Fp *pre) {
+// Window table of ONE (IC_j, window w), built by one thread: entry d - 1 = d 2^(8w) IC_j for d = 1..digits
+// (255, or 128 for the signed digits of kzg_prove.cuh), affine.  A Jacobian chain P, 2P, .., digits P from
+// P = 2^(8w) IC_j (8w doublings, one inversion), then Montgomery's trick over the chain's Z.  IC_j is a
+// validated subgroup point, so no entry is the identity (d 2^(8w) < r is never a multiple of the prime r).
+// zs / pre: scratch of `digits` Fp each.
+ZKP_HD void groth16_window_table(const uint64_t *ic_xy, int w, Fp *out, Fp *zs, Fp *pre, int digits = ZKP_G16_DIGITS) {
     bool bad = false;
     Jac<OpsFp> p;
     p.x = load_fp(ic_xy, bad);
@@ -63,14 +64,14 @@ ZKP_HD void groth16_window_table(const uint64_t *ic_xy, int w, Fp *out, Fp *zs, 
     Fp px = fmul(p.x, zi2), py = fmul(p.y, fmul(zi2, zi));
     Jac<OpsFp> e;
     e.x = px; e.y = py; e.z = fp_one();
-    for (int d = 0; d < ZKP_G16_DIGITS; d++) {
+    for (int d = 0; d < digits; d++) {
         if (d) jac_add_affine(e, e, px, py);
         out[2 * d] = e.x;
         out[2 * d + 1] = e.y;
         zs[d] = e.z;
     }
-    fp_batch_inv(zs, pre, ZKP_G16_DIGITS);
-    for (int d = 0; d < ZKP_G16_DIGITS; d++) {
+    fp_batch_inv(zs, pre, digits);
+    for (int d = 0; d < digits; d++) {
         Fp z2 = fsqr(zs[d]);
         out[2 * d] = fmul(out[2 * d], z2);
         out[2 * d + 1] = fmul(out[2 * d + 1], fmul(z2, zs[d]));

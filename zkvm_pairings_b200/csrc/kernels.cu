@@ -29,6 +29,7 @@
 #include "groth16.cuh"
 #include "kzg.cuh"
 #include "blob.cuh"
+#include "kzg_prove.cuh"
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -247,6 +248,114 @@ k_blob_eval(const uint8_t *__restrict__ blobs, const Fr *__restrict__ roots, uin
         __syncthreads();
     }
     if (t == 0) blob_eval_finish(sh, zm, o);
+}
+
+// ---- EIP-4844 prover (kzg_prove.cuh)
+
+// Signed-digit window tables of the Lagrange points of bases [first, first + count): one THREAD per (base, window).
+// Table i holds L_brp(i) (lag = the points in the setup file's natural order); scratch: 2 * ZKP_MSM_DIGITS Fp per thread.
+__global__ void __launch_bounds__(ZKP_TPB)
+k_kzg_lagrange_tables(const uint64_t *__restrict__ lag, int first, int count, Fp *__restrict__ tables, Fp *__restrict__ scratch) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= count * ZKP_MSM_WINDOWS) return;
+    const int i = first + t / ZKP_MSM_WINDOWS, w = t % ZKP_MSM_WINDOWS;
+    Fp *zs = scratch + (size_t)t * 2 * ZKP_MSM_DIGITS;
+    groth16_window_table(lag + 12 * blob_brp(i), w, tables + (size_t)i * ZKP_MSM_TABLE_FP + (size_t)w * ZKP_MSM_DIGITS * 2, zs,
+                         zs + ZKP_MSM_DIGITS, ZKP_MSM_DIGITS);
+}
+
+// The setup's consistency rows: row 0 all ones (sum_k L_k) and row 1 roots_brp (sum_k omega^k L_k), big-endian
+__global__ void k_kzg_check_rows(const Fr *__restrict__ roots, uint8_t *__restrict__ rows) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ZKP_BLOB_N) return;
+    Fr one = fr_zero();
+    one.l[0] = 1;
+    store_be32(rows + 32 * i, one);
+    store_be32(rows + ZKP_BLOB_BYTES_ + 32 * i, fr_from_mont(roots[i]));
+}
+
+#ifndef ZKP_MSM_MIN_BLOCKS
+#define ZKP_MSM_MIN_BLOCKS 2   // resident k_kzg_msm blocks per SM: 128 registers, 16 % faster than one (profiles/r3d_kzg_msm_bounds.txt)
+#endif
+
+// sum_i s_i L_brp(i) for every scalar row (4096 x 32 big-endian bytes): one block per row, thread t owning the bases
+// t + 256 k; a row with pre[b] != 0 is already rejected.  status may alias pre.
+__global__ void __launch_bounds__(ZKP_MSM_TPB, ZKP_MSM_MIN_BLOCKS)
+k_kzg_msm(const Fp *__restrict__ tables, const uint8_t *__restrict__ rows, const uint8_t *pre, uint64_t *__restrict__ out,
+          uint8_t *__restrict__ out_inf, uint8_t *status) {
+    __shared__ MsmShared sh;
+    const int t = threadIdx.x;
+    const size_t b = blockIdx.x;
+    const uint8_t p = pre ? pre[b] : 0;
+    if (t == 0) msm_init(sh);
+    __syncthreads();
+    msm_partial(t, tables, rows + b * ZKP_BLOB_BYTES_, p != 0, sh);
+    __syncthreads();
+    for (int w = ZKP_MSM_TPB / 2; w >= 1; w >>= 1) {
+        if (t < w) msm_tree_add(sh, t, w);
+        __syncthreads();
+    }
+    if (t == 0) status[b] = msm_finish(sh, p, out + 12 * b, out_inf + b);
+}
+
+// compute_blob_kzg_proof's front: C's check and z, one thread per blob (commitments = n x 12 u64)
+__global__ void __launch_bounds__(ZKP_BLOB_CHALLENGE_TPB)
+k_kzg_prove_challenge(const uint8_t *__restrict__ blobs, const uint64_t *__restrict__ c, const uint8_t *__restrict__ cinf, size_t n,
+                      uint64_t *__restrict__ zy, uint8_t *__restrict__ status) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    status[i] = prove_challenge_one(blobs + i * ZKP_BLOB_BYTES_, c + 12 * i, cinf ? cinf[i] : 0, zy + 8 * i);
+}
+
+// The quotient row of every blob (compute_kzg_proof_impl): y = p(z) by k_blob_eval's steps, then q_i in place of the
+// inverses 1/(z - omega_i) that step 5 leaves in the row.  z from z_in (n x 4) or, when z_in is NULL, already in zy;
+// y also to y_out (optional, n x 4; 0 for a rejected blob).  pre (may alias status): earlier rejections, or NULL.
+__global__ void __launch_bounds__(ZKP_BLOB_TPB)
+k_kzg_quotient(const uint8_t *__restrict__ blobs, const Fr *__restrict__ roots, const uint64_t *__restrict__ z_in, uint64_t *__restrict__ zy,
+               uint64_t *__restrict__ y_out, uint8_t *__restrict__ rows, const uint8_t *pre, uint8_t *status) {
+    __shared__ QuotShared sh;
+    const int t = threadIdx.x;
+    const size_t b = blockIdx.x;
+    const uint8_t *blob = blobs + b * ZKP_BLOB_BYTES_;
+    uint8_t *row = rows + b * ZKP_BLOB_BYTES_;
+    uint64_t *o = zy + 8 * b;
+    const uint8_t p = pre ? pre[b] : 0;
+    BlobLane ln;
+    if (t == 0) quot_init(sh, z_in ? z_in + 4 * b : nullptr, o);
+    __syncthreads();
+    const Fr zm = sh.zm;
+    blob_eval_prefix(t, roots, zm, sh.b, ln);
+    __syncthreads();
+    for (int w = ZKP_BLOB_TPB / 2; w >= 1; w >>= 1) {
+        if (t < w) blob_tree_mul(sh.b.tree, w + t);
+        __syncthreads();
+    }
+    if (t == 0) blob_tree_invert_root(sh.b.tree);
+    __syncthreads();
+    for (int w = 1; w < ZKP_BLOB_TPB; w <<= 1) {
+        if (t < w) blob_tree_inv(sh.b.tree, w + t);
+        __syncthreads();
+    }
+    blob_eval_terms<true>(t, blob, roots, zm, sh.b, ln, (Fr *)row);
+    __syncthreads();
+    for (int w = ZKP_BLOB_TPB / 2; w >= 1; w >>= 1) {
+        if (t < w) blob_tree_add(sh.b.tree, w + t);
+        __syncthreads();
+    }
+    if (t == 0) {
+        blob_eval_finish(sh.b, zm, o);
+        status[b] = quot_status(sh, p, o, y_out ? y_out + 4 * b : nullptr);
+    }
+    __syncthreads();
+    quot_terms(t, blob, roots, sh, row);
+    __syncthreads();
+    if (sh.b.hit) {   // z = omega_m: one more sum for the entry m
+        for (int w = ZKP_BLOB_TPB / 2; w >= 1; w >>= 1) {
+            if (t < w) blob_tree_add(sh.b.tree, w + t);
+            __syncthreads();
+        }
+        if (t == 0) quot_within_domain(sh, row);
+    }
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -582,9 +691,11 @@ struct KzgDev {   // one device's copy of a setup, in one allocation
     const Fp *prep = nullptr;    // prepared tables of G2 and -[tau]G2
     const Fp *table = nullptr;   // window table of G1 (ZKP_G16_TABLE_FP)
     const Fr *roots = nullptr;   // the blob domain roots_brp (ZKP_BLOB_N Fr, Montgomery)
+    void *lag_mem = nullptr;     // prover setups only: the signed-digit window tables of L_brp(0) .. L_brp(4095)
 };
 struct zkp_kzg_setup {
     zkp_ctx *ctx = nullptr;
+    bool prover = false;        // made by zkp_kzg_setup_create_prover
     std::vector<KzgDev> devs;   // one per device of ctx, same order
 };
 
@@ -653,6 +764,41 @@ static cudaError_t launch_kzg_blob(zkp_ctx *ctx, DevState &d, const KzgDev &k, c
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     return launch_kzg(ctx, d, k, proofs, proof_inf, zy, n, status, (uint8_t *)scratch + blob_zy_bytes(n), err, st);
+}
+
+// ---- EIP-4844 prover: commitments by k_kzg_msm over the blobs, proofs by k_kzg_quotient then k_kzg_msm over the rows
+
+// scratch of one batch of n proofs: the quotient rows (n x ZKP_BLOB_BYTES), then z | y (n x 64 bytes)
+static size_t prove_rows_bytes(size_t n) { return align256(n * ZKP_BLOB_BYTES); }
+extern "C" size_t zkp_kzg_prover_scratch_bytes(size_t n) { return prove_rows_bytes(n) + align256(n * 64); }
+
+static cudaError_t launch_kzg_commit(zkp_ctx *ctx, const KzgDev &k, const uint8_t *blobs, size_t n, uint64_t *out, uint8_t *out_inf,
+                                     uint8_t *status, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    k_kzg_msm<<<(unsigned)n, ZKP_MSM_TPB, 0, st>>>((const Fp *)k.lag_mem, blobs, nullptr, out, out_inf, status);
+    ctx->launches++;
+    return cudaGetLastError();
+}
+
+// z != NULL: compute_kzg_proof at z (n x 4), y to y_out.  z == NULL: compute_blob_kzg_proof for the commitments c
+// (n x 12, flags cinf or NULL), z | y to zy (optional).
+static cudaError_t launch_kzg_prove(zkp_ctx *ctx, const KzgDev &k, const uint8_t *blobs, const uint64_t *z, const uint64_t *c,
+                                    const uint8_t *cinf, size_t n, uint64_t *out, uint8_t *out_inf, uint64_t *y_out, uint64_t *zy,
+                                    uint8_t *status, void *scratch, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    uint8_t *rows = (uint8_t *)scratch;
+    if (!zy) zy = (uint64_t *)(rows + prove_rows_bytes(n));
+    const uint8_t *pre = nullptr;
+    if (!z) {
+        k_kzg_prove_challenge<<<(unsigned)((n + ZKP_BLOB_CHALLENGE_TPB - 1) / ZKP_BLOB_CHALLENGE_TPB), ZKP_BLOB_CHALLENGE_TPB, 0, st>>>(
+            blobs, c, cinf, n, zy, status);
+        ctx->launches++;
+        pre = status;
+    }
+    k_kzg_quotient<<<(unsigned)n, ZKP_BLOB_TPB, 0, st>>>(blobs, k.roots, z, zy, y_out, rows, pre, status);
+    k_kzg_msm<<<(unsigned)n, ZKP_MSM_TPB, 0, st>>>((const Fp *)k.lag_mem, rows, status, out, out_inf, status);
+    ctx->launches += 2;
+    return cudaGetLastError();
 }
 
 extern "C" {
@@ -903,6 +1049,8 @@ struct HostJob {
     const zkp_groth16_vk *vk = nullptr;   // mode 80 = Groth16 verification (proofs in pts, their flags in g1inf, inputs in scalars)
     const zkp_kzg_setup *kzg = nullptr;   // mode 96 = KZG verification (proofs in pts, their flags in g1inf, z | y in scalars)
     const uint8_t *blobs = nullptr;       // mode 112 = KZG blob verification (setup in kzg, proofs in pts, flags in g1inf, z | y out in out)
+    // modes 128 / 144 / 160 = commitments / proofs at z (z in scalars, y out in out) / blob proofs (commitments in pts, their
+    // flags in g1inf, z | y out in out): blobs in blobs, the points out in og1 / og1inf, the statuses in flags
 };
 
 // Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
@@ -921,7 +1069,7 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
     CUS(cudaStreamSynchronize(d.stream[0]));
     int na = 0, nb = 0, nr = 0;
     if (j.mode == 16) tower_op_shape(j.op, na, nb, nr);
-    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : j.mode == 112 ? (size_t)ZKP_BLOB_CHUNK : (size_t)ZKP_CHUNK;
+    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : j.mode >= 112 ? (size_t)ZKP_BLOB_CHUNK : (size_t)ZKP_CHUNK;
     int s = 0;
     cudaStream_t st = nullptr;
     d.pend[0].clear();   // (a job that failed half-way leaves nothing behind for the next one)
@@ -1096,6 +1244,46 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
                                 B[B_OUT].p, d.d_err, st));
             CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
             if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, B[B_OUT].p, cn * 64));   // z | y, first in the scratch
+        } else if (j.mode >= 128) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
+            CUS(B[B_G2].ensure(cn * 96));
+            CUS(B[B_G2INF].ensure(cn));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
+            uint64_t *dout = (uint64_t *)B[B_G2].p;
+            uint8_t *dinf = (uint8_t *)B[B_G2INF].p, *dst = (uint8_t *)B[B_FLAG].p;
+            if (j.mode == 128) {
+                CUS(launch_kzg_commit(ctx, kd, (const uint8_t *)B[B_IN].p, cn, dout, dinf, dst, st));
+            } else {
+                CUS(B[B_OUT].ensure(zkp_kzg_prover_scratch_bytes(cn)));
+                uint64_t *dzy = (uint64_t *)((uint8_t *)B[B_OUT].p + prove_rows_bytes(cn));   // z | y, after the rows
+                const uint64_t *dz = nullptr, *dc = nullptr;
+                const uint8_t *dci = nullptr;
+                uint64_t *dy = nullptr;
+                if (j.mode == 144) {
+                    CUS(B[B_G1].ensure(cn * 32));
+                    CUS(B[B_TAB].ensure(cn * 32));
+                    CUS(h2d(B_G1, B[B_G1].p, j.scalars + c0 * 4, cn * 32));
+                    dz = (const uint64_t *)B[B_G1].p;
+                    dy = (uint64_t *)B[B_TAB].p;
+                } else {
+                    CUS(B[B_G1].ensure(cn * 96));
+                    CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 12, cn * 96));
+                    dc = (const uint64_t *)B[B_G1].p;
+                    if (j.g1inf) {
+                        CUS(B[B_G1INF].ensure(cn));
+                        CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
+                        dci = (const uint8_t *)B[B_G1INF].p;
+                    }
+                }
+                CUS(launch_kzg_prove(ctx, kd, (const uint8_t *)B[B_IN].p, dz, dc, dci, cn, dout, dinf, dy, dzy, dst, B[B_OUT].p, st));
+                if (j.mode == 144) CUS(d2h(B_TAB, j.out + c0 * 4, dy, cn * 32));
+                else if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, dzy, cn * 64));
+            }
+            CUS(d2h(B_G2, j.og1 + c0 * 12, dout, cn * 96));
+            CUS(d2h(B_G2INF, j.og1inf + c0, dinf, cn));
+            CUS(d2h(B_FLAG, j.flags + c0, dst, cn));
         } else if (j.mode == 96) {
             const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
             const uint8_t *dpi = nullptr;
@@ -1625,7 +1813,54 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
 
 // ---- KZG point-evaluation verification
 
-int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup **out) {
+// Lagrange tables of a prover setup on one device, and the consistency check of the points against [tau]G1: one MSM
+// of two rows, sum_k L_k (must be G1) and sum_k omega^k L_k (= [tau]G1), then e(S1, G2) e(G1, -[tau]G2) == 1 on the
+// setup's prepared tables.  *consistent receives the verdict.  tmp holds G1 at byte offset 96 (k_kzg_generators).
+static cudaError_t kzg_lagrange_build(zkp_ctx *ctx, DevState &d, KzgDev &k, const uint64_t *g1_lagrange, const uint8_t *tmp,
+                                      bool *consistent) {
+    const size_t slice = 1024;   // bases per table launch: 32 768 threads, 384 MiB of chain scratch
+    const size_t t_lag = 0, t_rows = align256((size_t)ZKP_BLOB_N * 96), t_pts = t_rows + 2 * ZKP_BLOB_BYTES, t_inf = t_pts + 512,
+                 t_gt = t_inf + 256, t_ws = t_gt + 1024;
+    const size_t tmp_b = t_ws + slice * ZKP_MSM_WINDOWS * 2 * ZKP_MSM_DIGITS * sizeof(Fp);
+    cudaStream_t st = d.stream[0];
+    void *scratch = nullptr;
+    cudaError_t e = cudaMalloc(&k.lag_mem, (size_t)ZKP_BLOB_N * ZKP_MSM_TABLE_FP * sizeof(Fp));
+    if (e == cudaSuccess) e = cudaMalloc(&scratch, tmp_b);
+    if (e == cudaSuccess) {
+        uint8_t *t = (uint8_t *)scratch;
+        uint64_t *pts = (uint64_t *)(t + t_pts);   // S0 | S1 | G1
+        uint8_t *inf = t + t_inf;                  // their flags | the two statuses | is_one
+        e = cudaMemcpyAsync(t + t_lag, g1_lagrange, (size_t)ZKP_BLOB_N * 96, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(inf, 0, 8, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(pts + 24, tmp + 96, 96, cudaMemcpyDeviceToDevice, st);
+        for (size_t f = 0; f < ZKP_BLOB_N && e == cudaSuccess; f += slice) {
+            k_kzg_lagrange_tables<<<(unsigned)(slice * ZKP_MSM_WINDOWS / ZKP_TPB), ZKP_TPB, 0, st>>>(
+                (const uint64_t *)(t + t_lag), (int)f, (int)slice, (Fp *)k.lag_mem, (Fp *)(t + t_ws));
+            ctx->launches++;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) {
+            k_kzg_check_rows<<<ZKP_BLOB_N / 128, 128, 0, st>>>(k.roots, t + t_rows);
+            k_kzg_msm<<<2, ZKP_MSM_TPB, 0, st>>>((const Fp *)k.lag_mem, t + t_rows, nullptr, pts, inf, inf + 4);
+            ctx->launches += 2;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess)
+            e = launch_pairing(ctx, d, 3, pts + 12, inf + 1, nullptr, nullptr, 1, 2, nullptr, (uint64_t *)(t + t_gt), inf + 7, nullptr, st,
+                               k.prep, nullptr, 2);
+        uint64_t h[36];
+        uint8_t hf[8];
+        if (e == cudaSuccess) e = cudaMemcpyAsync(h, pts, sizeof h, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(hf, inf, sizeof hf, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) *consistent = !hf[0] && !memcmp(h, h + 24, 96) && hf[7] == 1;
+    }
+    if (scratch) cudaFree(scratch);
+    return e;
+}
+
+// zkp_kzg_setup_create, and with g1_lagrange (4096 points, natural order) zkp_kzg_setup_create_prover
+static int32_t kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, const uint64_t *g1_lagrange, zkp_kzg_setup **out) {
     if (!out) return fail(ZKP_ERR_INVALID_ARG, "out is NULL");
     *out = nullptr;
     if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
@@ -1634,12 +1869,22 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
     int32_t rc = zkp_g2_check_batch(ctx, tau_g2, nullptr, 1, &st2);   // validated on the GPU
     if (rc != ZKP_OK) return rc;
     if (st2) return fail(ZKP_ERR_INVALID_ARG, std::string("tau_g2 ") + g16_point_error(st2));
+    if (g1_lagrange) {   // every Lagrange point, validated on the GPU
+        std::vector<uint8_t> st1(ZKP_BLOB_N);
+        rc = zkp_g1_check_batch(ctx, g1_lagrange, nullptr, ZKP_BLOB_N, st1.data());
+        if (rc == ZKP_ERR_NONCANONICAL) return fail(rc, "g1_lagrange has a limb >= p (non-canonical field element)");
+        if (rc != ZKP_OK) return rc;
+        for (int i = 0; i < ZKP_BLOB_N; i++)
+            if (st1[i]) return fail(ZKP_ERR_INVALID_ARG, "g1_lagrange[" + std::to_string(i) + "] " + g16_point_error(st1[i]));
+    }
 
     std::lock_guard<std::mutex> lk(ctx->mu);
     DeviceGuard guard;
     zkp_kzg_setup *s = new zkp_kzg_setup();
     s->ctx = ctx;
+    s->prover = g1_lagrange != nullptr;
     s->devs.resize(ctx->devs.size());
+    bool consistent = true;
     const size_t prep_b = align256(2 * (size_t)ZKP_G2_PREPARED_U64 * 8), tab_b = align256((size_t)ZKP_G16_TABLE_FP * sizeof(Fp));
     const size_t roots_b = (size_t)ZKP_BLOB_N * sizeof(Fr);
     // temporary layout: IC_0 = 0 | IC_1 = G1 (the window-table kernel's key layout, one table) | their two flags | G2 |
@@ -1647,7 +1892,7 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
     const size_t t_inf = 256, t_g2 = 512, t_tau = 768, t_ws = 1024;
     const size_t tmp_b = t_ws + (size_t)ZKP_G16_WINDOWS * 2 * ZKP_G16_DIGITS * sizeof(Fp);
     cudaError_t e = cudaSuccess;
-    for (size_t di = 0; di < ctx->devs.size() && e == cudaSuccess; di++) {
+    for (size_t di = 0; di < ctx->devs.size() && e == cudaSuccess && consistent; di++) {
         DevState &d = ctx->devs[di];
         KzgDev &k = s->devs[di];
         k.id = d.id;
@@ -1675,6 +1920,7 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
                 e = cudaGetLastError();
             }
             if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+            if (e == cudaSuccess && g1_lagrange) e = kzg_lagrange_build(ctx, d, k, g1_lagrange, t, &consistent);
         }
         if (tmp) cudaFree(tmp);
     }
@@ -1683,17 +1929,34 @@ int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup
         zkp_kzg_setup_destroy(s);
         return fail(ZKP_ERR_CUDA, msg);
     }
+    if (!consistent) {
+        zkp_kzg_setup_destroy(s);
+        return fail(ZKP_ERR_INVALID_ARG, "g1_lagrange is inconsistent with tau_g2");
+    }
     *out = s;
     return ZKP_OK;
+}
+
+int32_t zkp_kzg_setup_create(zkp_ctx *ctx, const uint64_t *tau_g2, zkp_kzg_setup **out) {
+    return kzg_setup_create(ctx, tau_g2, nullptr, out);
+}
+
+int32_t zkp_kzg_setup_create_prover(zkp_ctx *ctx, const uint64_t *tau_g2, const uint64_t *g1_lagrange, zkp_kzg_setup **out) {
+    if (!g1_lagrange) {
+        if (out) *out = nullptr;
+        return fail(ZKP_ERR_INVALID_ARG, "g1_lagrange is NULL");
+    }
+    return kzg_setup_create(ctx, tau_g2, g1_lagrange, out);
 }
 
 void zkp_kzg_setup_destroy(zkp_kzg_setup *s) {
     if (!s) return;
     DeviceGuard guard;
     for (KzgDev &k : s->devs) {
-        if (!k.mem) continue;
+        if (!k.mem && !k.lag_mem) continue;
         cudaSetDevice(k.id);
-        cudaFree(k.mem);
+        if (k.mem) cudaFree(k.mem);
+        if (k.lag_mem) cudaFree(k.lag_mem);
     }
     delete s;
 }
@@ -1753,6 +2016,98 @@ int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *
     CU(cudaSetDevice(d.id));
     cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
     CU(launch_kzg_blob(ctx, d, s->devs[dev], d_blobs, d_proofs, d_proof_inf, n, d_status, d_out_zy, d_scratch, nullptr, st));
+    return ZKP_OK;
+}
+
+// ---- EIP-4844 prover
+
+static int32_t check_prover(zkp_ctx *ctx, const zkp_kzg_setup *s) {
+    if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (!s->prover) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup has no Lagrange points (create it with zkp_kzg_setup_create_prover)");
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_blob_to_commitment_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint64_t *out_c,
+                                         uint8_t *out_c_inf, uint8_t *out_status) {
+    int32_t rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!blobs || !out_c || !out_c_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 128; j.kzg = s; j.blobs = blobs; j.og1 = out_c; j.og1inf = out_c_inf; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_compute_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *z, size_t n,
+                                    uint64_t *out_proof, uint8_t *out_proof_inf, uint64_t *out_y, uint8_t *out_status) {
+    int32_t rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!blobs || !z || !out_proof || !out_proof_inf || !out_y || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 144; j.kzg = s; j.blobs = blobs; j.scalars = z; j.og1 = out_proof; j.og1inf = out_proof_inf; j.out = out_y;
+    j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_compute_blob_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *commitments,
+                                         const uint8_t *commitment_inf, size_t n, uint64_t *out_proof, uint8_t *out_proof_inf,
+                                         uint8_t *out_status, uint64_t *out_zy) {
+    int32_t rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!blobs || !commitments || !out_proof || !out_proof_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 160; j.kzg = s; j.blobs = blobs; j.pts = commitments; j.g1inf = commitment_inf; j.og1 = out_proof; j.og1inf = out_proof_inf;
+    j.flags = out_status; j.out = out_zy;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_blob_to_commitment_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
+                                       uint64_t *d_c, uint8_t *d_c_inf, uint8_t *d_status, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_blobs || !d_c || !d_c_inf || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if ((uintptr_t)d_blobs & 15) return fail(ZKP_ERR_INVALID_ARG, "d_blobs must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    CU(launch_kzg_commit(ctx, s->devs[dev], d_blobs, n, d_c, d_c_inf, d_status, (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_compute_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_z, size_t n,
+                                  uint64_t *d_proof, uint8_t *d_proof_inf, uint64_t *d_y, uint8_t *d_status, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_blobs || !d_z || !d_proof || !d_proof_inf || !d_y || !d_status || !d_scratch))
+        return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, d_z, nullptr, nullptr, n, d_proof, d_proof_inf, d_y, nullptr, d_status, d_scratch,
+                        (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_commitments,
+                                       const uint8_t *d_commitment_inf, size_t n, uint64_t *d_proof, uint8_t *d_proof_inf, uint8_t *d_status,
+                                       uint64_t *d_out_zy, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_prover(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_blobs || !d_commitments || !d_proof || !d_proof_inf || !d_status || !d_scratch))
+        return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, nullptr, d_commitments, d_commitment_inf, n, d_proof, d_proof_inf, nullptr, d_out_zy,
+                        d_status, d_scratch, (cudaStream_t)stream));
     return ZKP_OK;
 }
 

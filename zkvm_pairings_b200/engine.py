@@ -41,7 +41,8 @@ GROTH16_MAX_PUBLIC = 256
 # per-proof verdicts of kzg_verify_batch / kzg_verify_dev (include/zkpair.h ZKP_KZG_*)
 KZG_VALID, KZG_INVALID, KZG_BAD_POINT, KZG_BAD_SCALAR = 0, 1, 2, 3
 KZG_PROOF_U64 = 24
-BLOB_BYTES = 32 * 4096   # one EIP-4844 blob: 4096 big-endian field elements (include/zkpair.h ZKP_BLOB_BYTES)
+BLOB_N = 4096            # EIP-4844 FIELD_ELEMENTS_PER_BLOB (include/zkpair.h ZKP_BLOB_FIELD_ELEMENTS)
+BLOB_BYTES = 32 * BLOB_N   # one EIP-4844 blob: 4096 big-endian field elements (include/zkpair.h ZKP_BLOB_BYTES)
 
 
 class ZkpError(RuntimeError):
@@ -383,12 +384,18 @@ class PairingEngine:
                                                      n, _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ KZG point-evaluation verification
-    def kzg_setup(self, tau_g2) -> KzgSetup:
+    def kzg_setup(self, tau_g2, g1_lagrange=None) -> KzgSetup:
         """[tau]G2 (24,) -> a setup validated and resident on the GPU.  Raises NonCanonicalError for a limb >= p,
-        ZkpError (INVALID_ARG) for an off-curve or non-subgroup point."""
+        ZkpError (INVALID_ARG) for an off-curve or non-subgroup point.  With g1_lagrange, the 4096 G1 Lagrange points of
+        the trusted setup (4096, 12) in the setup file's natural order, the setup can also prove (kzg_blob_to_commitment_batch,
+        kzg_compute_proof_batch, kzg_compute_blob_proof_batch); points inconsistent with tau_g2 raise ZkpError."""
         t = np.ascontiguousarray(tau_g2, dtype=np.uint64).reshape(24)
         h = ctypes.c_void_p()
-        self._check(self._lib.zkp_kzg_setup_create(self._ctx, _ptr(t), ctypes.byref(h)))
+        if g1_lagrange is None:
+            self._check(self._lib.zkp_kzg_setup_create(self._ctx, _ptr(t), ctypes.byref(h)))
+        else:
+            lag = np.ascontiguousarray(g1_lagrange, dtype=np.uint64).reshape(BLOB_N * 12)
+            self._check(self._lib.zkp_kzg_setup_create_prover(self._ctx, _ptr(t), _ptr(lag), ctypes.byref(h)))
         return KzgSetup(self, h)
 
     def kzg_verify_batch(self, setup: KzgSetup, proofs, zy, proof_inf=None):
@@ -432,6 +439,60 @@ class PairingEngine:
         and d_scratch 16-byte aligned."""
         self._check(self._lib.zkp_kzg_verify_blob_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), _dptr(d_proofs), _dptr(d_proof_inf), n,
                                                       _dptr(d_status), _dptr(d_out_zy), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
+    # ------------------------------------------------------------------ EIP-4844 commitments and proofs
+    def kzg_blob_to_commitment_batch(self, setup: KzgSetup, blobs):
+        """blobs (n, BLOB_BYTES) -> (C (n, 12), C_inf (n,), status (n,)) (blob_to_kzg_commitment; KZG_BAD_SCALAR for an
+        element >= r, with a zeroed slot)."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        c, ci, st = np.zeros((n, 12), np.uint64), np.zeros(n, np.uint8), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_blob_to_commitment_batch(self._ctx, setup.handle, _ptr(b), n, _ptr(c), _ptr(ci), _ptr(st)))
+        return c, ci, st
+
+    def kzg_compute_proof_batch(self, setup: KzgSetup, blobs, z):
+        """blobs (n, BLOB_BYTES), z (n, 4) Fr limbs -> (pi (n, 12), pi_inf (n,), y (n, 4), status (n,)) (compute_kzg_proof)."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        zz = np.ascontiguousarray(z, dtype=np.uint64).reshape(n, 4)
+        pr, pi, y, st = np.zeros((n, 12), np.uint64), np.zeros(n, np.uint8), np.zeros((n, 4), np.uint64), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_compute_proof_batch(self._ctx, setup.handle, _ptr(b), _ptr(zz), n, _ptr(pr), _ptr(pi), _ptr(y), _ptr(st)))
+        return pr, pi, y, st
+
+    def kzg_compute_blob_proof_batch(self, setup: KzgSetup, blobs, commitments, commitment_inf=None, return_zy: bool = False):
+        """blobs (n, BLOB_BYTES), commitments (n, 12), commitment_inf (n,) or None -> (pi (n, 12), pi_inf (n,), status (n,))
+        (compute_blob_kzg_proof), with return_zy also z | y (n, 8) as kzg_verify_blob_batch returns them."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        c = np.ascontiguousarray(commitments, dtype=np.uint64).reshape(n, 12)
+        ci = _np8(commitment_inf, n)
+        pr, pi, st = np.zeros((n, 12), np.uint64), np.zeros(n, np.uint8), np.zeros(n, np.uint8)
+        zy = np.zeros((n, 8), np.uint64) if return_zy else None
+        self._check(self._lib.zkp_kzg_compute_blob_proof_batch(self._ctx, setup.handle, _ptr(b), _ptr(c), _ptr(ci), n, _ptr(pr), _ptr(pi),
+                                                               _ptr(st), _ptr(zy)))
+        return (pr, pi, st, zy) if return_zy else (pr, pi, st)
+
+    def kzg_prover_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_kzg_prover_scratch_bytes(n))
+
+    def kzg_blob_to_commitment_dev(self, setup: KzgSetup, d_blobs, n: int, d_c, d_c_inf, d_status, stream: int = 0, dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_blobs 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_blob_to_commitment_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), n, _dptr(d_c), _dptr(d_c_inf),
+                                                             _dptr(d_status), ctypes.c_void_p(stream)))
+
+    def kzg_compute_proof_dev(self, setup: KzgSetup, d_blobs, d_z, n: int, d_proof, d_proof_inf, d_y, d_status, d_scratch, stream: int = 0,
+                              dev: int = 0):
+        """Asynchronous form; d_scratch holds kzg_prover_scratch_bytes(n) bytes, d_blobs and d_scratch 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_compute_proof_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), _dptr(d_z), n, _dptr(d_proof),
+                                                        _dptr(d_proof_inf), _dptr(d_y), _dptr(d_status), _dptr(d_scratch),
+                                                        ctypes.c_void_p(stream)))
+
+    def kzg_compute_blob_proof_dev(self, setup: KzgSetup, d_blobs, d_commitments, n: int, d_proof, d_proof_inf, d_status, d_scratch,
+                                   d_commitment_inf=None, d_out_zy=None, stream: int = 0, dev: int = 0):
+        """Asynchronous form; d_scratch holds kzg_prover_scratch_bytes(n) bytes, d_blobs and d_scratch 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_compute_blob_proof_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), _dptr(d_commitments),
+                                                             _dptr(d_commitment_inf), n, _dptr(d_proof), _dptr(d_proof_inf), _dptr(d_status),
+                                                             _dptr(d_out_zy), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ byte (de)serialisation (SURVEY 8f)
     def fp_from_bytes_batch(self, data):

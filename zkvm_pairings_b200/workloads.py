@@ -204,12 +204,18 @@ BLOB_BYTES = 32 * BLOB_N
 P_BASE = 0x1a0111ea397fe69a4b1ba7b6434bacd764774b84f38512bf6730d2a0f6b0f6241eabfffeb153ffffb9feffffffffaaab
 
 
-def blob_domain():
-    """roots_brp: the 4096th roots of unity of Fr (generator 7^((r - 1) / 4096)) in bit-reversed order."""
+def _roots_of_unity():
+    """The 4096th roots of unity of Fr, omega^k for k = 0 .. 4095 (omega = 7^((r - 1) / 4096))."""
     w = pow(7, (R_ORDER - 1) // BLOB_N, R_ORDER)
     roots = [1] * BLOB_N
     for i in range(1, BLOB_N):
         roots[i] = roots[i - 1] * w % R_ORDER
+    return roots
+
+
+def blob_domain():
+    """roots_brp: the 4096th roots of unity of Fr (generator 7^((r - 1) / 4096)) in bit-reversed order."""
+    roots = _roots_of_unity()
     return [roots[int(format(i, "012b")[::-1], 2)] for i in range(BLOB_N)]
 
 
@@ -223,6 +229,25 @@ def _batch_inv(vals):
         out[i] = inv * pre[i] % R_ORDER
         inv = inv * vals[i] % R_ORDER
     return out
+
+
+def lagrange_at(tau, roots):
+    """The Lagrange basis of the domain `roots` at tau: l_k(tau) = (tau^N - 1) / N * w_k / (tau - w_k), for tau outside
+    the domain."""
+    scale = (pow(tau, BLOB_N, R_ORDER) - 1) * pow(BLOB_N, -1, R_ORDER) % R_ORDER
+    return [scale * w % R_ORDER * i % R_ORDER for w, i in zip(roots, _batch_inv([(tau - w) % R_ORDER for w in roots]))]
+
+
+def kzg_lagrange_setup(engine, seed: int = 0x4844):
+    """A trusted setup from a seeded tau: (tau, [tau]G2 (24,), g1_lagrange (4096, 12)), g1_lagrange in the natural order
+    of a setup file, L_k = [l_k(tau)]G1 at omega^k (engine.g1_mul_batch of the Lagrange coefficients)."""
+    import random
+    rng = random.Random(seed)
+    tau = rng.randrange(1, R_ORDER)
+    g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
+    tg, _ = engine.g2_mul_batch(g2gen[None], _fr_matrix([tau]))
+    lag, _ = engine.g1_mul_batch(np.tile(g1gen, (BLOB_N, 1)), _fr_matrix(lagrange_at(tau, _roots_of_unity())))
+    return tau, tg[0], lag
 
 
 def blob_eval(poly, z, roots):
@@ -272,8 +297,7 @@ def kzg_blob_proofs(engine, n: int, seed: int = 0x4844, distinct: int = 64, corr
     roots = blob_domain()
     g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
     tg, _ = engine.g2_mul_batch(g2gen[None], _fr_matrix([tau]))
-    scale = (pow(tau, BLOB_N, R_ORDER) - 1) * pow(BLOB_N, -1, R_ORDER) % R_ORDER
-    lag = [scale * w % R_ORDER * i % R_ORDER for w, i in zip(roots, _batch_inv([(tau - w) % R_ORDER for w in roots]))]
+    lag = lagrange_at(tau, roots)
     polys = [[rng.randrange(R_ORDER) for _ in range(BLOB_N)] for _ in range(m)]
     blobs = np.frombuffer(b"".join(v.to_bytes(32, "big") for p in polys for v in p), dtype=np.uint8).reshape(m, BLOB_BYTES)
     cs = [sum(p * l for p, l in zip(poly, lag)) % R_ORDER for poly in polys]
