@@ -10,8 +10,11 @@
 // even lane's Fp at u64 12 j and the odd lane's at 12 j + 6 (six u64 = the twelve 32-bit words of Fp, low first).
 // Fp-level bodies run lane-locally, so each element carries two independent Fp cases (one per lane); an FpW value
 // takes two consecutive slots (low half, high half).  Fp6 / Fp12 operands are consecutive Fp2 slots in struct order.
+// Fr-level bodies (fr.cuh, and the byte paths of blob.cuh / kzg_prove.cuh) also run lane-locally and read and write the
+// low 256 bits of the lane's Fp in a slot (eight words, low first); the bits above stay zero in the results.
 #pragma once
 #include "../../zkvm_pairings_b200/csrc/ops.cuh"
+#include "../../zkvm_pairings_b200/csrc/kzg_prove.cuh"
 
 #define BODY_SLOTS 16
 #define BODY_U64 (12 * BODY_SLOTS)
@@ -57,6 +60,17 @@ enum Body {
     B_FP12_MUL_BY_014_INPLACE,
     B_FP12_CYC_SQR,       // r0..5 = fp12_cyclotomic_sqr(x0..5)
     B_FP12_INV,           // r0..5 = 1 / (x0..5)
+    // Fr level, per lane: x_j / r_j = the low 256 bits of this lane's Fp in slot j
+    B_FR_ADD = 64,        // r0 = fr_add(x0, x1)
+    B_FR_SUB,             // r0 = fr_sub(x0, x1)
+    B_FR_MUL,             // r0 = fr_mul(x0, x1)
+    B_FR_REDUCE_ONCE,     // r0 = fr_reduce_once(x0)
+    B_FR_GEQ_R,           // r0 = fr_geq_r(x0) (0 / 1)
+    B_FR_TO_MONT,         // r0 = fr_to_mont(x0)
+    B_FR_FROM_MONT,       // r0 = fr_from_mont(x0)
+    B_FR_INV,             // r0 = fr_inv(x0)
+    B_BLOB_ELEMENT,       // r0 = the element, r1 = ok (0 / 1): blob_element of x0 as 32 big-endian bytes
+    B_STORE_BE32,         // r0 = the 32 bytes store_be32 writes for x0, in memory order
 };
 
 ZKP_HD Fp raw_fp(const uint64_t *s) {
@@ -83,6 +97,16 @@ ZKP_HD void split_w(Fp &lo, Fp &hi, const FpW &t) {
         lo.l[i] = t.l[i];
         hi.l[i] = t.l[ZKP_NL + i];
     }
+}
+ZKP_HD Fr low_fr(const Fp &a) {
+    Fr r;
+    for (int i = 0; i < ZKP_FR_NL; i++) r.l[i] = a.l[i];
+    return r;
+}
+ZKP_HD Fp fr_slot(const Fr &a) {
+    Fp r = fp_zero();
+    for (int i = 0; i < ZKP_FR_NL; i++) r.l[i] = a.l[i];
+    return r;
 }
 
 // One element, executed by a lane pair (both lanes make the same calls).  `live` = store the result (tail lanes of
@@ -146,6 +170,34 @@ ZKP_HD void body_one(int body, const uint64_t *in, uint64_t *out, bool live) {
         } break;
         case B_FP12_CYC_SQR: fp12_cyclotomic_sqr(r12[0], x12[0]); break;
         case B_FP12_INV: fp12_inv(r12[0], x12[0]); break;
+        case B_FR_ADD: r[0].c = fr_slot(fr_add(low_fr(x[0].c), low_fr(x[1].c))); break;
+        case B_FR_SUB: r[0].c = fr_slot(fr_sub(low_fr(x[0].c), low_fr(x[1].c))); break;
+        case B_FR_MUL: r[0].c = fr_slot(fr_mul(low_fr(x[0].c), low_fr(x[1].c))); break;
+        case B_FR_REDUCE_ONCE: r[0].c = fr_slot(fr_reduce_once(low_fr(x[0].c))); break;
+        case B_FR_GEQ_R: r[0].c.l[0] = fr_geq_r(low_fr(x[0].c)) ? 1u : 0u; break;
+        case B_FR_TO_MONT: r[0].c = fr_slot(fr_to_mont(low_fr(x[0].c))); break;
+        case B_FR_FROM_MONT: r[0].c = fr_slot(fr_from_mont(low_fr(x[0].c))); break;
+        case B_FR_INV: r[0].c = fr_slot(fr_inv(low_fr(x[0].c))); break;
+        case B_BLOB_ELEMENT: {
+            // element 1 of a 16-byte aligned two-element row, as blob_element reads a blob (uint4 loads on the device)
+            alignas(16) uint8_t row[64];
+            const Fr v = low_fr(x[0].c);
+            for (int k = 0; k < 32; k++) {
+                row[k] = 0;
+                row[63 - k] = (uint8_t)(v.l[k >> 2] >> (8 * (k & 3)));
+            }
+            Fr e;
+            const bool ok = blob_element(row, 1, e);
+            r[0].c = fr_slot(e);
+            r[1].c.l[0] = ok ? 1u : 0u;
+        } break;
+        case B_STORE_BE32: {
+            alignas(16) uint8_t row[32];
+            store_be32(row, low_fr(x[0].c));
+            for (int k = 0; k < 8; k++)
+                r[0].c.l[k] = (uint32_t)row[4 * k] | ((uint32_t)row[4 * k + 1] << 8) | ((uint32_t)row[4 * k + 2] << 16) |
+                              ((uint32_t)row[4 * k + 3] << 24);
+        } break;
         default: break;
     }
     if (live)

@@ -12,6 +12,13 @@ the last of them: the internal value 3 * 2^379 makes its last swap in iteration 
 Canonical 3/32 and 1/16 load as exactly these values (R = 2^384), so the worst cases are reachable through the C ABI
 too; those rows go through zkp_tower_op_batch and the simulation.
 
+Fr (fr.cuh) keeps every value in [0, r) (4r > 2^256 rules out a redundant form), so its bodies run at the corners of
+that range: 0, 1, 2, r - 1, r - 2, the long carry patterns, and sums of exactly r and 2r - 2; the range checks
+(fr_geq_r, fr_reduce_once, blob_element) also at r, r + 1, 2r - 1 and 2^256 - 1.  fr_inv runs a fixed 2 * 255 - 1
+iterations: the internal value 3 * 2^253 (canonical 3/8) makes its last swap in iteration 508.  blob_element and
+store_be32 read and write bytes through uint4 and __byte_perm on the device and through byte loops in the
+simulation, so their device words are compared with the simulation's too.
+
 Last, the multi-pairing entry points at every check width 1..8 and the prepared-table path at (pairs, prepared)
 combinations the other tests do not use, with points at infinity in the first, the last and every pair of a check."""
 import ctypes
@@ -32,7 +39,8 @@ import util
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "zkvm_pairings_b200", "csrc")
 HARNESS_DIR = os.path.join(ROOT, "tests", "device_harness")
-HEADERS = [os.path.join(CSRC, f) for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh")]
+HEADERS = [os.path.join(CSRC, f) for f in ("fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "consts.cuh", "fr.cuh", "blob.cuh",
+                                           "kzg.cuh", "groth16.cuh", "kzg_prove.cuh")]
 
 P = pyref.P
 R = 1 << 384
@@ -232,10 +240,11 @@ def fp_body_cases(rng):
 INV_EDGE_REPS = [1 << 380, 3 << 379, (1 << 380) + P, (3 << 379) + P, 1 << 379, 0, P, 2 * P]
 
 
-def gcd_trace(y):
-    """tower.cuh fp_inv's loop for y = the representative reduced mod p: (iterations until a = 0, the iteration of
-    the last swap).  v, the result, changes only in swap iterations, so the loop count must reach the last swap."""
-    a, b, it, last = y, P, 0, 0
+def gcd_trace(y, m=P):
+    """tower.cuh fp_inv's loop (fr.cuh fr_inv's for m = r) for y = the representative reduced mod m: (iterations until
+    a = 0, the iteration of the last swap).  v, the result, changes only in swap iterations, so the loop count must
+    reach the last swap."""
+    a, b, it, last = y, m, 0, 0
     while a:
         it += 1
         if a & 1:
@@ -563,6 +572,105 @@ def test_sim_tower_bodies_at_the_vertices(coracle, lazy):
         check_tower(name, run_sim(sim, name, vals), tower_expected(coracle, name, vals, n), n)
 
 
+# ---------------------------------------------------------------- Fr bodies (fr.cuh, the byte paths of blob.cuh / kzg_prove.cuh)
+
+FR = 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001
+FR_MONT = 1 << 256
+FR_MINV = pow(FR_MONT, -1, FR)
+W256 = FR_MONT - 1
+
+# internal values whose inversion runs fr_inv's full 2 * 255 - 1 iterations (canonical 3/8 and 1/4), and neighbours
+FR_INV_EDGE = [3 << 253, 1 << 254, 1 << 253, (3 << 253) - 1, (3 << 253) + 1, (1 << 254) - 1, (1 << 254) + 1,
+               (1 << 253) - 1, (1 << 253) + 1, 0, 1, FR - 1]
+
+
+def fr_operand_set():
+    """0, 1, 2, r - 2, r - 1, 2^32k - 1 below r, and the top word of r minus one with all ones below"""
+    s = {0, 1, 2, FR - 2, FR - 1, (((FR >> 224) - 1) << 224) | ((1 << 224) - 1)}
+    s |= {(1 << (32 * k)) - 1 for k in range(1, 8)}
+    return sorted(x for x in s if x < FR)
+
+
+def fr_body_cases(rng):
+    """body -> list of operand tuples: the corners and seeded random values of each body's input range"""
+    s = fr_operand_set()
+    rr = lambda: rng.randrange(FR)
+    wide = s + [FR, FR + 1, 2 * FR - 2, 2 * FR - 1, W256, 1 << 255, W256 - (1 << 32)]
+    pairs = [(a, b) for a in s for b in s]
+    pairs += [(a, FR - a) for a in s if a] + [(FR - 1, FR - 1)]          # sums of exactly r and 2r - 2
+    pairs += [(a, FR - a) for a in (rr() for _ in range(50))] + [(a, a) for a in (rr() for _ in range(50))]
+    pairs += [(rr(), rr()) for _ in range(N_RANDOM)]
+    cases = {"fr_add": pairs, "fr_sub": list(pairs), "fr_mul": list(pairs)}
+    cases["fr_reduce_once"] = [(a,) for a in sorted(set(s + [FR + a for a in s] + [2 * FR - 1]))] + \
+        [(rng.randrange(2 * FR),) for _ in range(N_RANDOM)]
+    cases["fr_geq_r"] = [(a,) for a in wide] + [(rng.getrandbits(256),) for _ in range(N_RANDOM)]
+    cases["blob_element"] = list(cases["fr_geq_r"])
+    cases["fr_to_mont"] = [(a,) for a in s] + [(rr(),) for _ in range(N_RANDOM)]
+    cases["fr_from_mont"] = list(cases["fr_to_mont"])
+    cases["fr_inv"] = [(a,) for a in FR_INV_EDGE + s] + [(rr(),) for _ in range(200)]
+    cases["store_be32"] = [(a,) for a in s] + [(rr(),) for _ in range(N_RANDOM)]
+    return cases
+
+
+def check_fr_body(name, case, res):
+    """the reference of one Fr-level case; the words above the low 256 bits of every result must stay zero"""
+    a = case[0]
+    o = res[0]
+    msg = (name, [hex(x) for x in case], [hex(x) for x in res[:2]])
+    assert o >> 256 == 0 and res[1] >> 256 == 0, msg
+    if name == "fr_add":
+        assert o == (a + case[1]) % FR, msg
+    elif name == "fr_sub":
+        assert o == (a - case[1]) % FR, msg
+    elif name == "fr_mul":
+        assert o == a * case[1] * FR_MINV % FR, msg
+    elif name == "fr_reduce_once":
+        assert o == (a - FR if a >= FR else a), msg
+    elif name == "fr_geq_r":
+        assert o == (1 if a >= FR else 0), msg
+    elif name == "fr_to_mont":
+        assert o == a * FR_MONT % FR, msg
+    elif name == "fr_from_mont":
+        assert o == a * FR_MINV % FR, msg
+    elif name == "fr_inv":
+        assert o == (0 if a == 0 else FR_MONT * FR_MONT * pow(a, -1, FR) % FR), msg
+    elif name == "blob_element":
+        assert (o, res[1]) == ((a, 1) if a < FR else (0, 0)), msg
+    elif name == "store_be32":
+        assert o.to_bytes(48, "little")[:32] == a.to_bytes(32, "big"), msg
+    else:
+        raise KeyError(name)
+
+
+def check_fr_bodies(runner, lib):
+    """every Fr body's cases through runner (run_sim / run_dev) against the references; returns {body: (values, out)}"""
+    done = {}
+    for name, cs in fr_body_cases(random.Random(0xF4)).items():
+        vals = fp_cases(cs)
+        out = runner(lib, name, vals)
+        for c, r in zip(cs, fp_results(out, len(cs))):
+            check_fr_body(name, c, r)
+        done[name] = (vals, out)
+    return done
+
+
+def test_fr_inv_iteration_count_is_tight():
+    """The Python model of fr_inv's loop: the fixed count 2 * 255 - 1 is reached, 3 * 2^253 swaps in its last
+    iteration but one, and canonical 3/8 and 1/4 load as 3 * 2^253 and 2^254 (RF = 2^256); random inputs stop
+    swapping long before, so only the edge values notice a shorter loop."""
+    assert 2 * 255 - 1 == 509
+    assert gcd_trace(3 << 253, FR) == (509, 508) and gcd_trace(1 << 254, FR) == (509, 255)
+    assert 3 * pow(8, -1, FR) * FR_MONT % FR == 3 << 253 and pow(4, -1, FR) * FR_MONT % FR == 1 << 254
+    rng = random.Random(0x1F4)
+    assert max(gcd_trace(rng.randrange(1, FR), FR)[1] for _ in range(2000)) < 450
+
+
+def test_sim_fr_bodies_at_the_bounds():
+    """Fr bodies of the simulation (which asserts the operand bound of every sum, difference and product) at the
+    corners of their input ranges: Python big-int references."""
+    check_fr_bodies(run_sim, build_sim(0))
+
+
 # ---------------------------------------------------------------- GPU: the device builds
 
 @pytest.fixture(scope="module", params=VARIANTS)
@@ -630,6 +738,15 @@ def test_device_tower_bodies_at_the_vertices(device_variant, coracle):
         check_tower(name, out, expected, n)
         idx, sub = spread(vals, n, SIM_COMPARE)
         assert np.array_equal(out[idx], run_sim(sim, name, sub)), (name_v, name)
+
+
+@pytest.mark.gpu
+def test_device_fr_bodies_at_the_bounds(device_variant):
+    """Fr bodies on the device at the corners of their input ranges: Python big-int references, and every raw output
+    word equal to the simulation's (blob_element and store_be32 take the device's uint4 / __byte_perm paths there)."""
+    name_v, lib, sim = device_variant
+    for name, (vals, out) in check_fr_bodies(run_dev, lib).items():
+        assert np.array_equal(out, run_sim(sim, name, vals)), (name_v, name)
 
 
 # ---------------------------------------------------------------- GPU: the C ABI at its reachable edges
