@@ -419,6 +419,62 @@ int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_
                                        const uint8_t *d_commitment_inf, size_t n, uint64_t *d_proof, uint8_t *d_proof_inf, uint8_t *d_status,
                                        uint64_t *d_out_zy, void *d_scratch, void *stream);
 
+/* ---- EIP-7594 cells and cell proofs (one status per blob or per cell) -----------------------------
+ * compute_cells, compute_cells_and_kzg_proofs and the per-cell check of verify_cell_kzg_proof_batch of the consensus
+ * specs (fulu polynomial-commitments-sampling.md) on the GPU.  The extended blob is the blob's polynomial evaluated over
+ * the 8192nd roots of unity in bit-reversed order, cut into 128 cells of 64 big-endian elements (2048 bytes); cells
+ * 0 .. 63 are the blob's own bytes.  Proof k is [q_k(tau)]G1 over the monomial setup, q_k = p div (X^64 - c_k) with
+ * c_k = h_k^64 and h_k the first point of cell k.  A cell is accepted iff C and pi are canonical, on the curve and
+ * torsion free, every element is < r, the index is < 128 and e(C + [c_k]pi - [I_k(tau)]G1, G2) e(pi, -[tau^64]G2) == 1,
+ * I_k = the cell's interpolation polynomial.  Statuses are ZKP_KZG_*: ZKP_KZG_BAD_SCALAR for a blob or cell element
+ * >= r or a cell index >= 128, ZKP_KZG_BAD_POINT for C or pi (precedes BAD_SCALAR).  The spec's boolean for a batch is
+ * the AND of the cells' statuses being ZKP_KZG_VALID.  A rejected blob's slots hold zero cells and proofs of zero limbs
+ * with the flag set; the calls return ZKP_OK for malformed blobs and cells.
+ * Host paths stream double-buffered chunks per device: at most 2^11 blobs for cells (2 x 768 MiB of device buffers),
+ * 2^7 blobs with proofs (128 quotient rows of 128 KiB per blob: 2 x 2.2 GiB) and 2^16 cells for verification
+ * (2 x 180 MiB), plus the resident setup. */
+#define ZKP_CELLS_PER_EXT_BLOB 128
+#define ZKP_FIELD_ELEMENTS_PER_CELL 64
+#define ZKP_CELL_BYTES (32 * ZKP_FIELD_ELEMENTS_PER_CELL)
+
+/* The EIP-7594 trusted setup: g2_monomial = 65 G2 points [tau^i]G2 (65 x 24 u64), g1_monomial = 4096 G1 points
+ * [tau^i]G1 (4096 x 12 u64) and, optionally, g1_lagrange as for zkp_kzg_setup_create_prover (NULL: the setup cannot run
+ * the EIP-4844 prover calls).  Builds everything zkp_kzg_setup_create builds, with tau_g2 = g2_monomial[1], plus the
+ * prepared table of -[tau^64]G2, the twiddles of the extended domain (256 KiB) and signed-digit window tables of the
+ * monomial points (1.5 GiB per device, like the Lagrange tables).  Every point is validated on the GPU (a limb >= p
+ * gives ZKP_ERR_NONCANONICAL; an off-curve or non-subgroup point ZKP_ERR_INVALID_ARG naming its index); then
+ * g1_monomial[0] must be G1, g2_monomial[0] must be G2, e(M_{i+1}, G2) = e(M_i, g2_monomial[1]) for i < 4095 and
+ * e(M_i, G2) = e(G1, g2_monomial[i]) for i <= 64 (ZKP_ERR_INVALID_ARG naming the first point that fails).  The cells
+ * calls fail with ZKP_ERR_INVALID_ARG on setups made otherwise. */
+int32_t zkp_kzg_setup_create_cells(zkp_ctx *ctx, const uint64_t *g2_monomial, const uint64_t *g1_monomial, const uint64_t *g1_lagrange,
+                                   zkp_kzg_setup **out);
+/* n blobs (n x ZKP_BLOB_BYTES) -> out_cells (n x 128 x ZKP_CELL_BYTES) and out_status (n). */
+int32_t zkp_kzg_compute_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
+                                    uint8_t *out_status);
+/* n blobs -> out_cells, out_proofs (n x 128 x 12 u64), out_proof_inf (n x 128) and out_status (n). */
+int32_t zkp_kzg_compute_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
+                                               uint64_t *out_proofs, uint8_t *out_proof_inf, uint8_t *out_status);
+/* n cells: commitments (n x 12 u64, commitment_inf n flags or NULL), cell_indices (n), cells (n x ZKP_CELL_BYTES),
+ * proofs (n x 12 u64, proof_inf n flags or NULL) -> out_status[i] = ZKP_KZG_*. */
+int32_t zkp_kzg_verify_cell_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *commitments, const uint8_t *commitment_inf,
+                                  const uint64_t *cell_indices, const uint8_t *cells, const uint64_t *proofs, const uint8_t *proof_inf, size_t n,
+                                  uint8_t *out_status);
+/* Bytes of d_scratch zkp_kzg_compute_cells_and_proofs_dev needs for n blobs (coefficients, quotient rows and their
+ * statuses: about 16 MiB per blob); zkp_kzg_compute_cells_dev needs none. */
+size_t zkp_kzg_cells_proofs_scratch_bytes(size_t n);
+/* Bytes of d_scratch zkp_kzg_verify_cell_dev needs for n cells (zkp_kzg_scratch_bytes(n), then [I_k(tau)]G1). */
+size_t zkp_kzg_verify_cell_scratch_bytes(size_t n);
+/* Device-resident forms on device `dev` of the setup's context; asynchronous, same buffer layouts; d_blobs, d_cells and
+ * d_scratch 16-byte aligned; stream NULL = the legacy default stream. */
+int32_t zkp_kzg_compute_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n, uint8_t *d_cells,
+                                  uint8_t *d_status, void *stream);
+int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
+                                             uint8_t *d_cells, uint64_t *d_proofs, uint8_t *d_proof_inf, uint8_t *d_status, void *d_scratch,
+                                             void *stream);
+int32_t zkp_kzg_verify_cell_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_commitments, const uint8_t *d_commitment_inf,
+                                const uint64_t *d_cell_indices, const uint8_t *d_cells, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
+                                size_t n, uint8_t *d_status, void *d_scratch, void *stream);
+
 /* ---- measurement helpers -------------------------------------------------------------------- */
 
 /* Integer-multiply roofline probe: runs independent IMAD.WIDE.U32 (kind 0), IMAD lo (kind 1) or

@@ -89,6 +89,20 @@ SYMBOLS = {
                                                    c_u8p, c_u64p, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_kzg_compute_blob_proof_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t,
                                                         c_u64p, c_u8p, c_u8p, c_u64p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_kzg_setup_create_cells": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u64p, c_u64p, ctypes.POINTER(ctypes.c_void_p)]),
+    "zkp_kzg_compute_cells_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u8p, c_u8p]),
+    "zkp_kzg_compute_cells_and_proofs_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u8p, c_u64p, c_u8p,
+                                                                c_u8p]),
+    "zkp_kzg_verify_cell_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t,
+                                                   c_u8p]),
+    "zkp_kzg_cells_proofs_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
+    "zkp_kzg_verify_cell_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
+    "zkp_kzg_compute_cells_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u8p, c_u8p,
+                                                   ctypes.c_void_p]),
+    "zkp_kzg_compute_cells_and_proofs_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u8p, ctypes.c_size_t, c_u8p,
+                                                              c_u64p, c_u8p, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_kzg_verify_cell_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, c_u8p, c_u64p, c_u8p,
+                                                 ctypes.c_size_t, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_imad_peak": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(ctypes.c_double)]),
     "zkp_launch_count": (ctypes.c_uint64, [ctypes.c_void_p]),
     "zkp_set_kernel_timing": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32]),

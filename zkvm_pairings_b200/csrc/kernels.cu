@@ -30,6 +30,7 @@
 #include "kzg.cuh"
 #include "blob.cuh"
 #include "kzg_prove.cuh"
+#include "kzg_cells.cuh"
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -252,15 +253,17 @@ k_blob_eval(const uint8_t *__restrict__ blobs, const Fr *__restrict__ roots, uin
 
 // ---- EIP-4844 prover (kzg_prove.cuh)
 
-// Signed-digit window tables of the Lagrange points of bases [first, first + count): one THREAD per (base, window).
-// Table i holds L_brp(i) (lag = the points in the setup file's natural order); scratch: 2 * ZKP_MSM_DIGITS Fp per thread.
+// Signed-digit window tables of the setup points of bases [first, first + count): one THREAD per (base, window).
+// permute: table i holds L_brp(i) (lag = the Lagrange points in the setup file's natural order); otherwise point i (the
+// monomial points [tau^i]G1 of a cells setup).  scratch: 2 * ZKP_MSM_DIGITS Fp per thread.
 __global__ void __launch_bounds__(ZKP_TPB)
-k_kzg_lagrange_tables(const uint64_t *__restrict__ lag, int first, int count, Fp *__restrict__ tables, Fp *__restrict__ scratch) {
+k_kzg_lagrange_tables(const uint64_t *__restrict__ lag, int first, int count, bool permute, Fp *__restrict__ tables,
+                      Fp *__restrict__ scratch) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= count * ZKP_MSM_WINDOWS) return;
     const int i = first + t / ZKP_MSM_WINDOWS, w = t % ZKP_MSM_WINDOWS;
     Fp *zs = scratch + (size_t)t * 2 * ZKP_MSM_DIGITS;
-    groth16_window_table(lag + 12 * blob_brp(i), w, tables + (size_t)i * ZKP_MSM_TABLE_FP + (size_t)w * ZKP_MSM_DIGITS * 2, zs,
+    groth16_window_table(lag + 12 * (permute ? blob_brp(i) : i), w, tables + (size_t)i * ZKP_MSM_TABLE_FP + (size_t)w * ZKP_MSM_DIGITS * 2, zs,
                          zs + ZKP_MSM_DIGITS, ZKP_MSM_DIGITS);
 }
 
@@ -356,6 +359,117 @@ k_kzg_quotient(const uint8_t *__restrict__ blobs, const Fr *__restrict__ roots, 
         }
         if (t == 0) quot_within_domain(sh, row);
     }
+}
+
+// ---- EIP-7594 cells (kzg_cells.cuh)
+
+// the cells setup's twiddle table pw[e] = omega_8192^e (Montgomery), one thread per entry
+__global__ void k_cells_powers(Fr *__restrict__ pw) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < ZKP_CELLS_EXT_N) pw[e] = cells_power(e);
+}
+
+// The inputs of the cells setup's pairing checks from the monomial points M_i (mono, 4096 x 12) and G1 (g1, 12):
+// chain[i] = [M_{i+1}, M_i] for i < 4095 (against G2, -[tau]G2), and pairs[i] = [-G1, M_i] for i <= 64 (against
+// g2_monomial[i] in the per-check slot, then G2).  One lane pair per i.
+__global__ void k_cells_setup_pairs(const uint64_t *__restrict__ mono, const uint64_t *__restrict__ g1, uint64_t *__restrict__ chain,
+                                    uint64_t *__restrict__ pairs) {
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= ZKP_BLOB_N - 1) return;
+    const int par = lane_par();
+    copy_u64(chain + 24 * i + 6 * par, mono + 12 * (i + 1) + 6 * par, 6, false);
+    copy_u64(chain + 24 * i + 12 + 6 * par, mono + 12 * i + 6 * par, 6, false);
+    if (i <= ZKP_CELL_N) {
+        bool b = false;
+        const Fp v = load_fp(g1 + 6 * par, b);
+        store_fp(pairs + 24 * i + 6 * par, par ? fp_neg(v) : v, nullptr);
+        copy_u64(pairs + 24 * i + 12 + 6 * par, mono + 12 * i + 6 * par, 6, false);
+    }
+}
+
+// compute_cells: the 128 cells of every blob (n x 256 KiB) and its status; coeffs (n x 4096 Fr, or NULL) receives the
+// blob's coefficients for the proofs.  One block per blob, the blob's 4096 Fr in dynamic shared memory (128 KiB).
+__global__ void __launch_bounds__(ZKP_CELLS_TPB)
+k_cells_extend(const uint8_t *__restrict__ blobs, const Fr *__restrict__ pw, uint8_t *__restrict__ cells, Fr *__restrict__ coeffs,
+               uint8_t *__restrict__ status) {
+    extern __shared__ Fr cells_x[];
+    __shared__ uint32_t bad;
+    const int t = threadIdx.x;
+    const size_t b = blockIdx.x;
+    const uint8_t *blob = blobs + b * ZKP_BLOB_BYTES_;
+    if (t == 0) bad = 0;
+    __syncthreads();
+    cells_load(t, blob, cells_x, &bad);
+    __syncthreads();
+    for (int h = 1; h < ZKP_BLOB_N; h <<= 1) {
+        cells_dit_pass(t, cells_x, pw, h);
+        __syncthreads();
+    }
+    cells_scale(t, cells_x, pw, coeffs ? coeffs + b * ZKP_BLOB_N : nullptr);
+    __syncthreads();
+    for (int h = ZKP_BLOB_N / 2; h >= 1; h >>= 1) {
+        cells_dif_pass(t, cells_x, pw, h);
+        __syncthreads();
+    }
+    cells_store(t, blob, cells_x, bad != 0, cells + b * 2 * ZKP_BLOB_BYTES_);
+    if (t == 0) status[b] = bad ? ZKP_KZG_BAD_SCALAR : ZKP_KZG_VALID;
+}
+
+// The quotient rows of every blob's 128 cosets (n x 128 rows of 4096 x 32 bytes), one thread per (blob, coset, chain);
+// row_status[128 b + k] = status[b], the rejection k_kzg_msm reads for the row
+__global__ void __launch_bounds__(ZKP_CELLS_QUOT_TPB)
+k_cells_quotient(const Fr *__restrict__ coeffs, const Fr *__restrict__ pw, const uint8_t *__restrict__ status, size_t n,
+                 uint8_t *__restrict__ rows, uint8_t *__restrict__ row_status) {
+    const size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N) return;
+    const size_t r = g / ZKP_CELL_N, b = r / ZKP_CELLS_PER_BLOB;
+    const int m = (int)(g % ZKP_CELL_N);
+    const uint8_t st = status[b];
+    if (m == 0) row_status[r] = st;
+    if (st) return;
+    cells_quotient_chain((int)(r % ZKP_CELLS_PER_BLOB), m, coeffs + b * ZKP_BLOB_N, pw, rows + r * ZKP_BLOB_BYTES_);
+}
+
+// The verifier's interpolation, one 64-thread block per cell: I_k from the cell, then [I_k(tau)]G1 over the first 64
+// monomial tables (ixy / iinf), and the status (ZKP_KZG_BAD_SCALAR for an element >= r or an index >= 128)
+__global__ void __launch_bounds__(ZKP_CELL_N)
+k_cells_interp(const uint8_t *__restrict__ cells, const uint64_t *__restrict__ idx, const Fr *__restrict__ pw, const Fp *__restrict__ mono,
+               uint64_t *__restrict__ ixy, uint8_t *__restrict__ iinf, uint8_t *__restrict__ status) {
+    __shared__ CellShared sh;
+    const int t = threadIdx.x;
+    const size_t c = blockIdx.x;
+    const uint64_t k = idx[c];
+    if (t == 0) cell_init(sh, k);
+    __syncthreads();
+    cell_load(t, cells + c * ZKP_CELL_BYTES_, sh);
+    __syncthreads();
+    for (int h = 1; h < ZKP_CELL_N; h <<= 1) {
+        if (t < ZKP_CELL_N / 2) cells_dit(sh.x, pw, t, h);
+        __syncthreads();
+    }
+    cell_interp_scale(t, k, pw, sh);
+    __syncthreads();
+    const uint8_t pre = sh.bad ? ZKP_KZG_BAD_SCALAR : ZKP_KZG_VALID;
+    msm_partial<ZKP_CELL_N>(t, mono, sh.row, pre != 0, sh.msm);
+    __syncthreads();
+    for (int w = ZKP_CELL_N / 2; w >= 1; w >>= 1) {
+        if (t < w) msm_tree_add(sh.msm, t, w);
+        __syncthreads();
+    }
+    if (t == 0) status[c] = msm_finish(sh.msm, pre, ixy + 12 * c, iinf + c);
+}
+
+// The verifier's pairs, one lane pair per cell (cell_prepare_one); status holds k_cells_interp's and is updated
+__global__ void __launch_bounds__(ZKP_TPB, ZKP_MIN_BLOCKS)
+k_cells_prepare(const uint64_t *__restrict__ c, const uint8_t *__restrict__ cinf, const uint64_t *__restrict__ idx,
+                const uint64_t *__restrict__ pi, const uint8_t *__restrict__ piinf, const Fr *__restrict__ pw, const uint64_t *__restrict__ ixy,
+                const uint8_t *__restrict__ iinf, size_t n, uint64_t *__restrict__ g1, uint8_t *__restrict__ g1inf, uint8_t *status) {
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= n) return;
+    const uint8_t pre = status[i];   // both lanes read it before the lane exchanges of cell_prepare_one; the even lane writes last
+    const uint8_t s = cell_prepare_one(c + 12 * i, cinf ? cinf[i] : 0, pi + 12 * i, piinf ? piinf[i] : 0, idx[i], pw, ixy + 12 * i, iinf[i],
+                                       pre, g1 + 24 * i, g1inf + 2 * i);
+    if (lane_par() == 0) status[i] = s;
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -692,10 +806,15 @@ struct KzgDev {   // one device's copy of a setup, in one allocation
     const Fp *table = nullptr;   // window table of G1 (ZKP_G16_TABLE_FP)
     const Fr *roots = nullptr;   // the blob domain roots_brp (ZKP_BLOB_N Fr, Montgomery)
     void *lag_mem = nullptr;     // prover setups only: the signed-digit window tables of L_brp(0) .. L_brp(4095)
+    void *cell_mem = nullptr;    // cells setups only, one allocation of the three below
+    const Fp *cell_prep = nullptr;   // prepared tables of G2 and -[tau^64]G2
+    const Fr *pw = nullptr;          // omega_8192^e, e < 8192 (Montgomery)
+    const Fp *mono = nullptr;        // the signed-digit window tables of [tau^i]G1, i < 4096
 };
 struct zkp_kzg_setup {
     zkp_ctx *ctx = nullptr;
-    bool prover = false;        // made by zkp_kzg_setup_create_prover
+    bool prover = false;        // has Lagrange tables: zkp_kzg_setup_create_prover, or zkp_kzg_setup_create_cells with g1_lagrange
+    bool cells = false;         // made by zkp_kzg_setup_create_cells
     std::vector<KzgDev> devs;   // one per device of ctx, same order
 };
 
@@ -798,6 +917,66 @@ static cudaError_t launch_kzg_prove(zkp_ctx *ctx, const KzgDev &k, const uint8_t
     k_kzg_quotient<<<(unsigned)n, ZKP_BLOB_TPB, 0, st>>>(blobs, k.roots, z, zy, y_out, rows, pre, status);
     k_kzg_msm<<<(unsigned)n, ZKP_MSM_TPB, 0, st>>>((const Fp *)k.lag_mem, rows, status, out, out_inf, status);
     ctx->launches += 2;
+    return cudaGetLastError();
+}
+
+// ---- EIP-7594 cells: k_cells_extend (then k_cells_quotient and k_kzg_msm over the monomial tables for the proofs);
+// verification by k_cells_interp and k_cells_prepare, then the prepared 2-pair check against G2 and -[tau^64]G2
+
+#ifndef ZKP_CELLS_CHUNK
+#define ZKP_CELLS_CHUNK (1u << 11)         // blobs per host chunk of compute_cells: 256 MiB of blobs, 512 MiB of cells per buffer set
+#endif
+#ifndef ZKP_CELL_PROOF_CHUNK
+#define ZKP_CELL_PROOF_CHUNK (1u << 7)     // blobs per host chunk with proofs: 2 GiB of quotient rows per buffer set
+#endif
+#ifndef ZKP_CELL_VERIFY_CHUNK
+#define ZKP_CELL_VERIFY_CHUNK (1u << 16)   // cells per host chunk of verification: 128 MiB of cells per buffer set
+#endif
+
+// scratch of cells and proofs for n blobs: the coefficients (n x 4096 Fr), the quotient rows (n x 128 x ZKP_BLOB_BYTES),
+// the rows' statuses (n x 128)
+static size_t cells_coeff_bytes(size_t n) { return align256(n * ZKP_BLOB_N * sizeof(Fr)); }
+static size_t cells_rows_bytes(size_t n) { return align256(n * ZKP_CELLS_PER_BLOB * ZKP_BLOB_BYTES); }
+extern "C" size_t zkp_kzg_cells_proofs_scratch_bytes(size_t n) {
+    return cells_coeff_bytes(n) + cells_rows_bytes(n) + align256(n * ZKP_CELLS_PER_BLOB);
+}
+// scratch of n cell checks: the point-evaluation pairs, then [I_k(tau)]G1 (n x 96 bytes) and its flags
+extern "C" size_t zkp_kzg_verify_cell_scratch_bytes(size_t n) { return kzg_layout(n, nullptr, nullptr) + align256(n * 96) + align256(n); }
+
+// proofs == NULL: cells only (no scratch)
+static cudaError_t launch_cells(zkp_ctx *ctx, const KzgDev &k, const uint8_t *blobs, size_t n, uint8_t *cells, uint64_t *proofs,
+                                uint8_t *proof_inf, uint8_t *status, void *scratch, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    Fr *coeffs = proofs ? (Fr *)scratch : nullptr;
+    k_cells_extend<<<(unsigned)n, ZKP_CELLS_TPB, ZKP_BLOB_N * sizeof(Fr), st>>>(blobs, k.pw, cells, coeffs, status);
+    ctx->launches++;
+    if (proofs) {
+        uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
+        const size_t nt = n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N;
+        k_cells_quotient<<<(unsigned)((nt + ZKP_CELLS_QUOT_TPB - 1) / ZKP_CELLS_QUOT_TPB), ZKP_CELLS_QUOT_TPB, 0, st>>>(coeffs, k.pw, status, n,
+                                                                                                                    rows, rst);
+        k_kzg_msm<<<(unsigned)(n * ZKP_CELLS_PER_BLOB), ZKP_MSM_TPB, 0, st>>>(k.mono, rows, rst, proofs, proof_inf, rst);
+        ctx->launches += 2;
+    }
+    return cudaGetLastError();
+}
+
+static cudaError_t launch_cells_verify(zkp_ctx *ctx, DevState &d, const KzgDev &k, const uint64_t *c, const uint8_t *cinf, const uint64_t *idx,
+                                       const uint8_t *cells, const uint64_t *pi, const uint8_t *piinf, size_t n, uint8_t *status, void *scratch,
+                                       uint32_t *err, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    KzgScratch s;
+    uint64_t *ixy = (uint64_t *)((uint8_t *)scratch + kzg_layout(n, scratch, &s));
+    uint8_t *iinf = (uint8_t *)ixy + align256(n * 96);
+    k_cells_interp<<<(unsigned)n, ZKP_CELL_N, 0, st>>>(cells, idx, k.pw, k.mono, ixy, iinf, status);
+    k_cells_prepare<<<grid_for(n), ZKP_TPB, 0, st>>>(c, cinf, idx, pi, piinf, k.pw, ixy, iinf, n, s.g1, s.g1inf, status);
+    ctx->launches += 2;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, nullptr, nullptr, n, 2, nullptr, s.gt, s.is_one, err, st, k.cell_prep, nullptr, 2);
+    if (e != cudaSuccess) return e;
+    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
+    ctx->launches++;
     return cudaGetLastError();
 }
 
@@ -1051,6 +1230,11 @@ struct HostJob {
     const uint8_t *blobs = nullptr;       // mode 112 = KZG blob verification (setup in kzg, proofs in pts, flags in g1inf, z | y out in out)
     // modes 128 / 144 / 160 = commitments / proofs at z (z in scalars, y out in out) / blob proofs (commitments in pts, their
     // flags in g1inf, z | y out in out): blobs in blobs, the points out in og1 / og1inf, the statuses in flags
+    // modes 176 / 192 = cells / cells and proofs: blobs in blobs, cells out in ocells, proofs in og1 / og1inf, statuses in flags.
+    // mode 208 = cell verification: commitments in pts (flags in g1inf), indices in idx, cells in cells, proofs in pi (flags in piinf)
+    uint8_t *ocells = nullptr;
+    const uint8_t *cells = nullptr, *piinf = nullptr;
+    const uint64_t *idx = nullptr, *pi = nullptr;
 };
 
 // Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
@@ -1069,7 +1253,12 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
     CUS(cudaStreamSynchronize(d.stream[0]));
     int na = 0, nb = 0, nr = 0;
     if (j.mode == 16) tower_op_shape(j.op, na, nb, nr);
-    size_t chunk = j.mode == 80 ? g16_chunk(j.vk->n_public) : j.mode >= 112 ? (size_t)ZKP_BLOB_CHUNK : (size_t)ZKP_CHUNK;
+    size_t chunk = j.mode == 80    ? g16_chunk(j.vk->n_public)
+                   : j.mode == 176 ? (size_t)ZKP_CELLS_CHUNK
+                   : j.mode == 192 ? (size_t)ZKP_CELL_PROOF_CHUNK
+                   : j.mode == 208 ? (size_t)ZKP_CELL_VERIFY_CHUNK
+                   : j.mode >= 112 ? (size_t)ZKP_BLOB_CHUNK
+                                   : (size_t)ZKP_CHUNK;
     int s = 0;
     cudaStream_t st = nullptr;
     d.pend[0].clear();   // (a job that failed half-way leaves nothing behind for the next one)
@@ -1244,6 +1433,55 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
                                 B[B_OUT].p, d.d_err, st));
             CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
             if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, B[B_OUT].p, cn * 64));   // z | y, first in the scratch
+        } else if (j.mode == 176 || j.mode == 192) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            const size_t cb = (size_t)ZKP_CELLS_PER_EXT_BLOB * ZKP_CELL_BYTES, np = cn * ZKP_CELLS_PER_EXT_BLOB;
+            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
+            CUS(B[B_G1].ensure(cn * cb));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
+            uint64_t *dpf = nullptr;
+            uint8_t *dpi = nullptr;
+            if (j.mode == 192) {
+                CUS(B[B_G2].ensure(np * 96));
+                CUS(B[B_G2INF].ensure(np));
+                CUS(B[B_OUT].ensure(zkp_kzg_cells_proofs_scratch_bytes(cn)));
+                dpf = (uint64_t *)B[B_G2].p;
+                dpi = (uint8_t *)B[B_G2INF].p;
+            }
+            CUS(launch_cells(ctx, kd, (const uint8_t *)B[B_IN].p, cn, (uint8_t *)B[B_G1].p, dpf, dpi, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, st));
+            CUS(d2h(B_G1, j.ocells + c0 * cb, B[B_G1].p, cn * cb));
+            if (j.mode == 192) {
+                CUS(d2h(B_G2, j.og1 + c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 96));
+                CUS(d2h(B_G2INF, j.og1inf + c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np));
+            }
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
+        } else if (j.mode == 208) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            const uint8_t *dci = nullptr, *dpi = nullptr;
+            CUS(B[B_G1].ensure(cn * 96));
+            CUS(B[B_G2].ensure(cn * 96));
+            CUS(B[B_TAB].ensure(cn * 8));
+            CUS(B[B_IN].ensure(cn * ZKP_CELL_BYTES));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(B[B_OUT].ensure(zkp_kzg_verify_cell_scratch_bytes(cn)));
+            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 12, cn * 96));
+            CUS(h2d(B_G2, B[B_G2].p, j.pi + c0 * 12, cn * 96));
+            CUS(h2d(B_TAB, B[B_TAB].p, j.idx + c0, cn * 8));
+            CUS(h2d(B_IN, B[B_IN].p, j.cells + c0 * ZKP_CELL_BYTES, cn * ZKP_CELL_BYTES));
+            if (j.g1inf) {
+                CUS(B[B_G1INF].ensure(cn));
+                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
+                dci = (const uint8_t *)B[B_G1INF].p;
+            }
+            if (j.piinf) {
+                CUS(B[B_G2INF].ensure(cn));
+                CUS(h2d(B_G2INF, B[B_G2INF].p, j.piinf + c0, cn));
+                dpi = (const uint8_t *)B[B_G2INF].p;
+            }
+            CUS(launch_cells_verify(ctx, d, kd, (const uint64_t *)B[B_G1].p, dci, (const uint64_t *)B[B_TAB].p, (const uint8_t *)B[B_IN].p,
+                                    (const uint64_t *)B[B_G2].p, dpi, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
         } else if (j.mode >= 128) {
             const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
             CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
@@ -1835,7 +2073,7 @@ static cudaError_t kzg_lagrange_build(zkp_ctx *ctx, DevState &d, KzgDev &k, cons
         if (e == cudaSuccess) e = cudaMemcpyAsync(pts + 24, tmp + 96, 96, cudaMemcpyDeviceToDevice, st);
         for (size_t f = 0; f < ZKP_BLOB_N && e == cudaSuccess; f += slice) {
             k_kzg_lagrange_tables<<<(unsigned)(slice * ZKP_MSM_WINDOWS / ZKP_TPB), ZKP_TPB, 0, st>>>(
-                (const uint64_t *)(t + t_lag), (int)f, (int)slice, (Fp *)k.lag_mem, (Fp *)(t + t_ws));
+                (const uint64_t *)(t + t_lag), (int)f, (int)slice, true, (Fp *)k.lag_mem, (Fp *)(t + t_ws));
             ctx->launches++;
             e = cudaGetLastError();
         }
@@ -1953,10 +2191,11 @@ void zkp_kzg_setup_destroy(zkp_kzg_setup *s) {
     if (!s) return;
     DeviceGuard guard;
     for (KzgDev &k : s->devs) {
-        if (!k.mem && !k.lag_mem) continue;
+        if (!k.mem && !k.lag_mem && !k.cell_mem) continue;
         cudaSetDevice(k.id);
         if (k.mem) cudaFree(k.mem);
         if (k.lag_mem) cudaFree(k.lag_mem);
+        if (k.cell_mem) cudaFree(k.cell_mem);
     }
     delete s;
 }
@@ -2108,6 +2347,206 @@ int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_
     CU(cudaSetDevice(d.id));
     CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, nullptr, d_commitments, d_commitment_inf, n, d_proof, d_proof_inf, nullptr, d_out_zy,
                         d_status, d_scratch, (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+// ---- EIP-7594 cells
+
+// The cells parts of a setup on one device: the prepared tables of G2 and -[tau^64]G2, the twiddles pw and the window
+// tables of the monomial points, then the checks of the points: g1_monomial[0] = G1, g2_monomial[0] = G2,
+// e(M_{i+1}, G2) e(M_i, -[tau]G2) == 1 for i < 4095 on the setup's prepared tables, and e(-G1, g2_monomial[i])
+// e(M_i, G2) == 1 for i <= 64 with g2_monomial[i] in the per-check slot.  why receives the first failed check.
+static cudaError_t kzg_cells_build(zkp_ctx *ctx, DevState &d, KzgDev &k, const uint64_t *g2_mono, const uint64_t *g1_mono, std::string &why) {
+    const int nc = ZKP_BLOB_N - 1, ng = ZKP_CELL_N + 1;   // chain checks, G2 checks
+    const size_t prep1 = (size_t)ZKP_G2_PREPARED_U64 * 8, slice = 1024;
+    const size_t c_pw = align256(2 * prep1), c_mono = c_pw + align256((size_t)ZKP_CELLS_EXT_N * sizeof(Fr));
+    const size_t cell_b = c_mono + (size_t)ZKP_BLOB_N * ZKP_MSM_TABLE_FP * sizeof(Fp);
+    // temporary layout: monomial points | G2 monomial points | G1 | G2 | chain pairs | G2-check pairs | Gt | is_one | table scratch
+    const size_t t_g2 = align256((size_t)ZKP_BLOB_N * 96), t_gen = t_g2 + align256(ng * 192), t_chain = t_gen + 512,
+                 t_pairs = t_chain + align256((size_t)nc * 192), t_gt = t_pairs + align256(ng * 192), t_one = t_gt + align256((size_t)nc * 576),
+                 t_ws = t_one + align256(nc + ng);
+    const size_t tmp_b = t_ws + slice * ZKP_MSM_WINDOWS * 2 * ZKP_MSM_DIGITS * sizeof(Fp);
+    cudaStream_t st = d.stream[0];
+    void *scratch = nullptr;
+    cudaError_t e = cudaFuncSetAttribute(k_cells_extend, cudaFuncAttributeMaxDynamicSharedMemorySize, ZKP_BLOB_N * sizeof(Fr));
+    if (e == cudaSuccess) e = cudaMalloc(&k.cell_mem, cell_b);
+    if (e == cudaSuccess) e = cudaMalloc(&scratch, tmp_b);
+    if (e == cudaSuccess) {
+        uint8_t *m = (uint8_t *)k.cell_mem, *t = (uint8_t *)scratch;
+        k.cell_prep = (const Fp *)m;
+        k.pw = (const Fr *)(m + c_pw);
+        k.mono = (const Fp *)(m + c_mono);
+        e = cudaMemcpyAsync(t, g1_mono, (size_t)ZKP_BLOB_N * 96, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(t + t_g2, g2_mono, ng * 192, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(m, k.prep, prep1, cudaMemcpyDeviceToDevice, st);   // G2's table
+        if (e == cudaSuccess) {
+            k_g16_neg_prepare<<<grid_for(1), ZKP_TPB, 0, st>>>((const uint64_t *)(t + t_g2) + 24 * ZKP_CELL_N, (Fp *)(m + prep1), 1);
+            k_cells_powers<<<ZKP_CELLS_EXT_N / 128, 128, 0, st>>>((Fr *)k.pw);
+            k_kzg_generators<<<1, 32, 0, st>>>((uint64_t *)(t + t_gen), (uint64_t *)(t + t_gen) + 12);
+            k_cells_setup_pairs<<<grid_for(nc), ZKP_TPB, 0, st>>>((const uint64_t *)t, (const uint64_t *)(t + t_gen), (uint64_t *)(t + t_chain),
+                                                                 (uint64_t *)(t + t_pairs));
+            ctx->launches += 4;
+            e = cudaGetLastError();
+        }
+        for (size_t f = 0; f < ZKP_BLOB_N && e == cudaSuccess; f += slice) {
+            k_kzg_lagrange_tables<<<(unsigned)(slice * ZKP_MSM_WINDOWS / ZKP_TPB), ZKP_TPB, 0, st>>>(
+                (const uint64_t *)t, (int)f, (int)slice, false, (Fp *)k.mono, (Fp *)(t + t_ws));
+            ctx->launches++;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess)
+            e = launch_pairing(ctx, d, 3, (const uint64_t *)(t + t_chain), nullptr, nullptr, nullptr, nc, 2, nullptr, (uint64_t *)(t + t_gt),
+                               t + t_one, nullptr, st, k.prep, nullptr, 2);
+        if (e == cudaSuccess)
+            e = launch_pairing(ctx, d, 3, (const uint64_t *)(t + t_pairs), nullptr, (const uint64_t *)(t + t_g2), nullptr, ng, 2, nullptr,
+                               (uint64_t *)(t + t_gt), t + t_one + nc, nullptr, st, k.prep, nullptr, 1);
+        uint64_t gen[36];
+        std::vector<uint8_t> one(nc + ng);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(gen, t + t_gen, sizeof gen, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(one.data(), t + t_one, one.size(), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e == cudaSuccess) {
+            if (memcmp(g1_mono, gen, 96)) why = "g1_monomial[0] is not the G1 generator";
+            else if (memcmp(g2_mono, gen + 12, 192)) why = "g2_monomial[0] is not the G2 generator";
+            for (int i = 0; i < nc && why.empty(); i++)
+                if (one[i] != 1)
+                    why = "g1_monomial[" + std::to_string(i + 1) + "] is inconsistent with g1_monomial[" + std::to_string(i) + "] and g2_monomial[1]";
+            for (int i = 0; i < ng && why.empty(); i++)
+                if (one[nc + i] != 1) why = "g2_monomial[" + std::to_string(i) + "] is inconsistent with g1_monomial[" + std::to_string(i) + "]";
+        }
+    }
+    if (scratch) cudaFree(scratch);
+    return e;
+}
+
+int32_t zkp_kzg_setup_create_cells(zkp_ctx *ctx, const uint64_t *g2_monomial, const uint64_t *g1_monomial, const uint64_t *g1_lagrange,
+                                   zkp_kzg_setup **out) {
+    if (!out) return fail(ZKP_ERR_INVALID_ARG, "out is NULL");
+    *out = nullptr;
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (!g2_monomial || !g1_monomial) return fail(ZKP_ERR_INVALID_ARG, "g2_monomial or g1_monomial is NULL");
+    std::vector<uint8_t> st2(ZKP_CELL_N + 1), st1(ZKP_BLOB_N);   // every point, validated on the GPU
+    int32_t rc = zkp_g2_check_batch(ctx, g2_monomial, nullptr, st2.size(), st2.data());
+    if (rc == ZKP_ERR_NONCANONICAL) return fail(rc, "g2_monomial has a limb >= p (non-canonical field element)");
+    if (rc != ZKP_OK) return rc;
+    for (size_t i = 0; i < st2.size(); i++)
+        if (st2[i]) return fail(ZKP_ERR_INVALID_ARG, "g2_monomial[" + std::to_string(i) + "] " + g16_point_error(st2[i]));
+    rc = zkp_g1_check_batch(ctx, g1_monomial, nullptr, st1.size(), st1.data());
+    if (rc == ZKP_ERR_NONCANONICAL) return fail(rc, "g1_monomial has a limb >= p (non-canonical field element)");
+    if (rc != ZKP_OK) return rc;
+    for (size_t i = 0; i < st1.size(); i++)
+        if (st1[i]) return fail(ZKP_ERR_INVALID_ARG, "g1_monomial[" + std::to_string(i) + "] " + g16_point_error(st1[i]));
+    zkp_kzg_setup *s = nullptr;
+    rc = kzg_setup_create(ctx, g2_monomial + 24, g1_lagrange, &s);   // tau from g2_monomial[1]
+    if (rc != ZKP_OK) return rc;
+    std::string why;
+    cudaError_t e = cudaSuccess;
+    {
+        std::lock_guard<std::mutex> lk(ctx->mu);
+        DeviceGuard guard;
+        for (size_t di = 0; di < ctx->devs.size() && e == cudaSuccess && why.empty(); di++) {
+            e = cudaSetDevice(ctx->devs[di].id);
+            if (e == cudaSuccess) e = kzg_cells_build(ctx, ctx->devs[di], s->devs[di], g2_monomial, g1_monomial, why);
+        }
+    }
+    if (e != cudaSuccess) {
+        std::string msg = std::string("KZG cells setup failed: ") + cudaGetErrorString(e);
+        zkp_kzg_setup_destroy(s);
+        return fail(ZKP_ERR_CUDA, msg);
+    }
+    if (!why.empty()) {
+        zkp_kzg_setup_destroy(s);
+        return fail(ZKP_ERR_INVALID_ARG, why);
+    }
+    s->cells = true;
+    *out = s;
+    return ZKP_OK;
+}
+
+static int32_t check_cells(zkp_ctx *ctx, const zkp_kzg_setup *s) {
+    if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
+    if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
+    if (!s->cells) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup has no monomial points (create it with zkp_kzg_setup_create_cells)");
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_compute_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
+                                    uint8_t *out_status) {
+    int32_t rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!blobs || !out_cells || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 176; j.kzg = s; j.blobs = blobs; j.ocells = out_cells; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_compute_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
+                                               uint64_t *out_proofs, uint8_t *out_proof_inf, uint8_t *out_status) {
+    int32_t rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!blobs || !out_cells || !out_proofs || !out_proof_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 192; j.kzg = s; j.blobs = blobs; j.ocells = out_cells; j.og1 = out_proofs; j.og1inf = out_proof_inf; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_verify_cell_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *commitments, const uint8_t *commitment_inf,
+                                  const uint64_t *cell_indices, const uint8_t *cells, const uint64_t *proofs, const uint8_t *proof_inf, size_t n,
+                                  uint8_t *out_status) {
+    int32_t rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!commitments || !cell_indices || !cells || !proofs || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 208; j.kzg = s; j.pts = commitments; j.g1inf = commitment_inf; j.idx = cell_indices; j.cells = cells; j.pi = proofs;
+    j.piinf = proof_inf; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_compute_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n, uint8_t *d_cells,
+                                  uint8_t *d_status, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_blobs || !d_cells || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_blobs & 15) || ((uintptr_t)d_cells & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_cells must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    CU(cudaSetDevice(ctx->devs[dev].id));
+    CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, nullptr, nullptr, d_status, nullptr, (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
+                                             uint8_t *d_cells, uint64_t *d_proofs, uint8_t *d_proof_inf, uint8_t *d_status, void *d_scratch,
+                                             void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_blobs || !d_cells || !d_proofs || !d_proof_inf || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_blobs & 15) || ((uintptr_t)d_cells & 15) || ((uintptr_t)d_scratch & 15))
+        return fail(ZKP_ERR_INVALID_ARG, "d_blobs, d_cells and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    CU(cudaSetDevice(ctx->devs[dev].id));
+    CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, d_proofs, d_proof_inf, d_status, d_scratch, (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_verify_cell_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_commitments, const uint8_t *d_commitment_inf,
+                                const uint64_t *d_cell_indices, const uint8_t *d_cells, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
+                                size_t n, uint8_t *d_status, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_cells(ctx, s);
+    if (rc) return rc;
+    if (n && (!d_commitments || !d_cell_indices || !d_cells || !d_proofs || !d_status || !d_scratch))
+        return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_scratch & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_cells and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    CU(launch_cells_verify(ctx, d, s->devs[dev], d_commitments, d_commitment_inf, d_cell_indices, d_cells, d_proofs, d_proof_inf, n, d_status,
+                           d_scratch, nullptr, (cudaStream_t)stream));
     return ZKP_OK;
 }
 

@@ -53,23 +53,29 @@ ZKP_HD void store_be32(uint8_t *p, const Fr &v) {
 
 // ------------------------------------------------------------------ fixed-base MSM over the Lagrange tables
 
-// Shared state of one row's block: each thread's Jacobian partial sum, then the tree of their sums in place.
-struct MsmShared {
-    Jac<OpsFp> acc[ZKP_MSM_TPB];
+// Shared state of one row's block of TPB threads: each thread's Jacobian partial sum, then the tree of their sums in
+// place.  k_kzg_msm runs 256 threads over 4096 bases; the cell verifier (kzg_cells.cuh) 64 threads over 64 bases.
+template <int TPB>
+struct MsmSharedN {
+    Jac<OpsFp> acc[TPB];
     uint32_t bad;    // some scalar >= r
 };
+typedef MsmSharedN<ZKP_MSM_TPB> MsmShared;
 
-ZKP_HD void msm_init(MsmShared &sh) { sh.bad = 0; }
-// Step 1, thread t: sum over the bases i = t + TPB k and every window of d_w 2^(8w) L_brp(i), one table lookup and one
-// mixed addition per non-zero digit, no doubling.  skip = the row is already rejected (the partial stays the identity).
-ZKP_HD void msm_partial(int t, const Fp *tables, const uint8_t *row, bool skip, MsmShared &sh) {
+template <int TPB>
+ZKP_HD void msm_init(MsmSharedN<TPB> &sh) { sh.bad = 0; }
+// Step 1, thread t: sum over the bases i = t + TPB k < NB and every window of d_w 2^(8w) L_brp(i), one table lookup and
+// one mixed addition per non-zero digit, no doubling.  skip = the row is already rejected (the partial stays the
+// identity).  The row holds NB scalars.
+template <int NB = ZKP_BLOB_N, int TPB>
+ZKP_HD void msm_partial(int t, const Fp *tables, const uint8_t *row, bool skip, MsmSharedN<TPB> &sh) {
     Jac<OpsFp> acc;
     acc.x = fp_zero(); acc.y = fp_one(); acc.z = fp_zero();
     bool bad = false;
     if (!skip) {
 #pragma unroll 1
-        for (int k = 0; k < ZKP_BLOB_N / ZKP_MSM_TPB; k++) {
-            const int i = t + ZKP_MSM_TPB * k;
+        for (int k = 0; k < NB / TPB; k++) {
+            const int i = t + TPB * k;
             Fr s;
             bad |= !blob_element(row, i, s);
             const Fp *tb = tables + (size_t)i * ZKP_MSM_TABLE_FP;
@@ -87,11 +93,13 @@ ZKP_HD void msm_partial(int t, const Fp *tables, const uint8_t *row, bool skip, 
     if (bad) sh.bad = 1;
 }
 // Step 2, level by level (t < w, w = TPB/2 .. 1): acc[t] += acc[t + w]
-ZKP_HD void msm_tree_add(MsmShared &sh, int t, int w) { jac_add(sh.acc[t], sh.acc[t], sh.acc[t + w]); }
+template <int TPB>
+ZKP_HD void msm_tree_add(MsmSharedN<TPB> &sh, int t, int w) { jac_add(sh.acc[t], sh.acc[t], sh.acc[t + w]); }
 // Step 3, one thread: the sum as canonical affine limbs and its flag; pre = an earlier rejection of this row (0 none).
 // A rejected row (pre, or a scalar >= r: ZKP_KZG_BAD_SCALAR) gets zero limbs with the flag set; the identity is (0, 1)
 // with the flag set.  Returns the row's status.
-ZKP_HD uint8_t msm_finish(const MsmShared &sh, uint8_t pre, uint64_t *xy, uint8_t *inf) {
+template <int TPB>
+ZKP_HD uint8_t msm_finish(const MsmSharedN<TPB> &sh, uint8_t pre, uint64_t *xy, uint8_t *inf) {
     const uint8_t st = pre ? pre : sh.bad ? ZKP_KZG_BAD_SCALAR : ZKP_KZG_VALID;
     const Jac<OpsFp> &p = sh.acc[0];
     const bool p_inf = fp_is_zero(p.z);

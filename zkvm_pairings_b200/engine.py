@@ -43,6 +43,9 @@ KZG_VALID, KZG_INVALID, KZG_BAD_POINT, KZG_BAD_SCALAR = 0, 1, 2, 3
 KZG_PROOF_U64 = 24
 BLOB_N = 4096            # EIP-4844 FIELD_ELEMENTS_PER_BLOB (include/zkpair.h ZKP_BLOB_FIELD_ELEMENTS)
 BLOB_BYTES = 32 * BLOB_N   # one EIP-4844 blob: 4096 big-endian field elements (include/zkpair.h ZKP_BLOB_BYTES)
+CELLS_PER_EXT_BLOB = 128            # EIP-7594 (include/zkpair.h ZKP_CELLS_PER_EXT_BLOB)
+FIELD_ELEMENTS_PER_CELL = 64        # include/zkpair.h ZKP_FIELD_ELEMENTS_PER_CELL
+CELL_BYTES = 32 * FIELD_ELEMENTS_PER_CELL   # include/zkpair.h ZKP_CELL_BYTES
 
 
 class ZkpError(RuntimeError):
@@ -493,6 +496,78 @@ class PairingEngine:
         self._check(self._lib.zkp_kzg_compute_blob_proof_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), _dptr(d_commitments),
                                                              _dptr(d_commitment_inf), n, _dptr(d_proof), _dptr(d_proof_inf), _dptr(d_status),
                                                              _dptr(d_out_zy), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
+    # ------------------------------------------------------------------ EIP-7594 cells and cell proofs
+    def kzg_setup_cells(self, g2_monomial, g1_monomial, g1_lagrange=None) -> KzgSetup:
+        """The EIP-7594 trusted setup, g2_monomial (65, 24) = [tau^i]G2 and g1_monomial (4096, 12) = [tau^i]G1, validated and
+        resident on the GPU; with g1_lagrange (4096, 12) as for kzg_setup the setup can also run the EIP-4844 prover.  It
+        verifies as kzg_setup(g2_monomial[1]) does.  Raises NonCanonicalError for a limb >= p, ZkpError (INVALID_ARG) for
+        an invalid or inconsistent point, naming it."""
+        g2 = np.ascontiguousarray(g2_monomial, dtype=np.uint64).reshape((FIELD_ELEMENTS_PER_CELL + 1) * 24)
+        g1 = np.ascontiguousarray(g1_monomial, dtype=np.uint64).reshape(BLOB_N * 12)
+        lag = None if g1_lagrange is None else np.ascontiguousarray(g1_lagrange, dtype=np.uint64).reshape(BLOB_N * 12)
+        h = ctypes.c_void_p()
+        self._check(self._lib.zkp_kzg_setup_create_cells(self._ctx, _ptr(g2), _ptr(g1), _ptr(lag), ctypes.byref(h)))
+        return KzgSetup(self, h)
+
+    def kzg_compute_cells_batch(self, setup: KzgSetup, blobs):
+        """blobs (n, BLOB_BYTES) -> (cells (n, 128, CELL_BYTES), status (n,)) (compute_cells; KZG_BAD_SCALAR for an element
+        >= r, with zero cells)."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        cells, st = np.zeros((n, CELLS_PER_EXT_BLOB, CELL_BYTES), np.uint8), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_compute_cells_batch(self._ctx, setup.handle, _ptr(b), n, _ptr(cells), _ptr(st)))
+        return cells, st
+
+    def kzg_compute_cells_and_proofs_batch(self, setup: KzgSetup, blobs):
+        """blobs (n, BLOB_BYTES) -> (cells (n, 128, CELL_BYTES), proofs (n, 128, 12), proof_inf (n, 128), status (n,))
+        (compute_cells_and_kzg_proofs)."""
+        b = np.ascontiguousarray(blobs, dtype=np.uint8).reshape(-1, BLOB_BYTES)
+        n = b.shape[0]
+        cells = np.zeros((n, CELLS_PER_EXT_BLOB, CELL_BYTES), np.uint8)
+        pr, pi, st = np.zeros((n, CELLS_PER_EXT_BLOB, 12), np.uint64), np.zeros((n, CELLS_PER_EXT_BLOB), np.uint8), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_compute_cells_and_proofs_batch(self._ctx, setup.handle, _ptr(b), n, _ptr(cells), _ptr(pr), _ptr(pi),
+                                                                     _ptr(st)))
+        return cells, pr, pi, st
+
+    def kzg_verify_cell_batch(self, setup: KzgSetup, commitments, cell_indices, cells, proofs, commitment_inf=None, proof_inf=None):
+        """Per cell: commitments (n, 12), cell_indices (n,), cells (n, CELL_BYTES), proofs (n, 12), flags (n,) or None ->
+        status (n,) of KZG_* (verify_cell_kzg_proof_batch is the AND of status == KZG_VALID)."""
+        c = np.ascontiguousarray(commitments, dtype=np.uint64).reshape(-1, 12)
+        n = c.shape[0]
+        idx = np.ascontiguousarray(cell_indices, dtype=np.uint64).reshape(n)
+        cl = np.ascontiguousarray(cells, dtype=np.uint8).reshape(n, CELL_BYTES)
+        pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(n, 12)
+        ci, pi = _np8(commitment_inf, n), _np8(proof_inf, n)
+        st = np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_verify_cell_batch(self._ctx, setup.handle, _ptr(c), _ptr(ci), _ptr(idx), _ptr(cl), _ptr(pr), _ptr(pi), n,
+                                                        _ptr(st)))
+        return st
+
+    def kzg_cells_proofs_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_kzg_cells_proofs_scratch_bytes(n))
+
+    def kzg_verify_cell_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_kzg_verify_cell_scratch_bytes(n))
+
+    def kzg_compute_cells_dev(self, setup: KzgSetup, d_blobs, n: int, d_cells, d_status, stream: int = 0, dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_blobs and d_cells 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_compute_cells_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), n, _dptr(d_cells), _dptr(d_status),
+                                                        ctypes.c_void_p(stream)))
+
+    def kzg_compute_cells_and_proofs_dev(self, setup: KzgSetup, d_blobs, n: int, d_cells, d_proofs, d_proof_inf, d_status, d_scratch,
+                                         stream: int = 0, dev: int = 0):
+        """Asynchronous form; d_scratch holds kzg_cells_proofs_scratch_bytes(n) bytes; d_blobs, d_cells, d_scratch 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_compute_cells_and_proofs_dev(self._ctx, dev, setup.handle, _dptr(d_blobs), n, _dptr(d_cells),
+                                                                   _dptr(d_proofs), _dptr(d_proof_inf), _dptr(d_status), _dptr(d_scratch),
+                                                                   ctypes.c_void_p(stream)))
+
+    def kzg_verify_cell_dev(self, setup: KzgSetup, d_commitments, d_cell_indices, d_cells, d_proofs, n: int, d_status, d_scratch,
+                            d_commitment_inf=None, d_proof_inf=None, stream: int = 0, dev: int = 0):
+        """Asynchronous form; d_scratch holds kzg_verify_cell_scratch_bytes(n) bytes; d_cells and d_scratch 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_verify_cell_dev(self._ctx, dev, setup.handle, _dptr(d_commitments), _dptr(d_commitment_inf),
+                                                      _dptr(d_cell_indices), _dptr(d_cells), _dptr(d_proofs), _dptr(d_proof_inf), n,
+                                                      _dptr(d_status), _dptr(d_scratch), ctypes.c_void_p(stream)))
 
     # ------------------------------------------------------------------ byte (de)serialisation (SURVEY 8f)
     def fp_from_bytes_batch(self, data):

@@ -250,6 +250,21 @@ def kzg_lagrange_setup(engine, seed: int = 0x4844):
     return tau, tg[0], lag
 
 
+def kzg_cell_setup(engine, seed: int = 0x7594):
+    """An EIP-7594 trusted setup from a seeded tau: (tau, g2_monomial (65, 24) = [tau^i]G2 for i <= 64, g1_monomial
+    (4096, 12) = [tau^i]G1, g1_lagrange (4096, 12) as kzg_lagrange_setup gives it), by engine.g1_mul_batch /
+    g2_mul_batch of the powers of tau."""
+    import random
+    rng = random.Random(seed)
+    tau = rng.randrange(1, R_ORDER)
+    powers = [pow(tau, i, R_ORDER) for i in range(BLOB_N)]
+    g1gen, g2gen = _fp_row([G1_GEN[0], G1_GEN[1]]), _fp_row([G2_GEN[0][0], G2_GEN[0][1], G2_GEN[1][0], G2_GEN[1][1]])
+    g2m, _ = engine.g2_mul_batch(np.tile(g2gen, (65, 1)), _fr_matrix(powers[:65]))
+    g1m, _ = engine.g1_mul_batch(np.tile(g1gen, (BLOB_N, 1)), _fr_matrix(powers))
+    lag, _ = engine.g1_mul_batch(np.tile(g1gen, (BLOB_N, 1)), _fr_matrix(lagrange_at(tau, _roots_of_unity())))
+    return tau, g2m, g1m, lag
+
+
 def blob_eval(poly, z, roots):
     """The blob's polynomial (values at roots) at z, barycentric (the value itself when z is a root)."""
     if z in roots:
