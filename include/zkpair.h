@@ -321,6 +321,7 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
 #define ZKP_KZG_INVALID 1      /* well formed, the equation fails */
 #define ZKP_KZG_BAD_POINT 2    /* C or pi has a limb >= p, is off the curve or is not torsion free (precedes 3) */
 #define ZKP_KZG_BAD_SCALAR 3   /* z >= r or y >= r */
+#define ZKP_KZG_BAD_CELLS 4    /* cell recovery: a cell count outside [64, 128], indices not strictly ascending or one >= 128 (precedes 3) */
 #define ZKP_KZG_PROOF_U64 24   /* C.x|C.y | pi.x|pi.y */
 
 typedef struct zkp_kzg_setup zkp_kzg_setup;
@@ -474,6 +475,30 @@ int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zk
 int32_t zkp_kzg_verify_cell_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_commitments, const uint8_t *d_commitment_inf,
                                 const uint64_t *d_cell_indices, const uint8_t *d_cells, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
                                 size_t n, uint8_t *d_status, void *d_scratch, void *stream);
+
+/* recover_cells_and_kzg_proofs: any 64 or more cells of each of n blobs -> all 128 cells (and proofs), exactly as the
+ * spec's recover_polynomialcoeff (coset shift 7) followed by compute_cells_and_kzg_proofs, for consistent and
+ * inconsistent cells alike.  Blob b's input is cell_indices[128 b ..] (n x 128 u64), cells[128 b ..] (n x 128 x
+ * ZKP_CELL_BYTES) and num_cells[b]: its first num_cells[b] entries are the spec's cell_indices and cells, the entries
+ * after them are ignored.  Outputs are those of zkp_kzg_compute_cells_and_proofs_batch.  Statuses per blob:
+ * ZKP_KZG_BAD_CELLS for a count outside [64, 128], indices not strictly ascending (duplicates included) or an index
+ * >= 128, else ZKP_KZG_BAD_SCALAR for an element >= r in a given cell; a rejected blob gets zero cells (and proofs of
+ * zero limbs with the flag set) and the call returns ZKP_OK.  Each blob is one cluster of two thread blocks with 128 KiB
+ * of shared memory each; a device on which no such cluster can be resident fails the call with ZKP_ERR_CUDA.  Host
+ * paths stream double-buffered chunks per device of at most 2^11 blobs (512 MiB of cells in and out per buffer set),
+ * 2^7 with proofs.  All four need a setup from zkp_kzg_setup_create_cells. */
+int32_t zkp_kzg_recover_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *cell_indices, const uint8_t *cells,
+                                    const uint64_t *num_cells, size_t n, uint8_t *out_cells, uint8_t *out_status);
+int32_t zkp_kzg_recover_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *cell_indices, const uint8_t *cells,
+                                               const uint64_t *num_cells, size_t n, uint8_t *out_cells, uint64_t *out_proofs,
+                                               uint8_t *out_proof_inf, uint8_t *out_status);
+/* Device-resident forms, conventions as zkp_kzg_compute_cells_dev; d_cells, d_out_cells and d_scratch 16-byte aligned;
+ * the proof form takes zkp_kzg_cells_proofs_scratch_bytes(n) bytes of d_scratch. */
+int32_t zkp_kzg_recover_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices, const uint8_t *d_cells,
+                                  const uint64_t *d_num_cells, size_t n, uint8_t *d_out_cells, uint8_t *d_status, void *stream);
+int32_t zkp_kzg_recover_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices,
+                                             const uint8_t *d_cells, const uint64_t *d_num_cells, size_t n, uint8_t *d_out_cells,
+                                             uint64_t *d_proofs, uint8_t *d_proof_inf, uint8_t *d_status, void *d_scratch, void *stream);
 
 /* ---- measurement helpers -------------------------------------------------------------------- */
 

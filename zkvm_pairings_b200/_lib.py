@@ -103,6 +103,13 @@ SYMBOLS = {
                                                               c_u64p, c_u8p, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_kzg_verify_cell_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, c_u8p, c_u64p, c_u8p,
                                                  ctypes.c_size_t, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_kzg_recover_cells_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u8p, c_u8p]),
+    "zkp_kzg_recover_cells_and_proofs_batch": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u8p,
+                                                                c_u64p, c_u8p, c_u8p]),
+    "zkp_kzg_recover_cells_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u8p,
+                                                   c_u8p, ctypes.c_void_p]),
+    "zkp_kzg_recover_cells_and_proofs_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, c_u64p, c_u8p, c_u64p,
+                                                              ctypes.c_size_t, c_u8p, c_u64p, c_u8p, c_u8p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_imad_peak": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(ctypes.c_double)]),
     "zkp_launch_count": (ctypes.c_uint64, [ctypes.c_void_p]),
     "zkp_set_kernel_timing": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32]),

@@ -31,6 +31,9 @@
 #include "blob.cuh"
 #include "kzg_prove.cuh"
 #include "kzg_cells.cuh"
+#include "kzg_recover.cuh"
+
+#include <cooperative_groups.h>
 
 #ifndef ZKP_TPB
 #define ZKP_TPB 128           // threads per block of the pairing kernels
@@ -430,6 +433,62 @@ k_cells_quotient(const Fr *__restrict__ coeffs, const Fr *__restrict__ pw, const
     cells_quotient_chain((int)(r % ZKP_CELLS_PER_BLOB), m, coeffs + b * ZKP_BLOB_N, pw, rows + r * ZKP_BLOB_BYTES_);
 }
 
+// recover_cells: one cluster of two blocks per blob (kzg_recover.cuh), rank r holding slots [4096 r, 4096 r + 4096) of
+// the extended blob in dynamic shared memory (128 KiB).  idx (n x 128), cells (n x 128 x 2048 bytes) and num (n) are
+// the input; out receives the 128 cells (n x 256 KiB), coeffs (n x 4096 Fr, or NULL) the coefficients for the proofs.
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ZKP_CELLS_TPB, 1)
+k_cells_recover(const uint64_t *__restrict__ idx, const uint8_t *__restrict__ cells, const uint64_t *__restrict__ num,
+                const Fr *__restrict__ pw, uint8_t *__restrict__ out, Fr *__restrict__ coeffs, uint8_t *__restrict__ status) {
+    namespace cg = cooperative_groups;
+    extern __shared__ Fr rec_x[];
+    __shared__ RecoverShared sh;
+    cg::cluster_group cl = cg::this_cluster();
+    const int r = (int)cl.block_rank(), t = threadIdx.x;
+    const size_t b = blockIdx.x / 2;
+    const uint64_t n = num[b];
+    recover_init(t, n, sh);
+    __syncthreads();
+    recover_index(t, n, idx + b * ZKP_CELLS_PER_BLOB, sh);
+    __syncthreads();
+    recover_vanish_part(r, t, pw, sh, rec_x);
+    __syncthreads();
+    if (t < ZKP_CELL_N) recover_vanish(t, rec_x, sh);
+    __syncthreads();
+    recover_load(r, t, cells + b * ZKP_CELLS_PER_BLOB * ZKP_CELL_BYTES_, sh, rec_x);
+    __syncthreads();
+    for (int h = 1; h < ZKP_RECOVER_HALF; h <<= 1) {
+        cells_dit_pass(t, rec_x, pw, h);
+        __syncthreads();
+    }
+    cl.sync();   // both halves transformed (and both blocks' sh.bad final)
+    Fr *half[2];
+    half[r] = rec_x;
+    half[r ^ 1] = cl.map_shared_rank(rec_x, r ^ 1);
+    const bool bad_other = cl.map_shared_rank(&sh, r ^ 1)->bad != 0;
+    const bool rej = sh.bad_cells || sh.bad || bad_other;
+    recover_cross_a(r, t, pw, half);
+    cl.sync();
+    for (int h = ZKP_RECOVER_HALF / 2; h >= 1; h >>= 1) {
+        cells_dif_pass(t, rec_x, pw, h);
+        __syncthreads();
+    }
+    recover_divide(t, sh, rec_x);
+    __syncthreads();
+    for (int h = 1; h < ZKP_RECOVER_HALF; h <<= 1) {
+        cells_dit_pass(t, rec_x, pw, h);
+        __syncthreads();
+    }
+    cl.sync();
+    recover_cross_b(r, t, pw, half, coeffs ? coeffs + b * ZKP_BLOB_N : nullptr);
+    cl.sync();   // also: no block reads the other's shared memory after this
+    for (int h = ZKP_RECOVER_HALF / 2; h >= 1; h >>= 1) {
+        cells_dif_pass(t, rec_x, pw, h);
+        __syncthreads();
+    }
+    recover_store(r, t, rec_x, rej, out + b * 2 * ZKP_BLOB_BYTES_);
+    if (r == 0 && t == 0) status[b] = recover_status(sh, bad_other);
+}
+
 // The verifier's interpolation, one 64-thread block per cell: I_k from the cell, then [I_k(tau)]G1 over the first 64
 // monomial tables (ixy / iinf), and the status (ZKP_KZG_BAD_SCALAR for an element >= r or an index >= 128)
 __global__ void __launch_bounds__(ZKP_CELL_N)
@@ -810,6 +869,8 @@ struct KzgDev {   // one device's copy of a setup, in one allocation
     const Fp *cell_prep = nullptr;   // prepared tables of G2 and -[tau^64]G2
     const Fr *pw = nullptr;          // omega_8192^e, e < 8192 (Montgomery)
     const Fp *mono = nullptr;        // the signed-digit window tables of [tau^i]G1, i < 4096
+    int recover_clusters = 0;        // cudaOccupancyMaxActiveClusters of k_cells_recover; recovery needs >= 1
+    cudaError_t recover_err = cudaSuccess;   // why that query failed
 };
 struct zkp_kzg_setup {
     zkp_ctx *ctx = nullptr;
@@ -929,6 +990,9 @@ static cudaError_t launch_kzg_prove(zkp_ctx *ctx, const KzgDev &k, const uint8_t
 #ifndef ZKP_CELL_PROOF_CHUNK
 #define ZKP_CELL_PROOF_CHUNK (1u << 7)     // blobs per host chunk with proofs: 2 GiB of quotient rows per buffer set
 #endif
+#ifndef ZKP_CELLS_RECOVER_CHUNK
+#define ZKP_CELLS_RECOVER_CHUNK (1u << 11) // blobs per host chunk of recovery: 512 MiB of cells in, 512 MiB out per buffer set
+#endif
 #ifndef ZKP_CELL_VERIFY_CHUNK
 #define ZKP_CELL_VERIFY_CHUNK (1u << 16)   // cells per host chunk of verification: 128 MiB of cells per buffer set
 #endif
@@ -949,6 +1013,24 @@ static cudaError_t launch_cells(zkp_ctx *ctx, const KzgDev &k, const uint8_t *bl
     if (n == 0) return cudaSuccess;
     Fr *coeffs = proofs ? (Fr *)scratch : nullptr;
     k_cells_extend<<<(unsigned)n, ZKP_CELLS_TPB, ZKP_BLOB_N * sizeof(Fr), st>>>(blobs, k.pw, cells, coeffs, status);
+    ctx->launches++;
+    if (proofs) {
+        uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
+        const size_t nt = n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N;
+        k_cells_quotient<<<(unsigned)((nt + ZKP_CELLS_QUOT_TPB - 1) / ZKP_CELLS_QUOT_TPB), ZKP_CELLS_QUOT_TPB, 0, st>>>(coeffs, k.pw, status, n,
+                                                                                                                    rows, rst);
+        k_kzg_msm<<<(unsigned)(n * ZKP_CELLS_PER_BLOB), ZKP_MSM_TPB, 0, st>>>(k.mono, rows, rst, proofs, proof_inf, rst);
+        ctx->launches += 2;
+    }
+    return cudaGetLastError();
+}
+
+// recover_cells (and, with proofs, as launch_cells from the recovered coefficients); proofs == NULL: cells only
+static cudaError_t launch_cells_recover(zkp_ctx *ctx, const KzgDev &k, const uint64_t *idx, const uint8_t *cells, const uint64_t *num, size_t n,
+                                        uint8_t *out, uint64_t *proofs, uint8_t *proof_inf, uint8_t *status, void *scratch, cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    Fr *coeffs = proofs ? (Fr *)scratch : nullptr;
+    k_cells_recover<<<(unsigned)(2 * n), ZKP_CELLS_TPB, ZKP_RECOVER_HALF * sizeof(Fr), st>>>(idx, cells, num, k.pw, out, coeffs, status);
     ctx->launches++;
     if (proofs) {
         uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
@@ -1232,6 +1314,7 @@ struct HostJob {
     // flags in g1inf, z | y out in out): blobs in blobs, the points out in og1 / og1inf, the statuses in flags
     // modes 176 / 192 = cells / cells and proofs: blobs in blobs, cells out in ocells, proofs in og1 / og1inf, statuses in flags.
     // mode 208 = cell verification: commitments in pts (flags in g1inf), indices in idx, cells in cells, proofs in pi (flags in piinf)
+    // modes 224 / 240 = recovery / recovery with proofs: indices in idx, cells in cells, counts in scalars; outputs as 176 / 192
     uint8_t *ocells = nullptr;
     const uint8_t *cells = nullptr, *piinf = nullptr;
     const uint64_t *idx = nullptr, *pi = nullptr;
@@ -1257,6 +1340,8 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
                    : j.mode == 176 ? (size_t)ZKP_CELLS_CHUNK
                    : j.mode == 192 ? (size_t)ZKP_CELL_PROOF_CHUNK
                    : j.mode == 208 ? (size_t)ZKP_CELL_VERIFY_CHUNK
+                   : j.mode == 224 ? (size_t)ZKP_CELLS_RECOVER_CHUNK
+                   : j.mode == 240 ? (size_t)ZKP_CELL_PROOF_CHUNK
                    : j.mode >= 112 ? (size_t)ZKP_BLOB_CHUNK
                                    : (size_t)ZKP_CHUNK;
     int s = 0;
@@ -1452,6 +1537,34 @@ static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo,
             CUS(launch_cells(ctx, kd, (const uint8_t *)B[B_IN].p, cn, (uint8_t *)B[B_G1].p, dpf, dpi, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, st));
             CUS(d2h(B_G1, j.ocells + c0 * cb, B[B_G1].p, cn * cb));
             if (j.mode == 192) {
+                CUS(d2h(B_G2, j.og1 + c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 96));
+                CUS(d2h(B_G2INF, j.og1inf + c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np));
+            }
+            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
+        } else if (j.mode == 224 || j.mode == 240) {
+            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
+            const size_t cb = (size_t)ZKP_CELLS_PER_EXT_BLOB * ZKP_CELL_BYTES, np = cn * ZKP_CELLS_PER_EXT_BLOB;
+            CUS(B[B_IN].ensure(cn * cb));
+            CUS(B[B_G1].ensure(cn * cb));
+            CUS(B[B_TAB].ensure(np * 8));
+            CUS(B[B_G1INF].ensure(cn * 8));
+            CUS(B[B_FLAG].ensure(cn));
+            CUS(h2d(B_IN, B[B_IN].p, j.cells + c0 * cb, cn * cb));
+            CUS(h2d(B_TAB, B[B_TAB].p, j.idx + c0 * ZKP_CELLS_PER_EXT_BLOB, np * 8));
+            CUS(h2d(B_G1INF, B[B_G1INF].p, j.scalars + c0, cn * 8));
+            uint64_t *dpf = nullptr;
+            uint8_t *dpi = nullptr;
+            if (j.mode == 240) {
+                CUS(B[B_G2].ensure(np * 96));
+                CUS(B[B_G2INF].ensure(np));
+                CUS(B[B_OUT].ensure(zkp_kzg_cells_proofs_scratch_bytes(cn)));
+                dpf = (uint64_t *)B[B_G2].p;
+                dpi = (uint8_t *)B[B_G2INF].p;
+            }
+            CUS(launch_cells_recover(ctx, kd, (const uint64_t *)B[B_TAB].p, (const uint8_t *)B[B_IN].p, (const uint64_t *)B[B_G1INF].p, cn,
+                                     (uint8_t *)B[B_G1].p, dpf, dpi, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, st));
+            CUS(d2h(B_G1, j.ocells + c0 * cb, B[B_G1].p, cn * cb));
+            if (j.mode == 240) {
                 CUS(d2h(B_G2, j.og1 + c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 96));
                 CUS(d2h(B_G2INF, j.og1inf + c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np));
             }
@@ -2369,6 +2482,20 @@ static cudaError_t kzg_cells_build(zkp_ctx *ctx, DevState &d, KzgDev &k, const u
     cudaStream_t st = d.stream[0];
     void *scratch = nullptr;
     cudaError_t e = cudaFuncSetAttribute(k_cells_extend, cudaFuncAttributeMaxDynamicSharedMemorySize, ZKP_BLOB_N * sizeof(Fr));
+    if (e == cudaSuccess) {   // recovery's clusters; a failure here only disables recovery (its calls report it)
+        k.recover_err = cudaFuncSetAttribute(k_cells_recover, cudaFuncAttributeMaxDynamicSharedMemorySize, ZKP_RECOVER_HALF * sizeof(Fr));
+        if (k.recover_err == cudaSuccess) {
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3(2);
+            cfg.blockDim = dim3(ZKP_CELLS_TPB);
+            cfg.dynamicSmemBytes = ZKP_RECOVER_HALF * sizeof(Fr);
+            k.recover_err = cudaOccupancyMaxActiveClusters(&k.recover_clusters, k_cells_recover, &cfg);
+        }
+        if (k.recover_err != cudaSuccess) {
+            cudaGetLastError();
+            k.recover_clusters = 0;
+        }
+    }
     if (e == cudaSuccess) e = cudaMalloc(&k.cell_mem, cell_b);
     if (e == cudaSuccess) e = cudaMalloc(&scratch, tmp_b);
     if (e == cudaSuccess) {
@@ -2529,6 +2656,78 @@ int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zk
     DeviceGuard guard;
     CU(cudaSetDevice(ctx->devs[dev].id));
     CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, d_proofs, d_proof_inf, d_status, d_scratch, (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+// recovery runs one cluster of two blocks with 128 KiB of shared memory each per blob: refuse (never substitute) a device
+// on which no such cluster can be resident; dev < 0: every device of the context
+static int32_t check_recover(zkp_ctx *ctx, const zkp_kzg_setup *s, int32_t dev) {
+    int32_t rc = check_cells(ctx, s);
+    if (rc) return rc;
+    for (size_t di = 0; di < s->devs.size(); di++) {
+        if (dev >= 0 && (size_t)dev != di) continue;
+        const KzgDev &k = s->devs[di];
+        if (k.recover_clusters < 1)
+            return fail(ZKP_ERR_CUDA, "k_cells_recover cannot run on device " + std::to_string(ctx->devs[di].id) +
+                                          ": no cluster of two 512-thread blocks with 128 KiB of shared memory each can be resident (" +
+                                          (k.recover_err != cudaSuccess ? cudaGetErrorString(k.recover_err) : "0 active clusters") + ")");
+    }
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_recover_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *cell_indices, const uint8_t *cells,
+                                    const uint64_t *num_cells, size_t n, uint8_t *out_cells, uint8_t *out_status) {
+    int32_t rc = check_recover(ctx, s, -1);
+    if (rc) return rc;
+    if (n && (!cell_indices || !cells || !num_cells || !out_cells || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 224; j.kzg = s; j.idx = cell_indices; j.cells = cells; j.scalars = num_cells; j.ocells = out_cells; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_recover_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *cell_indices, const uint8_t *cells,
+                                               const uint64_t *num_cells, size_t n, uint8_t *out_cells, uint64_t *out_proofs,
+                                               uint8_t *out_proof_inf, uint8_t *out_status) {
+    int32_t rc = check_recover(ctx, s, -1);
+    if (rc) return rc;
+    if (n && (!cell_indices || !cells || !num_cells || !out_cells || !out_proofs || !out_proof_inf || !out_status))
+        return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    HostJob j;
+    j.mode = 240; j.kzg = s; j.idx = cell_indices; j.cells = cells; j.scalars = num_cells; j.ocells = out_cells; j.og1 = out_proofs;
+    j.og1inf = out_proof_inf; j.flags = out_status;
+    return run_host_job(ctx, j, n);
+}
+
+int32_t zkp_kzg_recover_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices, const uint8_t *d_cells,
+                                  const uint64_t *d_num_cells, size_t n, uint8_t *d_out_cells, uint8_t *d_status, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_recover(ctx, s, dev);
+    if (rc) return rc;
+    if (n && (!d_cell_indices || !d_cells || !d_num_cells || !d_out_cells || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_out_cells & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_cells and d_out_cells must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    CU(cudaSetDevice(ctx->devs[dev].id));
+    CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, nullptr, nullptr, d_status, nullptr,
+                            (cudaStream_t)stream));
+    return ZKP_OK;
+}
+
+int32_t zkp_kzg_recover_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices,
+                                             const uint8_t *d_cells, const uint64_t *d_num_cells, size_t n, uint8_t *d_out_cells,
+                                             uint64_t *d_proofs, uint8_t *d_proof_inf, uint8_t *d_status, void *d_scratch, void *stream) {
+    int32_t rc = check_dev(ctx, dev);
+    if (rc == ZKP_OK) rc = check_recover(ctx, s, dev);
+    if (rc) return rc;
+    if (n && (!d_cell_indices || !d_cells || !d_num_cells || !d_out_cells || !d_proofs || !d_proof_inf || !d_status || !d_scratch))
+        return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_out_cells & 15) || ((uintptr_t)d_scratch & 15))
+        return fail(ZKP_ERR_INVALID_ARG, "d_cells, d_out_cells and d_scratch must be 16-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    CU(cudaSetDevice(ctx->devs[dev].id));
+    CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, d_proofs, d_proof_inf, d_status, d_scratch,
+                            (cudaStream_t)stream));
     return ZKP_OK;
 }
 

@@ -40,6 +40,7 @@ GROTH16_PROOF_U64 = 48
 GROTH16_MAX_PUBLIC = 256
 # per-proof verdicts of kzg_verify_batch / kzg_verify_dev (include/zkpair.h ZKP_KZG_*)
 KZG_VALID, KZG_INVALID, KZG_BAD_POINT, KZG_BAD_SCALAR = 0, 1, 2, 3
+KZG_BAD_CELLS = 4         # cell recovery: a bad cell count or bad cell indices (include/zkpair.h ZKP_KZG_BAD_CELLS)
 KZG_PROOF_U64 = 24
 BLOB_N = 4096            # EIP-4844 FIELD_ELEMENTS_PER_BLOB (include/zkpair.h ZKP_BLOB_FIELD_ELEMENTS)
 BLOB_BYTES = 32 * BLOB_N   # one EIP-4844 blob: 4096 big-endian field elements (include/zkpair.h ZKP_BLOB_BYTES)
@@ -543,6 +544,49 @@ class PairingEngine:
         self._check(self._lib.zkp_kzg_verify_cell_batch(self._ctx, setup.handle, _ptr(c), _ptr(ci), _ptr(idx), _ptr(cl), _ptr(pr), _ptr(pi), n,
                                                         _ptr(st)))
         return st
+
+    @staticmethod
+    def _recover_inputs(cell_indices, cells, num_cells):
+        idx = np.ascontiguousarray(cell_indices, dtype=np.uint64).reshape(-1, CELLS_PER_EXT_BLOB)
+        n = idx.shape[0]
+        cl = np.ascontiguousarray(cells, dtype=np.uint8).reshape(n, CELLS_PER_EXT_BLOB, CELL_BYTES)
+        num = np.ascontiguousarray(num_cells, dtype=np.uint64).reshape(n)
+        return idx, cl, num, n
+
+    def kzg_recover_cells_batch(self, setup: KzgSetup, cell_indices, cells, num_cells):
+        """recover_cells_and_kzg_proofs without the proofs.  Per blob: cell_indices (n, 128), cells (n, 128, CELL_BYTES) and
+        num_cells (n,), of which the first num_cells[b] entries are the given cells -> (cells (n, 128, CELL_BYTES), status
+        (n,)); KZG_BAD_CELLS for a count outside [64, 128], indices not strictly ascending or one >= 128, KZG_BAD_SCALAR
+        for an element >= r, both with zero cells."""
+        idx, cl, num, n = self._recover_inputs(cell_indices, cells, num_cells)
+        out, st = np.zeros((n, CELLS_PER_EXT_BLOB, CELL_BYTES), np.uint8), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_recover_cells_batch(self._ctx, setup.handle, _ptr(idx), _ptr(cl), _ptr(num), n, _ptr(out), _ptr(st)))
+        return out, st
+
+    def kzg_recover_cells_and_proofs_batch(self, setup: KzgSetup, cell_indices, cells, num_cells):
+        """recover_cells_and_kzg_proofs: inputs as kzg_recover_cells_batch -> (cells (n, 128, CELL_BYTES), proofs (n, 128, 12),
+        proof_inf (n, 128), status (n,)), as kzg_compute_cells_and_proofs_batch returns them."""
+        idx, cl, num, n = self._recover_inputs(cell_indices, cells, num_cells)
+        out = np.zeros((n, CELLS_PER_EXT_BLOB, CELL_BYTES), np.uint8)
+        pr, pi, st = np.zeros((n, CELLS_PER_EXT_BLOB, 12), np.uint64), np.zeros((n, CELLS_PER_EXT_BLOB), np.uint8), np.zeros(n, np.uint8)
+        self._check(self._lib.zkp_kzg_recover_cells_and_proofs_batch(self._ctx, setup.handle, _ptr(idx), _ptr(cl), _ptr(num), n, _ptr(out),
+                                                                     _ptr(pr), _ptr(pi), _ptr(st)))
+        return out, pr, pi, st
+
+    def kzg_recover_cells_dev(self, setup: KzgSetup, d_cell_indices, d_cells, d_num_cells, n: int, d_out_cells, d_status,
+                              stream: int = 0, dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_cells and d_out_cells 16-byte aligned."""
+        self._check(self._lib.zkp_kzg_recover_cells_dev(self._ctx, dev, setup.handle, _dptr(d_cell_indices), _dptr(d_cells), _dptr(d_num_cells),
+                                                        n, _dptr(d_out_cells), _dptr(d_status), ctypes.c_void_p(stream)))
+
+    def kzg_recover_cells_and_proofs_dev(self, setup: KzgSetup, d_cell_indices, d_cells, d_num_cells, n: int, d_out_cells, d_proofs,
+                                         d_proof_inf, d_status, d_scratch, stream: int = 0, dev: int = 0):
+        """Asynchronous form; d_scratch holds kzg_cells_proofs_scratch_bytes(n) bytes; d_cells, d_out_cells, d_scratch 16-byte
+        aligned."""
+        self._check(self._lib.zkp_kzg_recover_cells_and_proofs_dev(self._ctx, dev, setup.handle, _dptr(d_cell_indices), _dptr(d_cells),
+                                                                   _dptr(d_num_cells), n, _dptr(d_out_cells), _dptr(d_proofs),
+                                                                   _dptr(d_proof_inf), _dptr(d_status), _dptr(d_scratch),
+                                                                   ctypes.c_void_p(stream)))
 
     def kzg_cells_proofs_scratch_bytes(self, n: int) -> int:
         return int(self._lib.zkp_kzg_cells_proofs_scratch_bytes(n))
