@@ -19,6 +19,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -815,28 +816,39 @@ static size_t g16_chunk(int n_public) {
     return c ? c : 1;
 }
 
+// Carves scratch into consecutive parts of the given sizes, each rounded up to 256 bytes: part[i] is where part i
+// starts (NULL when base is NULL).  Returns the bytes of all parts.
+template <size_t N> static size_t carve(void *base, const size_t (&sz)[N], uint8_t *(&part)[N]) {
+    size_t o = 0;
+    for (size_t i = 0; i < N; i++) {
+        part[i] = base ? (uint8_t *)base + o : nullptr;
+        o += align256(sz[i]);
+    }
+    return o;
+}
+
+// The prepared check of n assembled checks (k pairs each, the last kf of them from the tables prep), then the verdicts
+// of the front end's status bytes.  The verifiers share it: Groth16 (k = 4, kf = 3), KZG and cells (k = kf = 2).
+static cudaError_t launch_check_verdict(zkp_ctx *ctx, DevState &d, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2,
+                                        const uint8_t *g2inf, size_t n, int k, const Fp *prep, int kf, uint64_t *gt, uint8_t *is_one,
+                                        uint8_t *status, uint32_t *err, cudaStream_t st) {
+    cudaError_t e = launch_pairing(ctx, d, 3, g1, g1inf, g2, g2inf, n, k, nullptr, gt, is_one, err, st, prep, nullptr, kf);
+    if (e != cudaSuccess) return e;
+    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(is_one, status, n);
+    ctx->launches++;
+    return cudaGetLastError();
+}
+
 // scratch of one batch of n proofs: assembled pairs [A, alpha, L, C] x [B], the Gt outputs and is_one
 struct G16Scratch {
     uint64_t *g1, *g2, *gt;
     uint8_t *g1inf, *g2inf, *is_one;
 };
 static size_t g16_layout(size_t n, void *base, G16Scratch *s) {
-    const size_t sz[6] = {n * 4 * 96, n * 192, n * 576, n * 4, n, n};
-    size_t off[6], o = 0;
-    for (int i = 0; i < 6; i++) {
-        off[i] = o;
-        o += align256(sz[i]);
-    }
-    if (s) {
-        uint8_t *b = (uint8_t *)base;
-        s->g1 = (uint64_t *)(b + off[0]);
-        s->g2 = (uint64_t *)(b + off[1]);
-        s->gt = (uint64_t *)(b + off[2]);
-        s->g1inf = b + off[3];
-        s->g2inf = b + off[4];
-        s->is_one = b + off[5];
-    }
-    return o;
+    uint8_t *p[6];
+    const size_t bytes = carve(base, {n * 4 * 96, n * 192, n * 576, n * 4, n, n}, p);
+    if (s) *s = {(uint64_t *)p[0], (uint64_t *)p[1], (uint64_t *)p[2], p[3], p[4], p[5]};
+    return bytes;
 }
 
 // front end -> prepared 4-pair check (k = 4, the last kf = 3 pairs from the key's tables) -> verdict
@@ -849,11 +861,7 @@ static cudaError_t launch_groth16(zkp_ctx *ctx, DevState &d, const G16Dev &k, co
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, s.g2, s.g2inf, n, 4, nullptr, s.gt, s.is_one, err, st, k.prep, nullptr, 3);
-    if (e != cudaSuccess) return e;
-    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
-    ctx->launches++;
-    return cudaGetLastError();
+    return launch_check_verdict(ctx, d, s.g1, s.g1inf, s.g2, s.g2inf, n, 4, k.prep, 3, s.gt, s.is_one, status, err, st);
 }
 
 // ---- KZG point-evaluation verification: resident setup and the per-batch launch sequence
@@ -885,20 +893,10 @@ struct KzgScratch {
     uint8_t *g1inf, *is_one;
 };
 static size_t kzg_layout(size_t n, void *base, KzgScratch *s) {
-    const size_t sz[4] = {n * 2 * 96, n * 576, n * 2, n};
-    size_t off[4], o = 0;
-    for (int i = 0; i < 4; i++) {
-        off[i] = o;
-        o += align256(sz[i]);
-    }
-    if (s) {
-        uint8_t *b = (uint8_t *)base;
-        s->g1 = (uint64_t *)(b + off[0]);
-        s->gt = (uint64_t *)(b + off[1]);
-        s->g1inf = b + off[2];
-        s->is_one = b + off[3];
-    }
-    return o;
+    uint8_t *p[4];
+    const size_t bytes = carve(base, {n * 2 * 96, n * 576, n * 2, n}, p);
+    if (s) *s = {(uint64_t *)p[0], (uint64_t *)p[1], p[2], p[3]};
+    return bytes;
 }
 
 // front end -> prepared 2-pair check (k = kf = 2: both G2 points from the setup's tables) -> verdict
@@ -911,11 +909,7 @@ static cudaError_t launch_kzg(zkp_ctx *ctx, DevState &d, const KzgDev &k, const 
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, nullptr, nullptr, n, 2, nullptr, s.gt, s.is_one, err, st, k.prep, nullptr, 2);
-    if (e != cudaSuccess) return e;
-    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
-    ctx->launches++;
-    return cudaGetLastError();
+    return launch_check_verdict(ctx, d, s.g1, s.g1inf, nullptr, nullptr, n, 2, k.prep, 2, s.gt, s.is_one, status, err, st);
 }
 
 // ---- EIP-4844 blob verification: z by k_blob_challenge, y by k_blob_eval, then the point-evaluation check
@@ -1007,6 +1001,18 @@ extern "C" size_t zkp_kzg_cells_proofs_scratch_bytes(size_t n) {
 // scratch of n cell checks: the point-evaluation pairs, then [I_k(tau)]G1 (n x 96 bytes) and its flags
 extern "C" size_t zkp_kzg_verify_cell_scratch_bytes(size_t n) { return kzg_layout(n, nullptr, nullptr) + align256(n * 96) + align256(n); }
 
+// the proofs of n blobs from their coefficients at the start of scratch: k_cells_quotient, then k_kzg_msm over the
+// monomial tables (the launch errors are left to the caller's cudaGetLastError)
+static void launch_cell_proofs(zkp_ctx *ctx, const KzgDev &k, const Fr *coeffs, size_t n, uint64_t *proofs, uint8_t *proof_inf,
+                               uint8_t *status, void *scratch, cudaStream_t st) {
+    uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
+    const size_t nt = n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N;
+    k_cells_quotient<<<(unsigned)((nt + ZKP_CELLS_QUOT_TPB - 1) / ZKP_CELLS_QUOT_TPB), ZKP_CELLS_QUOT_TPB, 0, st>>>(coeffs, k.pw, status, n,
+                                                                                                                rows, rst);
+    k_kzg_msm<<<(unsigned)(n * ZKP_CELLS_PER_BLOB), ZKP_MSM_TPB, 0, st>>>(k.mono, rows, rst, proofs, proof_inf, rst);
+    ctx->launches += 2;
+}
+
 // proofs == NULL: cells only (no scratch)
 static cudaError_t launch_cells(zkp_ctx *ctx, const KzgDev &k, const uint8_t *blobs, size_t n, uint8_t *cells, uint64_t *proofs,
                                 uint8_t *proof_inf, uint8_t *status, void *scratch, cudaStream_t st) {
@@ -1014,14 +1020,7 @@ static cudaError_t launch_cells(zkp_ctx *ctx, const KzgDev &k, const uint8_t *bl
     Fr *coeffs = proofs ? (Fr *)scratch : nullptr;
     k_cells_extend<<<(unsigned)n, ZKP_CELLS_TPB, ZKP_BLOB_N * sizeof(Fr), st>>>(blobs, k.pw, cells, coeffs, status);
     ctx->launches++;
-    if (proofs) {
-        uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
-        const size_t nt = n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N;
-        k_cells_quotient<<<(unsigned)((nt + ZKP_CELLS_QUOT_TPB - 1) / ZKP_CELLS_QUOT_TPB), ZKP_CELLS_QUOT_TPB, 0, st>>>(coeffs, k.pw, status, n,
-                                                                                                                    rows, rst);
-        k_kzg_msm<<<(unsigned)(n * ZKP_CELLS_PER_BLOB), ZKP_MSM_TPB, 0, st>>>(k.mono, rows, rst, proofs, proof_inf, rst);
-        ctx->launches += 2;
-    }
+    if (proofs) launch_cell_proofs(ctx, k, coeffs, n, proofs, proof_inf, status, scratch, st);
     return cudaGetLastError();
 }
 
@@ -1032,14 +1031,7 @@ static cudaError_t launch_cells_recover(zkp_ctx *ctx, const KzgDev &k, const uin
     Fr *coeffs = proofs ? (Fr *)scratch : nullptr;
     k_cells_recover<<<(unsigned)(2 * n), ZKP_CELLS_TPB, ZKP_RECOVER_HALF * sizeof(Fr), st>>>(idx, cells, num, k.pw, out, coeffs, status);
     ctx->launches++;
-    if (proofs) {
-        uint8_t *rows = (uint8_t *)scratch + cells_coeff_bytes(n), *rst = rows + cells_rows_bytes(n);
-        const size_t nt = n * ZKP_CELLS_PER_BLOB * ZKP_CELL_N;
-        k_cells_quotient<<<(unsigned)((nt + ZKP_CELLS_QUOT_TPB - 1) / ZKP_CELLS_QUOT_TPB), ZKP_CELLS_QUOT_TPB, 0, st>>>(coeffs, k.pw, status, n,
-                                                                                                                    rows, rst);
-        k_kzg_msm<<<(unsigned)(n * ZKP_CELLS_PER_BLOB), ZKP_MSM_TPB, 0, st>>>(k.mono, rows, rst, proofs, proof_inf, rst);
-        ctx->launches += 2;
-    }
+    if (proofs) launch_cell_proofs(ctx, k, coeffs, n, proofs, proof_inf, status, scratch, st);
     return cudaGetLastError();
 }
 
@@ -1055,11 +1047,172 @@ static cudaError_t launch_cells_verify(zkp_ctx *ctx, DevState &d, const KzgDev &
     ctx->launches += 2;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    e = launch_pairing(ctx, d, 3, s.g1, s.g1inf, nullptr, nullptr, n, 2, nullptr, s.gt, s.is_one, err, st, k.cell_prep, nullptr, 2);
-    if (e != cudaSuccess) return e;
-    k_groth16_verdict<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s.is_one, status, n);
-    ctx->launches++;
-    return cudaGetLastError();
+    return launch_check_verdict(ctx, d, s.g1, s.g1inf, nullptr, nullptr, n, 2, k.cell_prep, 2, s.gt, s.is_one, status, err, st);
+}
+
+// Runs launch(d, st) for a device-resident entry point whose arguments passed their checks: under the context lock, on
+// device dev of the context (the caller's current device is restored) and on the caller's stream (NULL = the legacy
+// default stream, the CUDA convention).
+template <class F> static int32_t on_device(zkp_ctx *ctx, int32_t dev, void *stream, F launch) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DevState &d = ctx->devs[dev];
+    DeviceGuard guard;
+    CU(cudaSetDevice(d.id));
+    return launch(d, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------ host-buffer pipeline
+
+// Split [0,n) into one contiguous slice per device.
+static void slice_of(size_t n, size_t ndev, size_t d, size_t &lo, size_t &hi) {
+    lo = n * d / ndev;
+    hi = n * (d + 1) / ndev;
+}
+
+// The devices a call of n elements runs on, one slice_of slice each: the first alone when a slice would hold
+// fewer than two elements.
+static size_t fan_out(const zkp_ctx *ctx, size_t n) {
+    const size_t nd = ctx->devs.size();
+    return nd == 1 || n < 2 * nd ? 1 : nd;
+}
+
+// A failed CUDA call inside a host-buffer call: thrown by CUT, caught by run_slice, so that nothing after it is launched.
+struct CudaFail {
+    std::string msg;
+};
+#define CUT(call)                                                                                  \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) throw CudaFail{std::string(#call) + ": " + cudaGetErrorString(e_)}; \
+    } while (0)
+
+// One chunk [c0, c0 + cn) of the slice [lo, hi) of device dev, on the stream and buffer set s.  Its copies go through
+// the buffer slots B_* of that set; pageable host buffers of at least ZKP_STAGE_MIN bytes are staged through the
+// set's pinned buffers (an async copy from or to pageable memory blocks the issuing thread, which would serialise
+// the two sets), and the staged outputs reach the caller's buffers when the set's stream has drained.
+struct Chunk {
+    zkp_ctx *ctx;
+    DevState &d;
+    size_t dev, lo, hi, c0, cn;
+    cudaStream_t st;
+    int s;
+
+    static bool pageable(const void *p) {
+        cudaPointerAttributes a;
+        if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+            cudaGetLastError();
+            return true;
+        }
+        return a.type == cudaMemoryTypeUnregistered;
+    }
+    // slot with room for n elements
+    template <class T> T *buf(int slot, size_t n) {
+        CUT(d.buf[s][slot].ensure(n * sizeof(T)));
+        return (T *)d.buf[s][slot].p;
+    }
+    // n elements from the host to dst (in slot's memory, or after it for B_TABINF)
+    template <class T> void h2d(int slot, T *dst, const T *src, size_t n) {
+        const size_t bytes = n * sizeof(T);
+        if (bytes >= ZKP_STAGE_MIN && pageable(src)) {
+            PinBuf &pb = d.pin_in[s][slot];
+            CUT(pb.ensure(bytes));
+            memcpy(pb.p, src, bytes);
+            src = (const T *)pb.p;
+        }
+        CUT(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st));
+    }
+    // elements [off, off + n) of the host buffer base in slot; NULL when base is NULL (an optional input)
+    template <class T> T *in(int slot, const T *base, size_t off, size_t n) {
+        if (!base) return nullptr;
+        T *p = buf<T>(slot, n);
+        h2d(slot, p, base + off, n);
+        return p;
+    }
+    // n elements from the device to the host buffer dst
+    template <class T> void out(int slot, T *dst, const T *src, size_t n) {
+        const size_t bytes = n * sizeof(T);
+        void *to = dst;
+        if (bytes >= ZKP_STAGE_MIN && pageable(dst)) {
+            PinBuf &pb = d.pin_out[s][slot];
+            CUT(pb.ensure(bytes));
+            d.pend[s].push_back(PendingOut{dst, pb.p, bytes});
+            to = pb.p;
+        }
+        CUT(cudaMemcpyAsync(to, src, bytes, cudaMemcpyDeviceToHost, st));
+    }
+};
+using ChunkBody = std::function<void(Chunk &)>;
+using SliceFinish = std::function<void(DevState &, size_t lo, size_t hi)>;   // after the slice's streams have drained
+
+// Runs elements [lo,hi) of a call on device dev, chunk elements at a time, on two streams and buffer sets in turn:
+// the copies of one chunk overlap the kernels of the other.
+static int32_t run_slice(zkp_ctx *ctx, size_t dev, size_t lo, size_t hi, size_t chunk, const ChunkBody &body, const SliceFinish &finish,
+                         std::string &msg) {
+    DevState &d = ctx->devs[dev];
+    auto flush = [&](int set) {   // after that set's stream has drained
+        for (const PendingOut &o : d.pend[set]) memcpy(o.user, o.stage, o.bytes);
+        d.pend[set].clear();
+    };
+    try {
+        DeviceGuard guard;
+        CUT(cudaSetDevice(d.id));
+        CUT(cudaMemsetAsync(d.d_err, 0, sizeof(uint32_t), d.stream[0]));
+        CUT(cudaStreamSynchronize(d.stream[0]));
+        d.pend[0].clear();   // (a call that failed half-way leaves nothing behind for the next one)
+        d.pend[1].clear();
+        int s = 0;
+        for (size_t c0 = lo; c0 < hi; c0 += chunk, s ^= 1) {
+            Chunk c{ctx, d, dev, lo, hi, c0, hi - c0 < chunk ? hi - c0 : chunk, d.stream[s], s};
+            CUT(cudaStreamSynchronize(c.st));   // this buffer set's previous chunk is fully drained
+            flush(s);
+            body(c);
+        }
+        CUT(cudaStreamSynchronize(d.stream[0]));
+        flush(0);
+        CUT(cudaStreamSynchronize(d.stream[1]));
+        flush(1);
+        if (finish) finish(d, lo, hi);
+        uint32_t herr = 0;
+        CUT(cudaMemcpy(&herr, d.d_err, sizeof herr, cudaMemcpyDeviceToHost));
+        if (herr & 1) {
+            msg = "input limb vector >= p (non-canonical field element)";
+            return ZKP_ERR_NONCANONICAL;
+        }
+        return ZKP_OK;
+    } catch (const CudaFail &f) {
+        msg = f.msg;
+        return ZKP_ERR_CUDA;
+    }
+}
+
+// Runs [0,n) over the fan_out devices, one thread per device; the first failing device's error is returned.
+// The caller holds ctx->mu.
+static int32_t run_slices(zkp_ctx *ctx, size_t n, size_t chunk, const ChunkBody &body, const SliceFinish &finish = nullptr) {
+    const size_t nd = fan_out(ctx, n);
+    std::vector<int32_t> rcs(nd, ZKP_OK);
+    std::vector<std::string> msgs(nd);
+    auto run = [&](size_t di) {
+        size_t lo, hi;
+        slice_of(n, nd, di, lo, hi);
+        rcs[di] = run_slice(ctx, di, lo, hi, chunk, body, finish, msgs[di]);
+    };
+    if (nd == 1) {
+        run(0);
+    } else {
+        std::vector<std::thread> th;
+        for (size_t di = 0; di < nd; di++) th.emplace_back(run, di);
+        for (auto &t : th) t.join();
+    }
+    for (size_t di = 0; di < nd; di++)
+        if (rcs[di] != ZKP_OK) return fail(rcs[di], msgs[di]);
+    return ZKP_OK;
+}
+
+static int32_t run_host_job(zkp_ctx *ctx, size_t n, size_t chunk, const ChunkBody &body) {
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (n == 0) return ZKP_OK;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return run_slices(ctx, n, chunk, body);
 }
 
 extern "C" {
@@ -1224,14 +1377,11 @@ int32_t zkp_pairing_dev(zkp_ctx *ctx, int32_t dev, int32_t mode, const uint64_t 
     if ((mode & 1) && (!d_g1_xy || !d_g2_xy || pairs_per_check < 1)) return fail(ZKP_ERR_INVALID_ARG, "NULL point buffers");
     if (!(mode & 1) && !d_in_fp12) return fail(ZKP_ERR_INVALID_ARG, "NULL Fp12 input");
     if (pairs_per_check > ZKP_MAX_PAIRS_PER_CHECK) return fail(ZKP_ERR_TOO_MANY_PAIRS, "pairs_per_check > 8");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_pairing(ctx, d, mode, d_g1_xy, d_g1_inf, d_g2_xy, d_g2_inf, n_checks, (mode & 1) ? pairs_per_check : 1,
-                      d_in_fp12, d_out, d_is_one, d_err, st));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_pairing(ctx, d, mode, d_g1_xy, d_g1_inf, d_g2_xy, d_g2_inf, n_checks, (mode & 1) ? pairs_per_check : 1,
+                          d_in_fp12, d_out, d_is_one, d_err, st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_tower_op_dev(zkp_ctx *ctx, int32_t dev, int32_t op, const uint64_t *d_a, const uint64_t *d_b, uint64_t *d_out,
@@ -1241,17 +1391,14 @@ int32_t zkp_tower_op_dev(zkp_ctx *ctx, int32_t dev, int32_t op, const uint64_t *
     int na, nb, nr;
     tower_op_shape(op, na, nb, nr);
     if (!d_a || !d_out || (nb && !d_b)) return fail(ZKP_ERR_INVALID_ARG, "NULL operand");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    if (n) {
-        k_tower_op<<<grid_for(n), ZKP_TPB, 0, st>>>(op, d_a, d_b, d_out, d_status, d_err, n);
-        ctx->launches++;
-        CU(cudaGetLastError());
-    }
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        if (n) {
+            k_tower_op<<<grid_for(n), ZKP_TPB, 0, st>>>(op, d_a, d_b, d_out, d_status, d_err, n);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_fp12_product_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_in, size_t n, uint64_t *d_scratch,
@@ -1259,13 +1406,10 @@ int32_t zkp_fp12_product_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_in, si
     int32_t rc = check_dev(ctx, dev);
     if (rc) return rc;
     if (!d_in || !d_out || !d_scratch || n == 0) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer or n == 0");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_product(ctx, d_in, n, d_scratch, d_out, d_err, st));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_product(ctx, d_in, n, d_scratch, d_out, d_err, st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_gen_points_dev(zkp_ctx *ctx, int32_t dev, uint64_t seed, uint64_t first, size_t n, uint64_t *d_g1_xy,
@@ -1273,469 +1417,17 @@ int32_t zkp_gen_points_dev(zkp_ctx *ctx, int32_t dev, uint64_t seed, uint64_t fi
     int32_t rc = check_dev(ctx, dev);
     if (rc) return rc;
     if (!d_g1_xy || !d_g1_inf || !d_g2_xy || !d_g2_inf) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    if (n) {
-        k_gen_points<<<grid_for(n), ZKP_TPB, 0, st>>>(seed, first, n, d_g1_xy, d_g1_inf, d_g2_xy, d_g2_inf);
-        ctx->launches++;
-        CU(cudaGetLastError());
-    }
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        if (n) {
+            k_gen_points<<<grid_for(n), ZKP_TPB, 0, st>>>(seed, first, n, d_g1_xy, d_g1_inf, d_g2_xy, d_g2_inf);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        return ZKP_OK;
+    });
 }
 
 // ------------------------------------------------------------------ host-buffer entry points
-
-// Split [0,n) into one contiguous slice per device.
-static void slice_of(size_t n, size_t ndev, size_t d, size_t &lo, size_t &hi) {
-    lo = n * d / ndev;
-    hi = n * (d + 1) / ndev;
-}
-
-struct HostJob {
-    int mode = 0;   // 1 miller, 2 final exp, 3 pairing ; 16 = tower op ; 32 = gen points ; 48 = group op ; 64 = Miller product ; 80 = Groth16 ; 96 = KZG ; 112 = KZG blobs
-    const uint64_t *pts = nullptr, *scalars = nullptr;   // group op inputs (inf in g1inf, outputs in out / flags)
-    const uint64_t *tab = nullptr;                       // prepared G2 line tables shared by all checks (kf of them)
-    const uint8_t *tabinf = nullptr;
-    int kf = 0;
-    const uint64_t *g1 = nullptr, *g2 = nullptr, *in12 = nullptr, *a = nullptr, *b = nullptr;
-    const uint8_t *g1inf = nullptr, *g2inf = nullptr;
-    uint64_t *out = nullptr, *og1 = nullptr, *og2 = nullptr;
-    uint8_t *flags = nullptr, *og1inf = nullptr, *og2inf = nullptr;
-    int k = 1, op = 0;
-    int miller_mode = 1;   // mode 64: 1 = SURVEY 9.1 line scaling (the Miller product is returned), 5 = free scaling (only Gt is)
-    uint64_t seed = 0, first = 0;
-    const zkp_groth16_vk *vk = nullptr;   // mode 80 = Groth16 verification (proofs in pts, their flags in g1inf, inputs in scalars)
-    const zkp_kzg_setup *kzg = nullptr;   // mode 96 = KZG verification (proofs in pts, their flags in g1inf, z | y in scalars)
-    const uint8_t *blobs = nullptr;       // mode 112 = KZG blob verification (setup in kzg, proofs in pts, flags in g1inf, z | y out in out)
-    // modes 128 / 144 / 160 = commitments / proofs at z (z in scalars, y out in out) / blob proofs (commitments in pts, their
-    // flags in g1inf, z | y out in out): blobs in blobs, the points out in og1 / og1inf, the statuses in flags
-    // modes 176 / 192 = cells / cells and proofs: blobs in blobs, cells out in ocells, proofs in og1 / og1inf, statuses in flags.
-    // mode 208 = cell verification: commitments in pts (flags in g1inf), indices in idx, cells in cells, proofs in pi (flags in piinf)
-    // modes 224 / 240 = recovery / recovery with proofs: indices in idx, cells in cells, counts in scalars; outputs as 176 / 192
-    uint8_t *ocells = nullptr;
-    const uint8_t *cells = nullptr, *piinf = nullptr;
-    const uint64_t *idx = nullptr, *pi = nullptr;
-};
-
-// Runs elements [lo,hi) of a job on one device with a two-stage copy/compute pipeline.
-static int32_t run_slice(zkp_ctx *ctx, DevState &d, const HostJob &j, size_t lo, size_t hi, std::string &msg) {
-#define CUS(call)                                                                     \
-    do {                                                                              \
-        cudaError_t e_ = (call);                                                      \
-        if (e_ != cudaSuccess) {                                                      \
-            msg = std::string(#call) + ": " + cudaGetErrorString(e_);                 \
-            return ZKP_ERR_CUDA;                                                      \
-        }                                                                             \
-    } while (0)
-    DeviceGuard guard;
-    CUS(cudaSetDevice(d.id));
-    CUS(cudaMemsetAsync(d.d_err, 0, sizeof(uint32_t), d.stream[0]));
-    CUS(cudaStreamSynchronize(d.stream[0]));
-    int na = 0, nb = 0, nr = 0;
-    if (j.mode == 16) tower_op_shape(j.op, na, nb, nr);
-    size_t chunk = j.mode == 80    ? g16_chunk(j.vk->n_public)
-                   : j.mode == 176 ? (size_t)ZKP_CELLS_CHUNK
-                   : j.mode == 192 ? (size_t)ZKP_CELL_PROOF_CHUNK
-                   : j.mode == 208 ? (size_t)ZKP_CELL_VERIFY_CHUNK
-                   : j.mode == 224 ? (size_t)ZKP_CELLS_RECOVER_CHUNK
-                   : j.mode == 240 ? (size_t)ZKP_CELL_PROOF_CHUNK
-                   : j.mode >= 112 ? (size_t)ZKP_BLOB_CHUNK
-                                   : (size_t)ZKP_CHUNK;
-    int s = 0;
-    cudaStream_t st = nullptr;
-    d.pend[0].clear();   // (a job that failed half-way leaves nothing behind for the next one)
-    d.pend[1].clear();
-    if (j.mode == 64) CUS(d.partial.ensure(((hi - lo + chunk - 1) / chunk + 1) * 576));
-    auto pageable = [](const void *p) {
-        cudaPointerAttributes a;
-        if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-            cudaGetLastError();
-            return true;
-        }
-        return a.type == cudaMemoryTypeUnregistered;
-    };
-    auto h2d = [&](int which, void *dst, const void *src, size_t bytes) -> cudaError_t {
-        if (bytes >= ZKP_STAGE_MIN && pageable(src)) {
-            PinBuf &pb = d.pin_in[s][which];
-            cudaError_t e = pb.ensure(bytes);
-            if (e != cudaSuccess) return e;
-            memcpy(pb.p, src, bytes);
-            src = pb.p;
-        }
-        return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
-    };
-    auto d2h = [&](int which, void *dst, const void *src, size_t bytes) -> cudaError_t {
-        if (bytes >= ZKP_STAGE_MIN && pageable(dst)) {
-            PinBuf &pb = d.pin_out[s][which];
-            cudaError_t e = pb.ensure(bytes);
-            if (e != cudaSuccess) return e;
-            d.pend[s].push_back(PendingOut{dst, pb.p, bytes});
-            dst = pb.p;
-        }
-        return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
-    };
-    auto flush = [&](int set) {   // after that set's stream has drained
-        for (const PendingOut &o : d.pend[set]) memcpy(o.user, o.stage, o.bytes);
-        d.pend[set].clear();
-    };
-    for (size_t c0 = lo; c0 < hi; c0 += chunk, s ^= 1) {
-        size_t cn = hi - c0 < chunk ? hi - c0 : chunk;
-        st = d.stream[s];
-        DevBuf *B = d.buf[s];
-        CUS(cudaStreamSynchronize(st));   // this buffer set's previous chunk is fully drained
-        flush(s);
-        if (j.mode == 16) {
-            CUS(B[B_IN].ensure(cn * na * 48));
-            CUS(B[B_OUT].ensure(cn * nr * 48));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(h2d(B_IN, B[B_IN].p, j.a + c0 * na * 6, cn * na * 48));
-            if (nb) {
-                CUS(B[B_G2].ensure(cn * nb * 48));
-                CUS(h2d(B_G2, B[B_G2].p, j.b + c0 * nb * 6, cn * nb * 48));
-            }
-            k_tower_op<<<grid_for(cn), ZKP_TPB, 0, st>>>(j.op, (const uint64_t *)B[B_IN].p, nb ? (const uint64_t *)B[B_G2].p : nullptr,
-                                                        (uint64_t *)B[B_OUT].p, (uint8_t *)B[B_FLAG].p, d.d_err, cn);
-            ctx->launches++;
-            CUS(cudaGetLastError());
-            CUS(d2h(B_OUT, j.out + c0 * nr * 6, B[B_OUT].p, cn * nr * 48));
-            if (j.flags) CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode == 48) {
-            const size_t w = (j.op & 1) ? 24 : 12;
-            const bool is_mul = j.op >= GOP_G1_MUL;          // has a second operand and an output point
-            const bool is_add = j.op >= GOP_G1_ADD;
-            const size_t w2 = is_add ? w : 4;                 // u64 per element of the second operand
-            CUS(B[B_IN].ensure(cn * w * 8));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(h2d(B_IN, B[B_IN].p, j.pts + c0 * w, cn * w * 8));
-            const uint8_t *dinf = nullptr, *dinf2 = nullptr;
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
-                dinf = (const uint8_t *)B[B_G1INF].p;
-            }
-            if (is_add && j.g2inf) {
-                CUS(B[B_G2INF].ensure(cn));
-                CUS(h2d(B_G2INF, B[B_G2INF].p, j.g2inf + c0, cn));
-                dinf2 = (const uint8_t *)B[B_G2INF].p;
-            }
-            if (is_mul) {
-                CUS(B[B_G2].ensure(cn * w2 * 8));
-                CUS(B[B_OUT].ensure(cn * w * 8));
-                CUS(h2d(B_G2, B[B_G2].p, j.scalars + c0 * w2, cn * w2 * 8));
-            }
-            k_group_op<<<grid_for(cn), ZKP_TPB, 0, st>>>(j.op, (const uint64_t *)B[B_IN].p, dinf, is_mul ? (const uint64_t *)B[B_G2].p : nullptr,
-                                                        is_mul ? (uint64_t *)B[B_OUT].p : nullptr, (uint8_t *)B[B_FLAG].p, d.d_err, cn, dinf2);
-            ctx->launches++;
-            CUS(cudaGetLastError());
-            if (is_mul) CUS(d2h(B_OUT, j.out + c0 * w, B[B_OUT].p, cn * w * 8));
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode == 32) {
-            CUS(B[B_G1].ensure(cn * 96));
-            CUS(B[B_G2].ensure(cn * 192));
-            CUS(B[B_G1INF].ensure(cn));
-            CUS(B[B_G2INF].ensure(cn));
-            k_gen_points<<<grid_for(cn), ZKP_TPB, 0, st>>>(j.seed, j.first + c0, cn, (uint64_t *)B[B_G1].p, (uint8_t *)B[B_G1INF].p,
-                                                          (uint64_t *)B[B_G2].p, (uint8_t *)B[B_G2INF].p);
-            ctx->launches++;
-            CUS(cudaGetLastError());
-            CUS(d2h(B_G1, j.og1 + c0 * 12, B[B_G1].p, cn * 96));
-            CUS(d2h(B_G2, j.og2 + c0 * 24, B[B_G2].p, cn * 192));
-            CUS(d2h(B_G1INF, j.og1inf + c0, B[B_G1INF].p, cn));
-            CUS(d2h(B_G2INF, j.og2inf + c0, B[B_G2INF].p, cn));
-        } else if (j.mode == 64) {
-            // One product over all pairs of the slice: the pairs of a chunk are grouped four to a lane pair and
-            // run as shared-accumulator Miller loops (one Fp12 squaring chain per FOUR pairs: 4,684 instead of
-            // 6,916 Fp products per pair, SURVEY 8a), the chunk's outputs are folded to one Fp12 in
-            // d.partial[chunk].  Same two-stream pipeline as the independent pairings: the copies of one chunk
-            // overlap the kernels of the other; nothing returns to the host per chunk.
-            size_t ci = (c0 - lo) / chunk, nc4 = cn / ZKP_PRODUCT_GROUP, rem = cn % ZKP_PRODUCT_GROUP, ne = nc4 + (rem ? 1 : 0);
-            const uint8_t *di1 = nullptr, *di2 = nullptr;
-            CUS(B[B_G1].ensure(cn * 96));
-            CUS(B[B_G2].ensure(cn * 192));
-            CUS(B[B_OUT].ensure(ne * 576));
-            CUS(B[B_IN].ensure(zkp_product_scratch_elems(ne) * 576));   // this buffer set's product scratch
-            CUS(h2d(B_G1, B[B_G1].p, j.g1 + c0 * 12, cn * 96));
-            CUS(h2d(B_G2, B[B_G2].p, j.g2 + c0 * 24, cn * 192));
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
-                di1 = (const uint8_t *)B[B_G1INF].p;
-            }
-            if (j.g2inf) {
-                CUS(B[B_G2INF].ensure(cn));
-                CUS(h2d(B_G2INF, B[B_G2INF].p, j.g2inf + c0, cn));
-                di2 = (const uint8_t *)B[B_G2INF].p;
-            }
-            if (nc4)
-                CUS(launch_pairing(ctx, d, j.miller_mode, (const uint64_t *)B[B_G1].p, di1, (const uint64_t *)B[B_G2].p, di2, nc4, ZKP_PRODUCT_GROUP,
-                                   nullptr, (uint64_t *)B[B_OUT].p, nullptr, d.d_err, st));
-            if (rem) {
-                size_t o = nc4 * ZKP_PRODUCT_GROUP;
-                CUS(launch_pairing(ctx, d, j.miller_mode, (const uint64_t *)B[B_G1].p + 12 * o, di1 ? di1 + o : nullptr,
-                                   (const uint64_t *)B[B_G2].p + 24 * o, di2 ? di2 + o : nullptr, 1, (int)rem, nullptr,
-                                   (uint64_t *)B[B_OUT].p + 72 * nc4, nullptr, d.d_err, st));
-            }
-            CUS(launch_product(ctx, (const uint64_t *)B[B_OUT].p, ne, (uint64_t *)B[B_IN].p, (uint64_t *)d.partial.p + 72 * ci, d.d_err, st));
-        } else if (j.mode == 80) {
-            const G16Dev &kd = j.vk->devs[&d - ctx->devs.data()];
-            const size_t np = (size_t)j.vk->n_public;
-            const uint8_t *dpi = nullptr;
-            const uint64_t *dx = nullptr;
-            CUS(B[B_G1].ensure(cn * 384));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(B[B_OUT].ensure(g16_layout(cn, nullptr, nullptr)));
-            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 48, cn * 384));
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn * 3));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 3, cn * 3));
-                dpi = (const uint8_t *)B[B_G1INF].p;
-            }
-            if (np) {
-                CUS(B[B_IN].ensure(cn * np * 32));
-                CUS(h2d(B_IN, B[B_IN].p, j.scalars + c0 * np * 4, cn * np * 32));
-                dx = (const uint64_t *)B[B_IN].p;
-            }
-            CUS(launch_groth16(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, dx, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode == 112) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            const uint8_t *dpi = nullptr;
-            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
-            CUS(B[B_G1].ensure(cn * 192));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(B[B_OUT].ensure(zkp_kzg_blob_scratch_bytes(cn)));
-            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
-            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 24, cn * 192));
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn * 2));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 2, cn * 2));
-                dpi = (const uint8_t *)B[B_G1INF].p;
-            }
-            CUS(launch_kzg_blob(ctx, d, kd, (const uint8_t *)B[B_IN].p, (const uint64_t *)B[B_G1].p, dpi, cn, (uint8_t *)B[B_FLAG].p, nullptr,
-                                B[B_OUT].p, d.d_err, st));
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-            if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, B[B_OUT].p, cn * 64));   // z | y, first in the scratch
-        } else if (j.mode == 176 || j.mode == 192) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            const size_t cb = (size_t)ZKP_CELLS_PER_EXT_BLOB * ZKP_CELL_BYTES, np = cn * ZKP_CELLS_PER_EXT_BLOB;
-            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
-            CUS(B[B_G1].ensure(cn * cb));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
-            uint64_t *dpf = nullptr;
-            uint8_t *dpi = nullptr;
-            if (j.mode == 192) {
-                CUS(B[B_G2].ensure(np * 96));
-                CUS(B[B_G2INF].ensure(np));
-                CUS(B[B_OUT].ensure(zkp_kzg_cells_proofs_scratch_bytes(cn)));
-                dpf = (uint64_t *)B[B_G2].p;
-                dpi = (uint8_t *)B[B_G2INF].p;
-            }
-            CUS(launch_cells(ctx, kd, (const uint8_t *)B[B_IN].p, cn, (uint8_t *)B[B_G1].p, dpf, dpi, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, st));
-            CUS(d2h(B_G1, j.ocells + c0 * cb, B[B_G1].p, cn * cb));
-            if (j.mode == 192) {
-                CUS(d2h(B_G2, j.og1 + c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 96));
-                CUS(d2h(B_G2INF, j.og1inf + c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np));
-            }
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode == 224 || j.mode == 240) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            const size_t cb = (size_t)ZKP_CELLS_PER_EXT_BLOB * ZKP_CELL_BYTES, np = cn * ZKP_CELLS_PER_EXT_BLOB;
-            CUS(B[B_IN].ensure(cn * cb));
-            CUS(B[B_G1].ensure(cn * cb));
-            CUS(B[B_TAB].ensure(np * 8));
-            CUS(B[B_G1INF].ensure(cn * 8));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(h2d(B_IN, B[B_IN].p, j.cells + c0 * cb, cn * cb));
-            CUS(h2d(B_TAB, B[B_TAB].p, j.idx + c0 * ZKP_CELLS_PER_EXT_BLOB, np * 8));
-            CUS(h2d(B_G1INF, B[B_G1INF].p, j.scalars + c0, cn * 8));
-            uint64_t *dpf = nullptr;
-            uint8_t *dpi = nullptr;
-            if (j.mode == 240) {
-                CUS(B[B_G2].ensure(np * 96));
-                CUS(B[B_G2INF].ensure(np));
-                CUS(B[B_OUT].ensure(zkp_kzg_cells_proofs_scratch_bytes(cn)));
-                dpf = (uint64_t *)B[B_G2].p;
-                dpi = (uint8_t *)B[B_G2INF].p;
-            }
-            CUS(launch_cells_recover(ctx, kd, (const uint64_t *)B[B_TAB].p, (const uint8_t *)B[B_IN].p, (const uint64_t *)B[B_G1INF].p, cn,
-                                     (uint8_t *)B[B_G1].p, dpf, dpi, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, st));
-            CUS(d2h(B_G1, j.ocells + c0 * cb, B[B_G1].p, cn * cb));
-            if (j.mode == 240) {
-                CUS(d2h(B_G2, j.og1 + c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 96));
-                CUS(d2h(B_G2INF, j.og1inf + c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np));
-            }
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode == 208) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            const uint8_t *dci = nullptr, *dpi = nullptr;
-            CUS(B[B_G1].ensure(cn * 96));
-            CUS(B[B_G2].ensure(cn * 96));
-            CUS(B[B_TAB].ensure(cn * 8));
-            CUS(B[B_IN].ensure(cn * ZKP_CELL_BYTES));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(B[B_OUT].ensure(zkp_kzg_verify_cell_scratch_bytes(cn)));
-            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 12, cn * 96));
-            CUS(h2d(B_G2, B[B_G2].p, j.pi + c0 * 12, cn * 96));
-            CUS(h2d(B_TAB, B[B_TAB].p, j.idx + c0, cn * 8));
-            CUS(h2d(B_IN, B[B_IN].p, j.cells + c0 * ZKP_CELL_BYTES, cn * ZKP_CELL_BYTES));
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
-                dci = (const uint8_t *)B[B_G1INF].p;
-            }
-            if (j.piinf) {
-                CUS(B[B_G2INF].ensure(cn));
-                CUS(h2d(B_G2INF, B[B_G2INF].p, j.piinf + c0, cn));
-                dpi = (const uint8_t *)B[B_G2INF].p;
-            }
-            CUS(launch_cells_verify(ctx, d, kd, (const uint64_t *)B[B_G1].p, dci, (const uint64_t *)B[B_TAB].p, (const uint8_t *)B[B_IN].p,
-                                    (const uint64_t *)B[B_G2].p, dpi, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p, d.d_err, st));
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else if (j.mode >= 128) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            CUS(B[B_IN].ensure(cn * ZKP_BLOB_BYTES));
-            CUS(B[B_G2].ensure(cn * 96));
-            CUS(B[B_G2INF].ensure(cn));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(h2d(B_IN, B[B_IN].p, j.blobs + c0 * ZKP_BLOB_BYTES, cn * ZKP_BLOB_BYTES));
-            uint64_t *dout = (uint64_t *)B[B_G2].p;
-            uint8_t *dinf = (uint8_t *)B[B_G2INF].p, *dst = (uint8_t *)B[B_FLAG].p;
-            if (j.mode == 128) {
-                CUS(launch_kzg_commit(ctx, kd, (const uint8_t *)B[B_IN].p, cn, dout, dinf, dst, st));
-            } else {
-                CUS(B[B_OUT].ensure(zkp_kzg_prover_scratch_bytes(cn)));
-                uint64_t *dzy = (uint64_t *)((uint8_t *)B[B_OUT].p + prove_rows_bytes(cn));   // z | y, after the rows
-                const uint64_t *dz = nullptr, *dc = nullptr;
-                const uint8_t *dci = nullptr;
-                uint64_t *dy = nullptr;
-                if (j.mode == 144) {
-                    CUS(B[B_G1].ensure(cn * 32));
-                    CUS(B[B_TAB].ensure(cn * 32));
-                    CUS(h2d(B_G1, B[B_G1].p, j.scalars + c0 * 4, cn * 32));
-                    dz = (const uint64_t *)B[B_G1].p;
-                    dy = (uint64_t *)B[B_TAB].p;
-                } else {
-                    CUS(B[B_G1].ensure(cn * 96));
-                    CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 12, cn * 96));
-                    dc = (const uint64_t *)B[B_G1].p;
-                    if (j.g1inf) {
-                        CUS(B[B_G1INF].ensure(cn));
-                        CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0, cn));
-                        dci = (const uint8_t *)B[B_G1INF].p;
-                    }
-                }
-                CUS(launch_kzg_prove(ctx, kd, (const uint8_t *)B[B_IN].p, dz, dc, dci, cn, dout, dinf, dy, dzy, dst, B[B_OUT].p, st));
-                if (j.mode == 144) CUS(d2h(B_TAB, j.out + c0 * 4, dy, cn * 32));
-                else if (j.out) CUS(d2h(B_OUT, j.out + c0 * 8, dzy, cn * 64));
-            }
-            CUS(d2h(B_G2, j.og1 + c0 * 12, dout, cn * 96));
-            CUS(d2h(B_G2INF, j.og1inf + c0, dinf, cn));
-            CUS(d2h(B_FLAG, j.flags + c0, dst, cn));
-        } else if (j.mode == 96) {
-            const KzgDev &kd = j.kzg->devs[&d - ctx->devs.data()];
-            const uint8_t *dpi = nullptr;
-            CUS(B[B_G1].ensure(cn * 192));
-            CUS(B[B_IN].ensure(cn * 64));
-            CUS(B[B_FLAG].ensure(cn));
-            CUS(B[B_OUT].ensure(kzg_layout(cn, nullptr, nullptr)));
-            CUS(h2d(B_G1, B[B_G1].p, j.pts + c0 * 24, cn * 192));
-            CUS(h2d(B_IN, B[B_IN].p, j.scalars + c0 * 8, cn * 64));
-            if (j.g1inf) {
-                CUS(B[B_G1INF].ensure(cn * 2));
-                CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + c0 * 2, cn * 2));
-                dpi = (const uint8_t *)B[B_G1INF].p;
-            }
-            CUS(launch_kzg(ctx, d, kd, (const uint64_t *)B[B_G1].p, dpi, (const uint64_t *)B[B_IN].p, cn, (uint8_t *)B[B_FLAG].p, B[B_OUT].p,
-                           d.d_err, st));
-            CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        } else {
-            size_t np = cn * (size_t)j.k, p0 = c0 * (size_t)j.k;
-            size_t nq = cn * (size_t)(j.k - j.kf), q0 = c0 * (size_t)(j.k - j.kf);   // per-check G2 points
-            const uint8_t *di1 = nullptr, *di2 = nullptr, *dti = nullptr;
-            if (j.mode & 1) {
-                CUS(B[B_G1].ensure(np * 96));
-                CUS(B[B_G2].ensure(nq * 192 + 16));
-                CUS(h2d(B_G1, B[B_G1].p, j.g1 + p0 * 12, np * 96));
-                if (nq) CUS(h2d(B_G2, B[B_G2].p, j.g2 + q0 * 24, nq * 192));
-                if (j.kf) {
-                    size_t tb = (size_t)j.kf * ZKP_LINE_STEPS * 3 * 2 * sizeof(Fp);
-                    CUS(B[B_TAB].ensure(tb + 16));
-                    CUS(h2d(B_TAB, B[B_TAB].p, j.tab, tb));
-                    if (j.tabinf) {
-                        CUS(h2d(B_TABINF, (uint8_t *)B[B_TAB].p + tb, j.tabinf, j.kf));
-                        dti = (const uint8_t *)B[B_TAB].p + tb;
-                    }
-                }
-                if (j.g1inf) {
-                    CUS(B[B_G1INF].ensure(np));
-                    CUS(h2d(B_G1INF, B[B_G1INF].p, j.g1inf + p0, np));
-                    di1 = (const uint8_t *)B[B_G1INF].p;
-                }
-                if (j.g2inf && nq) {
-                    CUS(B[B_G2INF].ensure(nq));
-                    CUS(h2d(B_G2INF, B[B_G2INF].p, j.g2inf + q0, nq));
-                    di2 = (const uint8_t *)B[B_G2INF].p;
-                }
-            } else {
-                CUS(B[B_IN].ensure(cn * 576));
-                CUS(h2d(B_IN, B[B_IN].p, j.in12 + c0 * 72, cn * 576));
-            }
-            CUS(B[B_OUT].ensure(cn * 576));
-            if (j.flags) CUS(B[B_FLAG].ensure(cn));
-            CUS(launch_pairing(ctx, d, j.mode, (const uint64_t *)B[B_G1].p, di1, (const uint64_t *)B[B_G2].p, di2, cn, j.k,
-                               (const uint64_t *)B[B_IN].p, (uint64_t *)B[B_OUT].p, j.flags ? (uint8_t *)B[B_FLAG].p : nullptr,
-                               d.d_err, st, j.kf ? B[B_TAB].p : nullptr, dti, j.kf));
-            CUS(d2h(B_OUT, j.out + c0 * 72, B[B_OUT].p, cn * 576));
-            if (j.flags) CUS(d2h(B_FLAG, j.flags + c0, B[B_FLAG].p, cn));
-        }
-    }
-    CUS(cudaStreamSynchronize(d.stream[0]));
-    flush(0);
-    CUS(cudaStreamSynchronize(d.stream[1]));
-    flush(1);
-    if (j.mode == 64) {   // fold this device's chunk partials into the slot after the last one
-        size_t nchunks = (hi - lo + chunk - 1) / chunk;
-        CUS(d.buf[0][B_IN].ensure(zkp_product_scratch_elems(nchunks) * 576));
-        CUS(launch_product(ctx, (const uint64_t *)d.partial.p, nchunks, (uint64_t *)d.buf[0][B_IN].p,
-                           (uint64_t *)d.partial.p + 72 * nchunks, d.d_err, d.stream[0]));
-        CUS(cudaStreamSynchronize(d.stream[0]));
-    }
-    uint32_t herr = 0;
-    CUS(cudaMemcpy(&herr, d.d_err, sizeof herr, cudaMemcpyDeviceToHost));
-    if (herr & 1) {
-        msg = "input limb vector >= p (non-canonical field element)";
-        return ZKP_ERR_NONCANONICAL;
-    }
-    return ZKP_OK;
-#undef CUS
-}
-
-static int32_t run_host_job(zkp_ctx *ctx, const HostJob &j, size_t n) {
-    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
-    if (n == 0) return ZKP_OK;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    size_t nd = ctx->devs.size();
-    std::vector<int32_t> rcs(nd, ZKP_OK);
-    std::vector<std::string> msgs(nd);
-    if (nd == 1 || n < 2 * nd) {
-        rcs[0] = run_slice(ctx, ctx->devs[0], j, 0, n, msgs[0]);
-    } else {
-        std::vector<std::thread> th;
-        for (size_t d = 0; d < nd; d++) {
-            size_t lo, hi;
-            slice_of(n, nd, d, lo, hi);
-            th.emplace_back([&, d, lo, hi]() { rcs[d] = run_slice(ctx, ctx->devs[d], j, lo, hi, msgs[d]); });
-        }
-        for (auto &t : th) t.join();
-    }
-    for (size_t d = 0; d < nd; d++)
-        if (rcs[d] != ZKP_OK) return fail(rcs[d], msgs[d]);
-    return ZKP_OK;
-}
 
 int32_t zkp_tower_op_batch(zkp_ctx *ctx, int32_t op, const uint64_t *a, const uint64_t *b, uint64_t *out, uint8_t *status, size_t n) {
     int na, nb, nr;
@@ -1744,9 +1436,17 @@ int32_t zkp_tower_op_batch(zkp_ctx *ctx, int32_t op, const uint64_t *a, const ui
                  (op >= OP_FP12_ADD && op <= OP_FP12_POW);
     if (!known) return fail(ZKP_ERR_INVALID_ARG, "unknown tower op");
     if (n && (!a || !out || (nb && !b))) return fail(ZKP_ERR_INVALID_ARG, "NULL operand");
-    HostJob j;
-    j.mode = 16; j.op = op; j.a = a; j.b = b; j.out = out; j.flags = status;
-    return run_host_job(ctx, j, n);
+    return run_host_job(ctx, n, ZKP_CHUNK, [=](Chunk &c) {
+        const uint64_t *da = c.in(B_IN, a, c.c0 * na * 6, c.cn * na * 6);
+        uint64_t *dout = c.buf<uint64_t>(B_OUT, c.cn * nr * 6);
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        const uint64_t *db = c.in(B_G2, nb ? b : nullptr, c.c0 * nb * 6, c.cn * nb * 6);
+        k_tower_op<<<grid_for(c.cn), ZKP_TPB, 0, c.st>>>(op, da, db, dout, dst, c.d.d_err, c.cn);
+        ctx->launches++;
+        CUT(cudaGetLastError());
+        c.out(B_OUT, out + c.c0 * nr * 6, dout, c.cn * nr * 6);
+        if (status) c.out(B_FLAG, status + c.c0, dst, c.cn);
+    });
 }
 int32_t zkp_fp_mul_batch(zkp_ctx *ctx, const uint64_t *a, const uint64_t *b, uint64_t *out, size_t n) {
     return zkp_tower_op_batch(ctx, OP_FP_MUL, a, b, out, nullptr, n);
@@ -1789,40 +1489,82 @@ int32_t zkp_fp12_mul_by_014_batch(zkp_ctx *ctx, const uint64_t *f, const uint64_
     return zkp_tower_op_batch(ctx, OP_FP12_MUL_BY_014, f, c, out, nullptr, n);
 }
 
+// launch_pairing over host buffers: mode 1 (Miller loops) or 3 (pairings) of n checks of k pairs, the last kf of
+// each check from the kf shared prepared tables (flags tabinf), or mode 2 (final exponentiations of in12)
 static int32_t pairs_job(zkp_ctx *ctx, int mode, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf,
-                         size_t n, int32_t k, uint64_t *out, uint8_t *flags) {
+                         const uint64_t *in12, size_t n, int k, uint64_t *out, uint8_t *flags, const uint64_t *tab = nullptr,
+                         const uint8_t *tabinf = nullptr, int kf = 0) {
+    return run_host_job(ctx, n, ZKP_CHUNK, [=](Chunk &c) {
+        const size_t np = c.cn * (size_t)k, p0 = c.c0 * (size_t)k;
+        const size_t nq = c.cn * (size_t)(k - kf), q0 = c.c0 * (size_t)(k - kf);   // per-check G2 points
+        const uint64_t *dg1 = nullptr, *dg2 = nullptr, *din = nullptr;
+        const uint8_t *di1 = nullptr, *di2 = nullptr, *dti = nullptr;
+        const uint8_t *dtab = nullptr;
+        if (mode & 1) {
+            dg1 = c.in(B_G1, g1, p0 * 12, np * 12);
+            uint64_t *p2 = c.buf<uint64_t>(B_G2, nq * 24 + 2);
+            if (nq) c.h2d(B_G2, p2, g2 + q0 * 24, nq * 24);
+            dg2 = p2;
+            if (kf) {
+                const size_t tb = (size_t)kf * ZKP_LINE_STEPS * 3 * 2 * sizeof(Fp);
+                uint8_t *t = c.buf<uint8_t>(B_TAB, tb + 16);
+                c.h2d(B_TAB, t, (const uint8_t *)tab, tb);
+                if (tabinf) {
+                    c.h2d(B_TABINF, t + tb, tabinf, (size_t)kf);
+                    dti = t + tb;
+                }
+                dtab = t;
+            }
+            di1 = c.in(B_G1INF, g1inf, p0, np);
+            di2 = c.in(B_G2INF, nq ? g2inf : nullptr, q0, nq);
+        } else {
+            din = c.in(B_IN, in12, c.c0 * 72, c.cn * 72);
+        }
+        uint64_t *dout = c.buf<uint64_t>(B_OUT, c.cn * 72);
+        uint8_t *dflag = flags ? c.buf<uint8_t>(B_FLAG, c.cn) : nullptr;
+        CUT(launch_pairing(ctx, c.d, mode, dg1, di1, dg2, di2, c.cn, k, din, dout, dflag, c.d.d_err, c.st, dtab, dti, kf));
+        c.out(B_OUT, out + c.c0 * 72, dout, c.cn * 72);
+        if (flags) c.out(B_FLAG, flags + c.c0, dflag, c.cn);
+    });
+}
+static int32_t checks_job(zkp_ctx *ctx, int mode, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf,
+                          size_t n, int32_t k, uint64_t *out, uint8_t *flags) {
     if (k < 1) return fail(ZKP_ERR_INVALID_ARG, "pairs_per_check < 1");
     if (k > ZKP_MAX_PAIRS_PER_CHECK) return fail(ZKP_ERR_TOO_MANY_PAIRS, "pairs_per_check > 8 (use zkp_multi_miller_product)");
     if (n && (!g1 || !g2 || !out)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = mode; j.g1 = g1; j.g1inf = g1inf; j.g2 = g2; j.g2inf = g2inf; j.k = k; j.out = out; j.flags = flags;
-    return run_host_job(ctx, j, n);
+    return pairs_job(ctx, mode, g1, g1inf, g2, g2inf, nullptr, n, k, out, flags);
 }
 int32_t zkp_miller_loop_batch(zkp_ctx *ctx, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf, size_t n, uint64_t *out) {
-    return pairs_job(ctx, 1, g1, g1inf, g2, g2inf, n, 1, out, nullptr);
+    return checks_job(ctx, 1, g1, g1inf, g2, g2inf, n, 1, out, nullptr);
 }
 int32_t zkp_pairing_batch(zkp_ctx *ctx, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf, size_t n, uint64_t *out) {
-    return pairs_job(ctx, 3, g1, g1inf, g2, g2inf, n, 1, out, nullptr);
+    return checks_job(ctx, 3, g1, g1inf, g2, g2inf, n, 1, out, nullptr);
 }
 int32_t zkp_multi_miller_loop_batch(zkp_ctx *ctx, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf,
                                     size_t n_checks, int32_t k, uint64_t *out) {
-    return pairs_job(ctx, 1, g1, g1inf, g2, g2inf, n_checks, k, out, nullptr);
+    return checks_job(ctx, 1, g1, g1inf, g2, g2inf, n_checks, k, out, nullptr);
 }
 int32_t zkp_multi_pairing_batch(zkp_ctx *ctx, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf,
                                 size_t n_checks, int32_t k, uint64_t *out, uint8_t *is_one) {
-    return pairs_job(ctx, 3, g1, g1inf, g2, g2inf, n_checks, k, out, is_one);
+    return checks_job(ctx, 3, g1, g1inf, g2, g2inf, n_checks, k, out, is_one);
 }
 int32_t zkp_final_exp_batch(zkp_ctx *ctx, const uint64_t *in, size_t n, uint64_t *out) {
     if (n && (!in || !out)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 2; j.in12 = in; j.out = out;
-    return run_host_job(ctx, j, n);
+    return pairs_job(ctx, 2, nullptr, nullptr, nullptr, nullptr, in, n, 1, out, nullptr);
 }
 int32_t zkp_gen_points(zkp_ctx *ctx, uint64_t seed, uint64_t first, size_t n, uint64_t *g1, uint8_t *g1inf, uint64_t *g2, uint8_t *g2inf) {
     if (n && (!g1 || !g1inf || !g2 || !g2inf)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 32; j.seed = seed; j.first = first; j.og1 = g1; j.og1inf = g1inf; j.og2 = g2; j.og2inf = g2inf;
-    return run_host_job(ctx, j, n);
+    return run_host_job(ctx, n, ZKP_CHUNK, [=](Chunk &c) {
+        uint64_t *d1 = c.buf<uint64_t>(B_G1, c.cn * 12), *d2 = c.buf<uint64_t>(B_G2, c.cn * 24);
+        uint8_t *d1i = c.buf<uint8_t>(B_G1INF, c.cn), *d2i = c.buf<uint8_t>(B_G2INF, c.cn);
+        k_gen_points<<<grid_for(c.cn), ZKP_TPB, 0, c.st>>>(seed, first + c.c0, c.cn, d1, d1i, d2, d2i);
+        ctx->launches++;
+        CUT(cudaGetLastError());
+        c.out(B_G1, g1 + c.c0 * 12, d1, c.cn * 12);
+        c.out(B_G2, g2 + c.c0 * 24, d2, c.cn * 24);
+        c.out(B_G1INF, g1inf + c.c0, d1i, c.cn);
+        c.out(B_G2INF, g2inf + c.c0, d2i, c.cn);
+    });
 }
 
 // ---- prepared G2 points (SURVEY 8f-4)
@@ -1855,17 +1597,14 @@ int32_t zkp_g2_prepare_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g2_xy, s
     int32_t rc = check_dev(ctx, dev);
     if (rc) return rc;
     if (n && (!d_g2_xy || !d_out_tables)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    if (n) {
-        k_g2_prepare<<<grid_for(n), ZKP_TPB, 0, st>>>(d_g2_xy, (Fp *)d_out_tables, d_err, n);
-        ctx->launches++;
-        CU(cudaGetLastError());
-    }
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        if (n) {
+            k_g2_prepare<<<grid_for(n), ZKP_TPB, 0, st>>>(d_g2_xy, (Fp *)d_out_tables, d_err, n);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        return ZKP_OK;
+    });
 }
 int32_t zkp_multi_pairing_prepared_batch(zkp_ctx *ctx, const uint64_t *g1, const uint8_t *g1inf, const uint64_t *g2, const uint8_t *g2inf,
                                          size_t n_checks, int32_t k, const uint64_t *tables, const uint8_t *tables_inf, int32_t kf,
@@ -1873,10 +1612,7 @@ int32_t zkp_multi_pairing_prepared_batch(zkp_ctx *ctx, const uint64_t *g1, const
     if (k < 1 || kf < 0 || kf > k) return fail(ZKP_ERR_INVALID_ARG, "need 0 <= prepared pairs <= pairs_per_check");
     if (k > ZKP_MAX_PAIRS_PER_CHECK) return fail(ZKP_ERR_TOO_MANY_PAIRS, "pairs_per_check > 8");
     if (n_checks && (!g1 || !out || (kf < k && !g2) || (kf && !tables))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 3; j.g1 = g1; j.g1inf = g1inf; j.g2 = g2; j.g2inf = g2inf; j.k = k; j.out = out; j.flags = is_one;
-    j.tab = tables; j.tabinf = tables_inf; j.kf = kf;
-    return run_host_job(ctx, j, n_checks);
+    return pairs_job(ctx, 3, g1, g1inf, g2, g2inf, nullptr, n_checks, k, out, is_one, tables, tables_inf, kf);
 }
 int32_t zkp_multi_pairing_prepared_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g1, const uint8_t *d_g1inf, const uint64_t *d_g2,
                                        const uint8_t *d_g2inf, size_t n_checks, int32_t k, const uint64_t *d_tables,
@@ -1886,13 +1622,10 @@ int32_t zkp_multi_pairing_prepared_dev(zkp_ctx *ctx, int32_t dev, const uint64_t
     if (rc) return rc;
     if (k < 1 || kf < 0 || kf > k || k > ZKP_MAX_PAIRS_PER_CHECK) return fail(ZKP_ERR_INVALID_ARG, "bad pairs_per_check / prepared count");
     if (!d_g1 || !d_out || (kf < k && !d_g2) || (kf && !d_tables)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_pairing(ctx, d, 3, d_g1, d_g1inf, d_g2, d_g2inf, n_checks, k, nullptr, d_out, d_is_one, d_err, st, d_tables, d_tables_inf, kf));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_pairing(ctx, d, 3, d_g1, d_g1inf, d_g2, d_g2inf, n_checks, k, nullptr, d_out, d_is_one, d_err, st, d_tables, d_tables_inf, kf));
+        return ZKP_OK;
+    });
 }
 
 // bytes <-> limbs on device-resident buffers (dir 0: from_bytes, 1: to_bytes)
@@ -1901,17 +1634,14 @@ int32_t zkp_fp_bytes_dev(zkp_ctx *ctx, int32_t dev, int32_t dir, const void *d_i
     if (rc) return rc;
     if (n && (!d_in || !d_out)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_in | (uintptr_t)d_out) & 15) return fail(ZKP_ERR_INVALID_ARG, "buffers must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    if (n) {
-        k_fp_bytes<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dir, (const uint4 *)d_in, (uint4 *)d_out, d_ok, n);
-        ctx->launches++;
-        CU(cudaGetLastError());
-    }
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        if (n) {
+            k_fp_bytes<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dir, (const uint4 *)d_in, (uint4 *)d_out, d_ok, n);
+            ctx->launches++;
+            CU(cudaGetLastError());
+        }
+        return ZKP_OK;
+    });
 }
 static int32_t bytes_job(zkp_ctx *ctx, int dir, const void *in, void *out, uint8_t *ok, size_t n) {
     if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
@@ -1950,9 +1680,27 @@ int32_t zkp_fp_to_bytes_batch(zkp_ctx *ctx, const uint64_t *limbs, size_t n, uin
 static int32_t group_job(zkp_ctx *ctx, int gop, const uint64_t *pts, const uint8_t *inf, const uint64_t *scalars, size_t n,
                          uint64_t *out, uint8_t *flags, const uint8_t *inf2 = nullptr) {
     if (n && (!pts || !flags || (gop >= GOP_G1_MUL && (!scalars || !out)))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 48; j.op = gop; j.pts = pts; j.g1inf = inf; j.g2inf = inf2; j.scalars = scalars; j.out = out; j.flags = flags;
-    return run_host_job(ctx, j, n);
+    const size_t w = (gop & 1) ? 24 : 12;
+    const bool is_mul = gop >= GOP_G1_MUL;   // has a second operand and an output point
+    const bool is_add = gop >= GOP_G1_ADD;
+    const size_t w2 = is_add ? w : 4;        // u64 per element of the second operand
+    return run_host_job(ctx, n, ZKP_CHUNK, [=](Chunk &c) {
+        const uint64_t *dp = c.in(B_IN, pts, c.c0 * w, c.cn * w);
+        uint8_t *dflag = c.buf<uint8_t>(B_FLAG, c.cn);
+        const uint8_t *dinf = c.in(B_G1INF, inf, c.c0, c.cn);
+        const uint8_t *dinf2 = c.in(B_G2INF, is_add ? inf2 : nullptr, c.c0, c.cn);
+        const uint64_t *dsc = nullptr;
+        uint64_t *dout = nullptr;
+        if (is_mul) {
+            dsc = c.in(B_G2, scalars, c.c0 * w2, c.cn * w2);
+            dout = c.buf<uint64_t>(B_OUT, c.cn * w);
+        }
+        k_group_op<<<grid_for(c.cn), ZKP_TPB, 0, c.st>>>(gop, dp, dinf, dsc, dout, dflag, c.d.d_err, c.cn, dinf2);
+        ctx->launches++;
+        CUT(cudaGetLastError());
+        if (is_mul) c.out(B_OUT, out + c.c0 * w, dout, c.cn * w);
+        c.out(B_FLAG, flags + c.c0, dflag, c.cn);
+    });
 }
 int32_t zkp_g1_add_batch(zkp_ctx *ctx, const uint64_t *a_xy, const uint8_t *a_inf, const uint64_t *b_xy, const uint8_t *b_inf, size_t n,
                          uint64_t *out_xy, uint8_t *out_flag) {
@@ -1985,27 +1733,39 @@ int32_t zkp_multi_miller_product(zkp_ctx *ctx, const uint64_t *g1, const uint8_t
     if (!g1 || !g2 || n == 0) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer or n == 0");
     std::lock_guard<std::mutex> lk(ctx->mu);
     DeviceGuard guard;
-    size_t nd = ctx->devs.size();
-    if (n < 2 * nd) nd = 1;
-    HostJob j;
-    j.mode = 64; j.g1 = g1; j.g1inf = g1inf; j.g2 = g2; j.g2inf = g2inf;
-    j.miller_mode = out_miller_product ? 1 : 5;   // the un-exponentiated product is only well defined with SURVEY 9.1's lines
-    std::vector<int32_t> rcs(nd, ZKP_OK);
-    std::vector<std::string> msgs(nd);
-    if (nd == 1) {
-        rcs[0] = run_slice(ctx, ctx->devs[0], j, 0, n, msgs[0]);
-    } else {
-        std::vector<std::thread> th;
-        for (size_t di = 0; di < nd; di++) {
-            size_t lo, hi;
-            slice_of(n, nd, di, lo, hi);
-            th.emplace_back([&, di, lo, hi]() { rcs[di] = run_slice(ctx, ctx->devs[di], j, lo, hi, msgs[di]); });
+    const size_t chunk = ZKP_CHUNK;
+    const int miller_mode = out_miller_product ? 1 : 5;   // the un-exponentiated product is only well defined with SURVEY 9.1's lines
+    // One product over all pairs of the slice: the pairs of a chunk are grouped four to a lane pair and run as
+    // shared-accumulator Miller loops (one Fp12 squaring chain per FOUR pairs: 4,684 instead of 6,916 Fp products
+    // per pair, SURVEY 8a), the chunk's outputs are folded to one Fp12 in d.partial[chunk].  Nothing returns to the
+    // host per chunk.
+    auto body = [=](Chunk &c) {
+        DevState &d = c.d;
+        if (c.c0 == c.lo) CUT(d.partial.ensure(((c.hi - c.lo + chunk - 1) / chunk + 1) * 576));   // the partials and their fold
+        const size_t ci = (c.c0 - c.lo) / chunk, nc4 = c.cn / ZKP_PRODUCT_GROUP, rem = c.cn % ZKP_PRODUCT_GROUP, ne = nc4 + (rem ? 1 : 0);
+        const uint64_t *dg1 = c.in(B_G1, g1, c.c0 * 12, c.cn * 12), *dg2 = c.in(B_G2, g2, c.c0 * 24, c.cn * 24);
+        uint64_t *dout = c.buf<uint64_t>(B_OUT, ne * 72);
+        uint64_t *dscr = c.buf<uint64_t>(B_IN, zkp_product_scratch_elems(ne) * 72);   // this buffer set's product scratch
+        const uint8_t *di1 = c.in(B_G1INF, g1inf, c.c0, c.cn), *di2 = c.in(B_G2INF, g2inf, c.c0, c.cn);
+        if (nc4) CUT(launch_pairing(ctx, d, miller_mode, dg1, di1, dg2, di2, nc4, ZKP_PRODUCT_GROUP, nullptr, dout, nullptr, d.d_err, c.st));
+        if (rem) {
+            const size_t o = nc4 * ZKP_PRODUCT_GROUP;
+            CUT(launch_pairing(ctx, d, miller_mode, dg1 + 12 * o, di1 ? di1 + o : nullptr, dg2 + 24 * o, di2 ? di2 + o : nullptr, 1, (int)rem,
+                               nullptr, dout + 72 * nc4, nullptr, d.d_err, c.st));
         }
-        for (auto &t : th) t.join();
-    }
-    for (size_t di = 0; di < nd; di++)
-        if (rcs[di] != ZKP_OK) return fail(rcs[di], msgs[di]);
+        CUT(launch_product(ctx, dout, ne, dscr, (uint64_t *)d.partial.p + 72 * ci, d.d_err, c.st));
+    };
+    auto fold = [=](DevState &d, size_t lo, size_t hi) {   // this device's chunk partials into the slot after the last one
+        const size_t nchunks = (hi - lo + chunk - 1) / chunk;
+        CUT(d.buf[0][B_IN].ensure(zkp_product_scratch_elems(nchunks) * 576));
+        CUT(launch_product(ctx, (const uint64_t *)d.partial.p, nchunks, (uint64_t *)d.buf[0][B_IN].p, (uint64_t *)d.partial.p + 72 * nchunks,
+                           d.d_err, d.stream[0]));
+        CUT(cudaStreamSynchronize(d.stream[0]));
+    };
+    int32_t rc = run_slices(ctx, n, chunk, body, fold);
+    if (rc != ZKP_OK) return rc;
     // gather: one 576-byte partial per device -> first device (peer copy over NVLink when available)
+    const size_t nd = fan_out(ctx, n);
     DevState &d0 = ctx->devs[0];
     CU(cudaSetDevice(d0.id));
     DevBuf &G = d0.buf[1][B_IN];
@@ -2014,7 +1774,7 @@ int32_t zkp_multi_miller_product(zkp_ctx *ctx, const uint64_t *g1, const uint8_t
         DevState &d = ctx->devs[di];
         size_t lo, hi;
         slice_of(n, nd, di, lo, hi);
-        size_t nchunks = (hi - lo + ZKP_CHUNK - 1) / ZKP_CHUNK;
+        size_t nchunks = (hi - lo + chunk - 1) / chunk;
         const uint64_t *src = (const uint64_t *)d.partial.p + 72 * nchunks;
         if (d.id == d0.id)
             CU(cudaMemcpyAsync((uint64_t *)G.p + 72 * di, src, 576, cudaMemcpyDeviceToDevice, d0.stream[0]));
@@ -2139,9 +1899,16 @@ int32_t zkp_groth16_verify_batch(zkp_ctx *ctx, const zkp_groth16_vk *vk, const u
     if (!ctx || !vk) return fail(ZKP_ERR_INVALID_ARG, "ctx or vk is NULL");
     if (vk->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the verifying key belongs to another context");
     if (n && (!proofs || !out_status || (vk->n_public && !public_inputs))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 80; j.vk = vk; j.pts = proofs; j.g1inf = proof_inf; j.scalars = public_inputs; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    const size_t np = (size_t)vk->n_public;
+    return run_host_job(ctx, n, g16_chunk(vk->n_public), [=](Chunk &c) {
+        const uint64_t *dp = c.in(B_G1, proofs, c.c0 * 48, c.cn * 48);
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        uint8_t *dscr = c.buf<uint8_t>(B_OUT, g16_layout(c.cn, nullptr, nullptr));
+        const uint8_t *dpi = c.in(B_G1INF, proof_inf, c.c0 * 3, c.cn * 3);
+        const uint64_t *dx = c.in(B_IN, np ? public_inputs : nullptr, c.c0 * np * 4, c.cn * np * 4);
+        CUT(launch_groth16(ctx, c.d, vk->devs[c.dev], dp, dpi, dx, c.cn, dst, dscr, c.d.d_err, c.st));
+        c.out(B_FLAG, out_status + c.c0, dst, c.cn);
+    });
 }
 
 int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *vk, const uint64_t *d_proofs,
@@ -2153,13 +1920,10 @@ int32_t zkp_groth16_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_groth16_vk *
     if (vk->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the verifying key belongs to another context");
     if (n && (!d_proofs || !d_status || !d_scratch || (vk->n_public && !d_public_inputs))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if ((uintptr_t)d_scratch & 15) return fail(ZKP_ERR_INVALID_ARG, "d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_groth16(ctx, d, vk->devs[dev], d_proofs, d_proof_inf, d_public_inputs, n, d_status, d_scratch, nullptr, st));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_groth16(ctx, d, vk->devs[dev], d_proofs, d_proof_inf, d_public_inputs, n, d_status, d_scratch, nullptr, st));
+        return ZKP_OK;
+    });
 }
 
 // ---- KZG point-evaluation verification
@@ -2320,9 +2084,14 @@ int32_t zkp_kzg_verify_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_
     if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
     if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
     if (n && (!proofs || !zy || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 96; j.kzg = s; j.pts = proofs; j.g1inf = proof_inf; j.scalars = zy; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return run_host_job(ctx, n, ZKP_CHUNK, [=](Chunk &c) {
+        const uint64_t *dp = c.in(B_G1, proofs, c.c0 * 24, c.cn * 24), *dzy = c.in(B_IN, zy, c.c0 * 8, c.cn * 8);
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        uint8_t *dscr = c.buf<uint8_t>(B_OUT, kzg_layout(c.cn, nullptr, nullptr));
+        const uint8_t *dpi = c.in(B_G1INF, proof_inf, c.c0 * 2, c.cn * 2);
+        CUT(launch_kzg(ctx, c.d, s->devs[c.dev], dp, dpi, dzy, c.cn, dst, dscr, c.d.d_err, c.st));
+        c.out(B_FLAG, out_status + c.c0, dst, c.cn);
+    });
 }
 
 int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_proofs, const uint8_t *d_proof_inf,
@@ -2333,13 +2102,10 @@ int32_t zkp_kzg_verify_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, co
     if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
     if (n && (!d_proofs || !d_zy || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if ((uintptr_t)d_scratch & 15) return fail(ZKP_ERR_INVALID_ARG, "d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_kzg(ctx, d, s->devs[dev], d_proofs, d_proof_inf, d_zy, n, d_status, d_scratch, nullptr, st));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_kzg(ctx, d, s->devs[dev], d_proofs, d_proof_inf, d_zy, n, d_status, d_scratch, nullptr, st));
+        return ZKP_OK;
+    });
 }
 
 // ---- EIP-4844 blob verification
@@ -2349,9 +2115,16 @@ int32_t zkp_kzg_verify_blob_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const ui
     if (!ctx || !s) return fail(ZKP_ERR_INVALID_ARG, "ctx or setup is NULL");
     if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
     if (n && (!blobs || !proofs || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 112; j.kzg = s; j.blobs = blobs; j.pts = proofs; j.g1inf = proof_inf; j.flags = out_status; j.out = out_zy;
-    return run_host_job(ctx, j, n);
+    return run_host_job(ctx, n, ZKP_BLOB_CHUNK, [=](Chunk &c) {
+        const uint8_t *db = c.in(B_IN, blobs, c.c0 * ZKP_BLOB_BYTES, c.cn * ZKP_BLOB_BYTES);
+        const uint64_t *dp = c.in(B_G1, proofs, c.c0 * 24, c.cn * 24);
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        uint8_t *dscr = c.buf<uint8_t>(B_OUT, zkp_kzg_blob_scratch_bytes(c.cn));
+        const uint8_t *dpi = c.in(B_G1INF, proof_inf, c.c0 * 2, c.cn * 2);
+        CUT(launch_kzg_blob(ctx, c.d, s->devs[c.dev], db, dp, dpi, c.cn, dst, nullptr, dscr, c.d.d_err, c.st));
+        c.out(B_FLAG, out_status + c.c0, dst, c.cn);
+        if (out_zy) c.out(B_OUT, out_zy + c.c0 * 8, (const uint64_t *)dscr, c.cn * 8);   // z | y, first in the scratch
+    });
 }
 
 int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_proofs,
@@ -2362,13 +2135,10 @@ int32_t zkp_kzg_verify_blob_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *
     if (s->ctx != ctx) return fail(ZKP_ERR_INVALID_ARG, "the KZG setup belongs to another context");
     if (n && (!d_blobs || !d_proofs || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream (CUDA convention)
-    CU(launch_kzg_blob(ctx, d, s->devs[dev], d_blobs, d_proofs, d_proof_inf, n, d_status, d_out_zy, d_scratch, nullptr, st));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_kzg_blob(ctx, d, s->devs[dev], d_blobs, d_proofs, d_proof_inf, n, d_status, d_out_zy, d_scratch, nullptr, st));
+        return ZKP_OK;
+    });
 }
 
 // ---- EIP-4844 prover
@@ -2380,14 +2150,46 @@ static int32_t check_prover(zkp_ctx *ctx, const zkp_kzg_setup *s) {
     return ZKP_OK;
 }
 
+// The three prover calls over host buffers: commitments (z and c NULL), proofs at z (y to y_out) or blob proofs for
+// the commitments c (flags cinf or NULL; z | y to zy_out when it is not NULL)
+static int32_t prover_job(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *z, const uint64_t *c_pts,
+                          const uint8_t *cinf, size_t n, uint64_t *out, uint8_t *out_inf, uint64_t *y_out, uint8_t *status, uint64_t *zy_out) {
+    return run_host_job(ctx, n, ZKP_BLOB_CHUNK, [=](Chunk &c) {
+        const KzgDev &kd = s->devs[c.dev];
+        const uint8_t *db = c.in(B_IN, blobs, c.c0 * ZKP_BLOB_BYTES, c.cn * ZKP_BLOB_BYTES);
+        uint64_t *dout = c.buf<uint64_t>(B_G2, c.cn * 12);
+        uint8_t *dinf = c.buf<uint8_t>(B_G2INF, c.cn), *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        if (!z && !c_pts) {
+            CUT(launch_kzg_commit(ctx, kd, db, c.cn, dout, dinf, dst, c.st));
+        } else {
+            uint8_t *dscr = c.buf<uint8_t>(B_OUT, zkp_kzg_prover_scratch_bytes(c.cn));
+            uint64_t *dzy = (uint64_t *)(dscr + prove_rows_bytes(c.cn));   // z | y, after the rows
+            const uint64_t *dz = nullptr, *dc = nullptr;
+            const uint8_t *dci = nullptr;
+            uint64_t *dy = nullptr;
+            if (z) {
+                dz = c.in(B_G1, z, c.c0 * 4, c.cn * 4);
+                dy = c.buf<uint64_t>(B_TAB, c.cn * 4);
+            } else {
+                dc = c.in(B_G1, c_pts, c.c0 * 12, c.cn * 12);
+                dci = c.in(B_G1INF, cinf, c.c0, c.cn);
+            }
+            CUT(launch_kzg_prove(ctx, kd, db, dz, dc, dci, c.cn, dout, dinf, dy, dzy, dst, dscr, c.st));
+            if (z) c.out(B_TAB, y_out + c.c0 * 4, dy, c.cn * 4);
+            else if (zy_out) c.out(B_OUT, zy_out + c.c0 * 8, dzy, c.cn * 8);
+        }
+        c.out(B_G2, out + c.c0 * 12, dout, c.cn * 12);
+        c.out(B_G2INF, out_inf + c.c0, dinf, c.cn);
+        c.out(B_FLAG, status + c.c0, dst, c.cn);
+    });
+}
+
 int32_t zkp_kzg_blob_to_commitment_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint64_t *out_c,
                                          uint8_t *out_c_inf, uint8_t *out_status) {
     int32_t rc = check_prover(ctx, s);
     if (rc) return rc;
     if (n && (!blobs || !out_c || !out_c_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 128; j.kzg = s; j.blobs = blobs; j.og1 = out_c; j.og1inf = out_c_inf; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return prover_job(ctx, s, blobs, nullptr, nullptr, nullptr, n, out_c, out_c_inf, nullptr, out_status, nullptr);
 }
 
 int32_t zkp_kzg_compute_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *z, size_t n,
@@ -2395,10 +2197,7 @@ int32_t zkp_kzg_compute_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const 
     int32_t rc = check_prover(ctx, s);
     if (rc) return rc;
     if (n && (!blobs || !z || !out_proof || !out_proof_inf || !out_y || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 144; j.kzg = s; j.blobs = blobs; j.scalars = z; j.og1 = out_proof; j.og1inf = out_proof_inf; j.out = out_y;
-    j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return prover_job(ctx, s, blobs, z, nullptr, nullptr, n, out_proof, out_proof_inf, out_y, out_status, nullptr);
 }
 
 int32_t zkp_kzg_compute_blob_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *commitments,
@@ -2407,10 +2206,7 @@ int32_t zkp_kzg_compute_blob_proof_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, c
     int32_t rc = check_prover(ctx, s);
     if (rc) return rc;
     if (n && (!blobs || !commitments || !out_proof || !out_proof_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 160; j.kzg = s; j.blobs = blobs; j.pts = commitments; j.g1inf = commitment_inf; j.og1 = out_proof; j.og1inf = out_proof_inf;
-    j.flags = out_status; j.out = out_zy;
-    return run_host_job(ctx, j, n);
+    return prover_job(ctx, s, blobs, nullptr, commitments, commitment_inf, n, out_proof, out_proof_inf, nullptr, out_status, out_zy);
 }
 
 int32_t zkp_kzg_blob_to_commitment_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
@@ -2420,12 +2216,10 @@ int32_t zkp_kzg_blob_to_commitment_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_
     if (rc) return rc;
     if (n && (!d_blobs || !d_c || !d_c_inf || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if ((uintptr_t)d_blobs & 15) return fail(ZKP_ERR_INVALID_ARG, "d_blobs must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    CU(launch_kzg_commit(ctx, s->devs[dev], d_blobs, n, d_c, d_c_inf, d_status, (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_kzg_commit(ctx, s->devs[dev], d_blobs, n, d_c, d_c_inf, d_status, st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_kzg_compute_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_z, size_t n,
@@ -2436,13 +2230,11 @@ int32_t zkp_kzg_compute_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup
     if (n && (!d_blobs || !d_z || !d_proof || !d_proof_inf || !d_y || !d_status || !d_scratch))
         return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, d_z, nullptr, nullptr, n, d_proof, d_proof_inf, d_y, nullptr, d_status, d_scratch,
-                        (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, d_z, nullptr, nullptr, n, d_proof, d_proof_inf, d_y, nullptr, d_status, d_scratch,
+                            st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, const uint64_t *d_commitments,
@@ -2454,13 +2246,11 @@ int32_t zkp_kzg_compute_blob_proof_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_
     if (n && (!d_blobs || !d_commitments || !d_proof || !d_proof_inf || !d_status || !d_scratch))
         return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_scratch & 15) || ((uintptr_t)d_blobs & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, nullptr, d_commitments, d_commitment_inf, n, d_proof, d_proof_inf, nullptr, d_out_zy,
-                        d_status, d_scratch, (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_kzg_prove(ctx, s->devs[dev], d_blobs, nullptr, d_commitments, d_commitment_inf, n, d_proof, d_proof_inf, nullptr, d_out_zy,
+                            d_status, d_scratch, st));
+        return ZKP_OK;
+    });
 }
 
 // ---- EIP-7594 cells
@@ -2597,14 +2387,52 @@ static int32_t check_cells(zkp_ctx *ctx, const zkp_kzg_setup *s) {
     return ZKP_OK;
 }
 
+// The cells of n blobs over host buffers, from the blobs or (blobs NULL) recovered from each blob's 128 indices, 128
+// cells and count; with the proofs when proofs is not NULL
+static int32_t cells_job(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, const uint64_t *idx, const uint8_t *cells,
+                         const uint64_t *num, size_t n, uint8_t *out_cells, uint64_t *proofs, uint8_t *proof_inf, uint8_t *status) {
+    const size_t cb = (size_t)ZKP_CELLS_PER_EXT_BLOB * ZKP_CELL_BYTES;
+    const size_t chunk = proofs ? ZKP_CELL_PROOF_CHUNK : blobs ? ZKP_CELLS_CHUNK : ZKP_CELLS_RECOVER_CHUNK;
+    return run_host_job(ctx, n, chunk, [=](Chunk &c) {
+        const size_t np = c.cn * ZKP_CELLS_PER_EXT_BLOB;
+        const uint8_t *db = nullptr, *dcells = nullptr;
+        const uint64_t *didx = nullptr, *dnum = nullptr;
+        uint8_t *dout;
+        if (blobs) {
+            db = c.in(B_IN, blobs, c.c0 * ZKP_BLOB_BYTES, c.cn * ZKP_BLOB_BYTES);
+            dout = c.buf<uint8_t>(B_G1, c.cn * cb);
+        } else {
+            dcells = c.in(B_IN, cells, c.c0 * cb, c.cn * cb);
+            dout = c.buf<uint8_t>(B_G1, c.cn * cb);
+            didx = c.in(B_TAB, idx, c.c0 * ZKP_CELLS_PER_EXT_BLOB, np);
+            dnum = c.in(B_G1INF, num, c.c0, c.cn);
+        }
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        uint64_t *dpf = nullptr;
+        uint8_t *dpi = nullptr, *dscr = nullptr;
+        if (proofs) {
+            dpf = c.buf<uint64_t>(B_G2, np * 12);
+            dpi = c.buf<uint8_t>(B_G2INF, np);
+            dscr = c.buf<uint8_t>(B_OUT, zkp_kzg_cells_proofs_scratch_bytes(c.cn));
+        }
+        const KzgDev &kd = s->devs[c.dev];
+        if (blobs) CUT(launch_cells(ctx, kd, db, c.cn, dout, dpf, dpi, dst, dscr, c.st));
+        else CUT(launch_cells_recover(ctx, kd, didx, dcells, dnum, c.cn, dout, dpf, dpi, dst, dscr, c.st));
+        c.out(B_G1, out_cells + c.c0 * cb, dout, c.cn * cb);
+        if (proofs) {
+            c.out(B_G2, proofs + c.c0 * ZKP_CELLS_PER_EXT_BLOB * 12, dpf, np * 12);
+            c.out(B_G2INF, proof_inf + c.c0 * ZKP_CELLS_PER_EXT_BLOB, dpi, np);
+        }
+        c.out(B_FLAG, status + c.c0, dst, c.cn);
+    });
+}
+
 int32_t zkp_kzg_compute_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
                                     uint8_t *out_status) {
     int32_t rc = check_cells(ctx, s);
     if (rc) return rc;
     if (n && (!blobs || !out_cells || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 176; j.kzg = s; j.blobs = blobs; j.ocells = out_cells; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return cells_job(ctx, s, blobs, nullptr, nullptr, nullptr, n, out_cells, nullptr, nullptr, out_status);
 }
 
 int32_t zkp_kzg_compute_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint8_t *blobs, size_t n, uint8_t *out_cells,
@@ -2612,9 +2440,7 @@ int32_t zkp_kzg_compute_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup
     int32_t rc = check_cells(ctx, s);
     if (rc) return rc;
     if (n && (!blobs || !out_cells || !out_proofs || !out_proof_inf || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 192; j.kzg = s; j.blobs = blobs; j.ocells = out_cells; j.og1 = out_proofs; j.og1inf = out_proof_inf; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return cells_job(ctx, s, blobs, nullptr, nullptr, nullptr, n, out_cells, out_proofs, out_proof_inf, out_status);
 }
 
 int32_t zkp_kzg_verify_cell_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *commitments, const uint8_t *commitment_inf,
@@ -2623,10 +2449,16 @@ int32_t zkp_kzg_verify_cell_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const ui
     int32_t rc = check_cells(ctx, s);
     if (rc) return rc;
     if (n && (!commitments || !cell_indices || !cells || !proofs || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 208; j.kzg = s; j.pts = commitments; j.g1inf = commitment_inf; j.idx = cell_indices; j.cells = cells; j.pi = proofs;
-    j.piinf = proof_inf; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return run_host_job(ctx, n, ZKP_CELL_VERIFY_CHUNK, [=](Chunk &c) {
+        const uint64_t *dc = c.in(B_G1, commitments, c.c0 * 12, c.cn * 12), *dpf = c.in(B_G2, proofs, c.c0 * 12, c.cn * 12);
+        const uint64_t *didx = c.in(B_TAB, cell_indices, c.c0, c.cn);
+        const uint8_t *dcells = c.in(B_IN, cells, c.c0 * ZKP_CELL_BYTES, c.cn * ZKP_CELL_BYTES);
+        uint8_t *dst = c.buf<uint8_t>(B_FLAG, c.cn);
+        uint8_t *dscr = c.buf<uint8_t>(B_OUT, zkp_kzg_verify_cell_scratch_bytes(c.cn));
+        const uint8_t *dci = c.in(B_G1INF, commitment_inf, c.c0, c.cn), *dpi = c.in(B_G2INF, proof_inf, c.c0, c.cn);
+        CUT(launch_cells_verify(ctx, c.d, s->devs[c.dev], dc, dci, didx, dcells, dpf, dpi, c.cn, dst, dscr, c.d.d_err, c.st));
+        c.out(B_FLAG, out_status + c.c0, dst, c.cn);
+    });
 }
 
 int32_t zkp_kzg_compute_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n, uint8_t *d_cells,
@@ -2636,11 +2468,10 @@ int32_t zkp_kzg_compute_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup
     if (rc) return rc;
     if (n && (!d_blobs || !d_cells || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_blobs & 15) || ((uintptr_t)d_cells & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_blobs and d_cells must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard guard;
-    CU(cudaSetDevice(ctx->devs[dev].id));
-    CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, nullptr, nullptr, d_status, nullptr, (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, nullptr, nullptr, d_status, nullptr, st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint8_t *d_blobs, size_t n,
@@ -2652,11 +2483,10 @@ int32_t zkp_kzg_compute_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zk
     if (n && (!d_blobs || !d_cells || !d_proofs || !d_proof_inf || !d_status || !d_scratch)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_blobs & 15) || ((uintptr_t)d_cells & 15) || ((uintptr_t)d_scratch & 15))
         return fail(ZKP_ERR_INVALID_ARG, "d_blobs, d_cells and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard guard;
-    CU(cudaSetDevice(ctx->devs[dev].id));
-    CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, d_proofs, d_proof_inf, d_status, d_scratch, (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_cells(ctx, s->devs[dev], d_blobs, n, d_cells, d_proofs, d_proof_inf, d_status, d_scratch, st));
+        return ZKP_OK;
+    });
 }
 
 // recovery runs one cluster of two blocks with 128 KiB of shared memory each per blob: refuse (never substitute) a device
@@ -2680,9 +2510,7 @@ int32_t zkp_kzg_recover_cells_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const 
     int32_t rc = check_recover(ctx, s, -1);
     if (rc) return rc;
     if (n && (!cell_indices || !cells || !num_cells || !out_cells || !out_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 224; j.kzg = s; j.idx = cell_indices; j.cells = cells; j.scalars = num_cells; j.ocells = out_cells; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return cells_job(ctx, s, nullptr, cell_indices, cells, num_cells, n, out_cells, nullptr, nullptr, out_status);
 }
 
 int32_t zkp_kzg_recover_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup *s, const uint64_t *cell_indices, const uint8_t *cells,
@@ -2692,10 +2520,7 @@ int32_t zkp_kzg_recover_cells_and_proofs_batch(zkp_ctx *ctx, const zkp_kzg_setup
     if (rc) return rc;
     if (n && (!cell_indices || !cells || !num_cells || !out_cells || !out_proofs || !out_proof_inf || !out_status))
         return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
-    HostJob j;
-    j.mode = 240; j.kzg = s; j.idx = cell_indices; j.cells = cells; j.scalars = num_cells; j.ocells = out_cells; j.og1 = out_proofs;
-    j.og1inf = out_proof_inf; j.flags = out_status;
-    return run_host_job(ctx, j, n);
+    return cells_job(ctx, s, nullptr, cell_indices, cells, num_cells, n, out_cells, out_proofs, out_proof_inf, out_status);
 }
 
 int32_t zkp_kzg_recover_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices, const uint8_t *d_cells,
@@ -2705,12 +2530,11 @@ int32_t zkp_kzg_recover_cells_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup
     if (rc) return rc;
     if (n && (!d_cell_indices || !d_cells || !d_num_cells || !d_out_cells || !d_status)) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_out_cells & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_cells and d_out_cells must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard guard;
-    CU(cudaSetDevice(ctx->devs[dev].id));
-    CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, nullptr, nullptr, d_status, nullptr,
-                            (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, nullptr, nullptr, d_status, nullptr,
+                                st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_kzg_recover_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_cell_indices,
@@ -2723,12 +2547,11 @@ int32_t zkp_kzg_recover_cells_and_proofs_dev(zkp_ctx *ctx, int32_t dev, const zk
         return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_out_cells & 15) || ((uintptr_t)d_scratch & 15))
         return fail(ZKP_ERR_INVALID_ARG, "d_cells, d_out_cells and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DeviceGuard guard;
-    CU(cudaSetDevice(ctx->devs[dev].id));
-    CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, d_proofs, d_proof_inf, d_status, d_scratch,
-                            (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_cells_recover(ctx, s->devs[dev], d_cell_indices, d_cells, d_num_cells, n, d_out_cells, d_proofs, d_proof_inf, d_status, d_scratch,
+                                st));
+        return ZKP_OK;
+    });
 }
 
 int32_t zkp_kzg_verify_cell_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *s, const uint64_t *d_commitments, const uint8_t *d_commitment_inf,
@@ -2740,13 +2563,11 @@ int32_t zkp_kzg_verify_cell_dev(zkp_ctx *ctx, int32_t dev, const zkp_kzg_setup *
     if (n && (!d_commitments || !d_cell_indices || !d_cells || !d_proofs || !d_status || !d_scratch))
         return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
     if (((uintptr_t)d_cells & 15) || ((uintptr_t)d_scratch & 15)) return fail(ZKP_ERR_INVALID_ARG, "d_cells and d_scratch must be 16-byte aligned");
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    DevState &d = ctx->devs[dev];
-    DeviceGuard guard;
-    CU(cudaSetDevice(d.id));
-    CU(launch_cells_verify(ctx, d, s->devs[dev], d_commitments, d_commitment_inf, d_cell_indices, d_cells, d_proofs, d_proof_inf, n, d_status,
-                           d_scratch, nullptr, (cudaStream_t)stream));
-    return ZKP_OK;
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        CU(launch_cells_verify(ctx, d, s->devs[dev], d_commitments, d_commitment_inf, d_cell_indices, d_cells, d_proofs, d_proof_inf, n, d_status,
+                               d_scratch, nullptr, st));
+        return ZKP_OK;
+    });
 }
 
 // ------------------------------------------------------------------ measurement
