@@ -266,6 +266,36 @@ int32_t zkp_g1_add_batch(zkp_ctx *ctx, const uint64_t *a_xy, const uint8_t *a_in
 int32_t zkp_g2_add_batch(zkp_ctx *ctx, const uint64_t *a_xy, const uint8_t *a_inf, const uint64_t *b_xy, const uint8_t *b_inf,
                          size_t n, uint64_t *out_xy, uint8_t *out_flag);
 
+/* ---- multi-scalar multiplication over caller-given points (blst p1s_mult_pippenger / p2s_mult_pippenger,
+ * arkworks VariableBaseMSM; absent from the reference) ------------------------------------------------
+ * sum_i [k_i]P_i over n caller-given points, one result per call (Pippenger with signed-digit buckets).
+ * Points and scalars follow zkp_g1_mul_batch / zkp_g2_mul_batch: canonical affine limbs, g*_inf optional (a flagged
+ * point contributes the identity), k_i = 4 little-endian u64 of ANY 256-bit value, taken as an integer and not
+ * reduced mod r.  The result is exactly the group element sum_i [k_i]P_i, in the prime-order subgroup or not: no
+ * endomorphism split is used, and subgroup membership is NOT checked (the sum is exact without it).  For subgroup
+ * points it equals the sum with every k_i reduced mod r.
+ * Output: one point, canonical affine x|y and out_inf; the identity is (0, 1) with out_inf = 1.  n = 0 gives the
+ * identity, out_status = ZKP_POINT_OK and ZKP_OK.
+ * Validation: a limb >= p fails the call with ZKP_ERR_NONCANONICAL (the _dev forms OR 1 into d_err instead).  An
+ * unflagged point off its curve gives out_status = ZKP_POINT_NOT_ON_CURVE, zero limbs and out_inf = 1; the call still
+ * returns ZKP_OK.  Otherwise out_status = ZKP_POINT_OK.
+ * Host forms: the points shard in contiguous slices over the context's devices; each device's Jacobian partial is
+ * gathered on the first device, so the affine result is the same for any number of devices.
+ * _dev forms: asynchronous on `stream` with d_scratch of zkp_g*_msm_scratch_bytes(n) bytes, 16-byte aligned; d_err
+ * may be NULL.  The caller's current device is restored. */
+int32_t zkp_g1_msm(zkp_ctx *ctx, const uint64_t *g1_xy, const uint8_t *g1_inf, const uint64_t *scalars, size_t n,
+                   uint64_t *out_xy, uint8_t *out_inf, uint8_t *out_status);
+int32_t zkp_g2_msm(zkp_ctx *ctx, const uint64_t *g2_xy, const uint8_t *g2_inf, const uint64_t *scalars, size_t n,
+                   uint64_t *out_xy, uint8_t *out_inf, uint8_t *out_status);
+size_t zkp_g1_msm_scratch_bytes(size_t n);
+size_t zkp_g2_msm_scratch_bytes(size_t n);
+int32_t zkp_g1_msm_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g1_xy, const uint8_t *d_g1_inf, const uint64_t *d_scalars,
+                       size_t n, uint64_t *d_out_xy, uint8_t *d_out_inf, uint8_t *d_status, uint32_t *d_err,
+                       void *d_scratch, void *stream);
+int32_t zkp_g2_msm_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g2_xy, const uint8_t *d_g2_inf, const uint64_t *d_scalars,
+                       size_t n, uint64_t *d_out_xy, uint8_t *d_out_inf, uint8_t *d_status, uint32_t *d_err,
+                       void *d_scratch, void *stream);
+
 /* ---- Groth16 verification (one verdict per proof) ----------------------------------------------
  * Verifying key: alpha in G1; beta, gamma, delta in G2; IC_0 .. IC_l in G1 (l = n_public).  Proof: A in G1,
  * B in G2, C in G1.  Public inputs: x_1 .. x_l, each an Fr as four little-endian u64 limbs.  A proof is

@@ -59,6 +59,14 @@ SYMBOLS = {
     "zkp_g2_mul_batch": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p]),
     "zkp_g1_add_batch": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t, c_u64p, c_u8p]),
     "zkp_g2_add_batch": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u8p, c_u64p, c_u8p, ctypes.c_size_t, c_u64p, c_u8p]),
+    "zkp_g1_msm": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p, c_u8p]),
+    "zkp_g2_msm": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p, c_u8p]),
+    "zkp_g1_msm_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
+    "zkp_g2_msm_scratch_bytes": (ctypes.c_size_t, [ctypes.c_size_t]),
+    "zkp_g1_msm_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p, c_u8p,
+                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
+    "zkp_g2_msm_dev": (ctypes.c_int32, [ctypes.c_void_p, ctypes.c_int32, c_u64p, c_u8p, c_u64p, ctypes.c_size_t, c_u64p, c_u8p, c_u8p,
+                                        ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "zkp_groth16_vk_create": (ctypes.c_int32, [ctypes.c_void_p, c_u64p, c_u64p, c_u64p, c_u64p, c_u64p, c_u8p, ctypes.c_int32,
                                                ctypes.POINTER(ctypes.c_void_p)]),
     "zkp_groth16_vk_destroy": (None, [ctypes.c_void_p]),

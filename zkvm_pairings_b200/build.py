@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libzkpair.so")
 SOURCES = ["kernels.cu", "pairing_kernel.cu", "fe_kernel.cu"]
-HEADERS = ["fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "fe_scratch.cuh", "groth16.cuh", "kzg.cuh", "fr.cuh", "blob.cuh", "kzg_prove.cuh", "kzg_cells.cuh", "kzg_recover.cuh", "consts.cuh", "../../include/zkpair.h"]
+HEADERS = ["fp.cuh", "tower.cuh", "pairing.cuh", "ops.cuh", "fe_scratch.cuh", "groth16.cuh", "kzg.cuh", "fr.cuh", "blob.cuh", "kzg_prove.cuh", "kzg_cells.cuh", "kzg_recover.cuh", "msm.cuh", "consts.cuh", "../../include/zkpair.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "--threads", "0"]   # the three units compile in parallel
 

@@ -33,6 +33,7 @@
 #include "kzg_prove.cuh"
 #include "kzg_cells.cuh"
 #include "kzg_recover.cuh"
+#include "msm.cuh"
 
 #include <cooperative_groups.h>
 
@@ -530,6 +531,85 @@ k_cells_prepare(const uint64_t *__restrict__ c, const uint8_t *__restrict__ cinf
     const uint8_t s = cell_prepare_one(c + 12 * i, cinf ? cinf[i] : 0, pi + 12 * i, piinf ? piinf[i] : 0, idx[i], pw, ixy + 12 * i, iinf[i],
                                        pre, g1 + 24 * i, g1inf + 2 * i);
     if (lane_par() == 0) status[i] = s;
+}
+
+// ---- multi-scalar multiplication over caller-given points (msm.cuh); O = OpsFp (G1, one thread per point or
+// segment) or OpsFp2 (G2, one lane pair)
+
+#define ZKP_MSM_KTPB 128   // threads per block of the per-point and per-segment kernels
+
+template <class O>
+__global__ void __launch_bounds__(ZKP_MSM_KTPB)
+k_msm_check(const uint64_t *__restrict__ xy, const uint8_t *__restrict__ inf, size_t n, Fp *__restrict__ pts, uint8_t *__restrict__ valid,
+            uint32_t *off, uint32_t *err) {
+    const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) / MsmWidth<O>::W;
+    if (i >= n) return;
+    msm_check<O>(i, xy, inf, pts, valid, off, err);
+}
+
+// every thread runs the window loop (the claims are warp-wide), also past n
+__global__ void __launch_bounds__(ZKP_MSM_KTPB)
+k_msm_digits(const uint64_t *__restrict__ scalars, const uint8_t *__restrict__ valid, size_t n, int c, uint32_t *ctr, uint32_t *keys,
+             uint32_t *vals) {
+    msm_digits((size_t)blockIdx.x * blockDim.x + threadIdx.x, n, scalars, valid, c, ctr, keys, vals);
+}
+
+__global__ void __launch_bounds__(ZKP_MSM_SCAN_TPB)
+k_msm_scan(const uint32_t *__restrict__ cnt, uint32_t nb, uint32_t *__restrict__ off, uint32_t *__restrict__ cur, uint32_t *len) {
+    __shared__ uint32_t part[ZKP_MSM_SCAN_TPB];
+    const int t = threadIdx.x;
+    msm_scan_sum(t, ZKP_MSM_SCAN_TPB, cnt, nb, part);
+    __syncthreads();
+    if (t == 0) msm_scan_prefix(ZKP_MSM_SCAN_TPB, part, off + nb, len);
+    __syncthreads();
+    msm_scan_write(t, ZKP_MSM_SCAN_TPB, cnt, nb, part, off, cur);
+}
+
+template <class O, bool AFF>
+__global__ void __launch_bounds__(ZKP_MSM_KTPB)
+k_msm_segment(const uint32_t *len_in, uint32_t *len_out, const uint32_t *__restrict__ keys, const uint32_t *__restrict__ vals,
+              const Fp *__restrict__ src, Fp *buckets, uint32_t *__restrict__ fkey, Fp *__restrict__ fval, size_t nseg) {
+    const size_t s = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) / MsmWidth<O>::W;
+    if (s >= nseg) return;
+    msm_segment<O, AFF>(s, ZKP_MSM_SEG, len_in, len_out, keys, vals, src, buckets, fkey, fval);
+}
+
+// one block per window: R ranges (R <= ZKP_MSM_RANGES), then the tree over ZKP_MSM_RANGES slots
+template <class O>
+__global__ void __launch_bounds__(ZKP_MSM_RANGES * 2)
+k_msm_reduce(const Fp *__restrict__ buckets, int M, int R, Fp *__restrict__ wsum) {
+    __shared__ Fp sh[ZKP_MSM_RANGES * 3 * MsmWidth<O>::W];
+    const int q = threadIdx.x / MsmWidth<O>::W, w = blockIdx.x;
+    Jac<O> r;
+    msm_id(r);
+    if (q < R) msm_range<O>(w, q, R, M, buckets, r);
+    msm_stj(sh, q, r);
+    __syncthreads();
+    for (int h = ZKP_MSM_RANGES / 2; h >= 1; h >>= 1) {
+        if (q < h) msm_tree_step<O>(sh, q, h);
+        __syncthreads();
+    }
+    if (q == 0) {
+        msm_ldj(r, sh, 0);
+        msm_stj(wsum, w, r);
+    }
+}
+
+template <class O>
+__global__ void k_msm_combine(int nw, int c, const Fp *__restrict__ wsum, Fp *__restrict__ part) {
+    msm_combine<O>(nw, c, wsum, part);
+}
+
+template <class O>
+__global__ void k_msm_sum(const Fp *__restrict__ parts, int np, Fp *__restrict__ out) {
+    msm_sum<O>(parts, np, out);
+}
+
+template <class O>
+__global__ void k_msm_final(const Fp *__restrict__ parts, int np, const uint32_t *__restrict__ offs, int noff, uint64_t *__restrict__ out_xy,
+                            uint8_t *__restrict__ out_inf, uint8_t *__restrict__ status) {
+    const uint8_t st = msm_final<O>(parts, np, offs, noff, out_xy, out_inf);
+    if (msm_writer<O>()) *status = st;
 }
 
 // Byte (de)serialisation at the boundary (SURVEY 8f-2): 48 big-endian bytes <-> six little-endian u64
@@ -1050,6 +1130,114 @@ static cudaError_t launch_cells_verify(zkp_ctx *ctx, DevState &d, const KzgDev &
     return launch_check_verdict(ctx, d, s.g1, s.g1inf, nullptr, nullptr, n, 2, k.cell_prep, 2, s.gt, s.is_one, status, err, st);
 }
 
+// ---- multi-scalar multiplication over caller-given points: count, scan, scatter, accumulation levels, reduction, Horner
+// (msm.cuh) for one batch of points, leaving one Jacobian partial on the device
+
+#ifndef ZKP_MSM_CHUNK
+#define ZKP_MSM_CHUNK (1u << 22)   // points per host chunk: 1.3 GiB (G1) / 2.1 GiB (G2) of scratch per buffer set (DESIGN.md 3.9)
+#endif
+
+// The window width for n points: msm_window's rule, or ZKPAIR_MSM_WINDOW (4 .. 20) when set, for measuring widths.
+static int msm_width(size_t n) {
+    const char *e = getenv("ZKPAIR_MSM_WINDOW");
+    const int c = e ? atoi(e) : 0;
+    return c >= 4 && c <= 20 ? c : msm_window(n);
+}
+
+struct MsmPlan {
+    int c, nw, M, levels;
+    size_t nb, emax, s0, s1;
+};
+static MsmPlan msm_plan(size_t n) {
+    MsmPlan p;
+    p.c = msm_width(n);
+    p.nw = msm_windows(p.c);
+    p.M = 1 << (p.c - 1);
+    p.nb = (size_t)p.nw * p.M;
+    p.emax = (size_t)p.nw * n;
+    p.levels = msm_levels(p.emax);
+    p.s0 = (p.emax + ZKP_MSM_SEG - 1) / ZKP_MSM_SEG;
+    p.s1 = (p.s0 + ZKP_MSM_SEG - 1) / ZKP_MSM_SEG;
+    return p;
+}
+// the largest batch one scratch holds: point indices take 31 bits and list positions 32
+static bool msm_fits(size_t n) { return n < ((size_t)1 << 31) && (size_t)msm_windows(msm_width(n)) * n < ((size_t)1 << 32) - 1; }
+
+struct MsmScratch {
+    uint32_t *off_curve, *lens;   // header: the off-curve word, the levels' list lengths
+    Fp *part;                     // header: the Jacobian result of the _dev forms
+    Fp *pts, *buckets, *fval[2], *wsum;
+    uint8_t *valid;
+    uint32_t *cnt, *off, *cur, *keys, *vals, *fkey[2];
+};
+#define ZKP_MSM_HDR 1024   // off-curve word at 0, list lengths at 64, the Jacobian result at 256
+static size_t msm_layout(size_t n, int w, void *base, MsmScratch *s) {
+    const MsmPlan p = msm_plan(n);
+    const size_t jb = 3 * (size_t)w * sizeof(Fp);   // bytes of one Jacobian point
+    uint8_t *q[14];
+    const size_t bytes = carve(base, {(size_t)ZKP_MSM_HDR, n * 2 * w * sizeof(Fp), n, p.nb * 4, (p.nb + 1) * 4, p.nb * 4, p.emax * 4,
+                                      p.emax * 4, p.nb * jb, p.s0 * 4, p.s0 * jb, p.s1 * 4, p.s1 * jb, p.nw * jb}, q);
+    if (s) {
+        s->off_curve = (uint32_t *)q[0];
+        s->lens = (uint32_t *)(q[0] + 64);
+        s->part = (Fp *)(q[0] + 256);
+        s->pts = (Fp *)q[1];
+        s->valid = q[2];
+        s->cnt = (uint32_t *)q[3];
+        s->off = (uint32_t *)q[4];
+        s->cur = (uint32_t *)q[5];
+        s->keys = (uint32_t *)q[6];
+        s->vals = (uint32_t *)q[7];
+        s->buckets = (Fp *)q[8];
+        s->fkey[0] = (uint32_t *)q[9];
+        s->fval[0] = (Fp *)q[10];
+        s->fkey[1] = (uint32_t *)q[11];
+        s->fval[1] = (Fp *)q[12];
+        s->wsum = (Fp *)q[13];
+    }
+    return bytes;
+}
+extern "C" size_t zkp_g1_msm_scratch_bytes(size_t n) { return msm_layout(n, 1, nullptr, nullptr); }
+extern "C" size_t zkp_g2_msm_scratch_bytes(size_t n) { return msm_layout(n, 2, nullptr, nullptr); }
+
+// sum_i [k_i]P_i over n > 0 device-resident points into the Jacobian point part; an unflagged point off the curve ORs 1
+// into *off_curve (zeroed by the caller), a limb >= p 1 into *err
+template <class O>
+static cudaError_t launch_msm(zkp_ctx *ctx, const uint64_t *xy, const uint8_t *inf, const uint64_t *scalars, size_t n, void *scratch, Fp *part,
+                              uint32_t *off_curve, uint32_t *err, cudaStream_t st) {
+    const int w = MsmWidth<O>::W;
+    const MsmPlan p = msm_plan(n);
+    MsmScratch s;
+    msm_layout(n, w, scratch, &s);
+    cudaError_t e = cudaMemsetAsync(s.cnt, 0, p.nb * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(s.buckets, 0, p.nb * 3 * w * sizeof(Fp), st);   // z = 0: every bucket the identity
+    if (e != cudaSuccess) return e;
+    const unsigned gp = (unsigned)((n + ZKP_MSM_KTPB - 1) / ZKP_MSM_KTPB);
+    k_msm_check<O><<<(unsigned)((n * w + ZKP_MSM_KTPB - 1) / ZKP_MSM_KTPB), ZKP_MSM_KTPB, 0, st>>>(xy, inf, n, s.pts, s.valid, off_curve, err);
+    k_msm_digits<<<gp, ZKP_MSM_KTPB, 0, st>>>(scalars, s.valid, n, p.c, s.cnt, nullptr, nullptr);
+    k_msm_scan<<<1, ZKP_MSM_SCAN_TPB, 0, st>>>(s.cnt, (uint32_t)p.nb, s.off, s.cur, s.lens);
+    k_msm_digits<<<gp, ZKP_MSM_KTPB, 0, st>>>(scalars, s.valid, n, p.c, s.cur, s.keys, s.vals);
+    ctx->launches += 4;
+    size_t m = p.emax;   // the bound of each level's list length (the length itself is on the device)
+    for (int lv = 0; lv < p.levels; lv++) {
+        const size_t nseg = (m + ZKP_MSM_SEG - 1) / ZKP_MSM_SEG;
+        const unsigned g = (unsigned)((nseg * w + ZKP_MSM_KTPB - 1) / ZKP_MSM_KTPB);
+        const int o = lv & 1, i = o ^ 1;   // level lv writes list o and reads list i (the sorted entries at level 0)
+        if (lv == 0)
+            k_msm_segment<O, true><<<g, ZKP_MSM_KTPB, 0, st>>>(s.lens, s.lens + 1, s.keys, s.vals, s.pts, s.buckets, s.fkey[0], s.fval[0], nseg);
+        else
+            k_msm_segment<O, false><<<g, ZKP_MSM_KTPB, 0, st>>>(s.lens + lv, s.lens + lv + 1, s.fkey[i], nullptr, s.fval[i], s.buckets, s.fkey[o],
+                                                                 s.fval[o], nseg);
+        ctx->launches++;
+        m = nseg;
+    }
+    const int R = p.M < ZKP_MSM_RANGES ? p.M : ZKP_MSM_RANGES;
+    k_msm_reduce<O><<<(unsigned)p.nw, ZKP_MSM_RANGES * w, 0, st>>>(s.buckets, p.M, R, s.wsum);
+    k_msm_combine<O><<<1, w, 0, st>>>(p.nw, p.c, s.wsum, part);
+    ctx->launches += 2;
+    return cudaGetLastError();
+}
+
 // Runs launch(d, st) for a device-resident entry point whose arguments passed their checks: under the context lock, on
 // device dev of the context (the caller's current device is restored) and on the caller's stream (NULL = the legacy
 // default stream, the CUDA convention).
@@ -1213,6 +1401,109 @@ static int32_t run_host_job(zkp_ctx *ctx, size_t n, size_t chunk, const ChunkBod
     if (n == 0) return ZKP_OK;
     std::lock_guard<std::mutex> lk(ctx->mu);
     return run_slices(ctx, n, chunk, body);
+}
+
+// One MSM over host buffers, in the shape of zkp_multi_miller_product: each device sums its slice chunk by chunk into
+// Jacobian partials in d.partial (followed by the device's off-curve word), its finish step folds them into the slot
+// after the last one, and the first device gathers one partial per device by peer copy, adds them and converts the sum
+// to affine.
+template <class O>
+static int32_t msm_job(zkp_ctx *ctx, const uint64_t *xy, const uint8_t *inf, const uint64_t *scalars, size_t n, uint64_t *out_xy,
+                       uint8_t *out_inf, uint8_t *out_status) {
+    const int w = MsmWidth<O>::W;
+    const size_t pw = MsmWidth<O>::U64, jb = 3 * w * sizeof(Fp);
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (!out_xy || !out_inf || !out_status || (n && (!xy || !scalars))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if (n == 0) {   // the identity (0, 1)
+        memset(out_xy, 0, pw * sizeof(uint64_t));
+        out_xy[pw / 2] = 1;
+        *out_inf = 1;
+        *out_status = ZKP_POINT_OK;
+        return ZKP_OK;
+    }
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    DeviceGuard guard;
+    const size_t chunk = ZKP_MSM_CHUNK;
+    auto nchunks = [=](size_t lo, size_t hi) { return (hi - lo + chunk - 1) / chunk; };
+    auto body = [=](Chunk &c) {
+        DevState &d = c.d;
+        const size_t nc = nchunks(c.lo, c.hi);
+        if (c.c0 == c.lo) {   // the partials, their fold and the off-curve word, zeroed before any chunk runs
+            CUT(d.partial.ensure((nc + 1) * jb + sizeof(uint32_t)));
+            CUT(cudaMemsetAsync((uint8_t *)d.partial.p + (nc + 1) * jb, 0, sizeof(uint32_t), c.st));
+            CUT(cudaStreamSynchronize(c.st));
+        }
+        const size_t ci = (c.c0 - c.lo) / chunk;
+        const uint64_t *dxy = c.in(B_G1, xy, c.c0 * pw, c.cn * pw), *dsc = c.in(B_IN, scalars, c.c0 * 4, c.cn * 4);
+        const uint8_t *dinf = c.in(B_G1INF, inf, c.c0, c.cn);
+        void *scratch = c.buf<uint8_t>(B_TAB, msm_layout(c.cn, w, nullptr, nullptr));
+        CUT(launch_msm<O>(ctx, dxy, dinf, dsc, c.cn, scratch, (Fp *)((uint8_t *)d.partial.p + ci * jb),
+                          (uint32_t *)((uint8_t *)d.partial.p + (nc + 1) * jb), d.d_err, c.st));
+    };
+    auto fold = [=](DevState &d, size_t lo, size_t hi) {
+        const size_t nc = nchunks(lo, hi);
+        k_msm_sum<O><<<1, w, 0, d.stream[0]>>>((const Fp *)d.partial.p, (int)nc, (Fp *)((uint8_t *)d.partial.p + nc * jb));
+        ctx->launches++;
+        CUT(cudaGetLastError());
+        CUT(cudaStreamSynchronize(d.stream[0]));
+    };
+    int32_t rc = run_slices(ctx, n, chunk, body, fold);
+    if (rc != ZKP_OK) return rc;
+    // gather: one partial and one off-curve word per device -> first device (peer copy over NVLink when available)
+    const size_t nd = fan_out(ctx, n);
+    DevState &d0 = ctx->devs[0];
+    CU(cudaSetDevice(d0.id));
+    DevBuf &G = d0.buf[1][B_IN];
+    const size_t offs = align256(nd * jb), res = offs + align256(nd * 4);   // partials | off-curve words | x|y, flag, status
+    CU(G.ensure(res + pw * sizeof(uint64_t) + 2));
+    uint8_t *g = (uint8_t *)G.p;
+    for (size_t di = 0; di < nd; di++) {
+        DevState &d = ctx->devs[di];
+        size_t lo, hi;
+        slice_of(n, nd, di, lo, hi);
+        const size_t nc = nchunks(lo, hi);
+        const uint8_t *src = (const uint8_t *)d.partial.p;
+        if (d.id == d0.id) {
+            CU(cudaMemcpyAsync(g + di * jb, src + nc * jb, jb, cudaMemcpyDeviceToDevice, d0.stream[0]));
+            CU(cudaMemcpyAsync(g + offs + 4 * di, src + (nc + 1) * jb, 4, cudaMemcpyDeviceToDevice, d0.stream[0]));
+        } else {
+            CU(cudaMemcpyPeerAsync(g + di * jb, d0.id, src + nc * jb, d.id, jb, d0.stream[0]));
+            CU(cudaMemcpyPeerAsync(g + offs + 4 * di, d0.id, src + (nc + 1) * jb, d.id, 4, d0.stream[0]));
+        }
+    }
+    uint64_t *rxy = (uint64_t *)(g + res);
+    uint8_t *rflag = g + res + pw * sizeof(uint64_t);
+    k_msm_final<O><<<1, w, 0, d0.stream[0]>>>((const Fp *)g, (int)nd, (const uint32_t *)(g + offs), (int)nd, rxy, rflag, rflag + 1);
+    ctx->launches++;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(out_xy, rxy, pw * sizeof(uint64_t), cudaMemcpyDeviceToHost, d0.stream[0]));
+    CU(cudaMemcpyAsync(out_inf, rflag, 1, cudaMemcpyDeviceToHost, d0.stream[0]));
+    CU(cudaMemcpyAsync(out_status, rflag + 1, 1, cudaMemcpyDeviceToHost, d0.stream[0]));
+    CU(cudaStreamSynchronize(d0.stream[0]));
+    return ZKP_OK;
+}
+
+// The _dev forms: the whole batch in one launch sequence on the caller's stream, the partial and the off-curve word in
+// the scratch header.
+template <class O>
+static int32_t msm_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *xy, const uint8_t *inf, const uint64_t *scalars, size_t n, uint64_t *out_xy,
+                       uint8_t *out_inf, uint8_t *status, uint32_t *err, void *scratch, void *stream) {
+    if (!ctx) return fail(ZKP_ERR_INVALID_ARG, "ctx is NULL");
+    if (dev < 0 || dev >= (int)ctx->devs.size()) return fail(ZKP_ERR_INVALID_ARG, "device index out of range");
+    if (!out_xy || !out_inf || !status || !scratch || (n && (!xy || !scalars))) return fail(ZKP_ERR_INVALID_ARG, "NULL buffer");
+    if ((uintptr_t)scratch & 15) return fail(ZKP_ERR_INVALID_ARG, "d_scratch is not 16-byte aligned");
+    if (!msm_fits(n)) return fail(ZKP_ERR_INVALID_ARG, "n too large for one device-resident MSM");
+    return on_device(ctx, dev, stream, [&](DevState &d, cudaStream_t st) {
+        (void)d;
+        MsmScratch s;
+        msm_layout(n, MsmWidth<O>::W, scratch, &s);
+        CU(cudaMemsetAsync(scratch, 0, ZKP_MSM_HDR, st));   // off-curve word 0, result the identity
+        if (n) CU(launch_msm<O>(ctx, xy, inf, scalars, n, scratch, s.part, s.off_curve, err, st));
+        k_msm_final<O><<<1, MsmWidth<O>::W, 0, st>>>(s.part, 1, s.off_curve, 1, out_xy, out_inf, status);
+        ctx->launches++;
+        CU(cudaGetLastError());
+        return ZKP_OK;
+    });
 }
 
 extern "C" {
@@ -1789,6 +2080,24 @@ int32_t zkp_multi_miller_product(zkp_ctx *ctx, const uint64_t *g1, const uint8_t
     if (out_gt) CU(cudaMemcpyAsync(out_gt, gt, 576, cudaMemcpyDeviceToHost, d0.stream[0]));
     CU(cudaStreamSynchronize(d0.stream[0]));
     return ZKP_OK;
+}
+
+// ---- multi-scalar multiplication over caller-given points
+int32_t zkp_g1_msm(zkp_ctx *ctx, const uint64_t *g1_xy, const uint8_t *g1_inf, const uint64_t *scalars, size_t n, uint64_t *out_xy,
+                   uint8_t *out_inf, uint8_t *out_status) {
+    return msm_job<OpsFp>(ctx, g1_xy, g1_inf, scalars, n, out_xy, out_inf, out_status);
+}
+int32_t zkp_g2_msm(zkp_ctx *ctx, const uint64_t *g2_xy, const uint8_t *g2_inf, const uint64_t *scalars, size_t n, uint64_t *out_xy,
+                   uint8_t *out_inf, uint8_t *out_status) {
+    return msm_job<OpsFp2>(ctx, g2_xy, g2_inf, scalars, n, out_xy, out_inf, out_status);
+}
+int32_t zkp_g1_msm_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g1_xy, const uint8_t *d_g1_inf, const uint64_t *d_scalars, size_t n,
+                       uint64_t *d_out_xy, uint8_t *d_out_inf, uint8_t *d_status, uint32_t *d_err, void *d_scratch, void *stream) {
+    return msm_dev<OpsFp>(ctx, dev, d_g1_xy, d_g1_inf, d_scalars, n, d_out_xy, d_out_inf, d_status, d_err, d_scratch, stream);
+}
+int32_t zkp_g2_msm_dev(zkp_ctx *ctx, int32_t dev, const uint64_t *d_g2_xy, const uint8_t *d_g2_inf, const uint64_t *d_scalars, size_t n,
+                       uint64_t *d_out_xy, uint8_t *d_out_inf, uint8_t *d_status, uint32_t *d_err, void *d_scratch, void *stream) {
+    return msm_dev<OpsFp2>(ctx, dev, d_g2_xy, d_g2_inf, d_scalars, n, d_out_xy, d_out_inf, d_status, d_err, d_scratch, stream);
 }
 
 // ---- Groth16 verification

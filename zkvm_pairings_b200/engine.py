@@ -691,6 +691,43 @@ class PairingEngine:
         """`&G2Affine + &G2Affine` (src/g2.rs:210-242)."""
         return self._add(self._lib.zkp_g2_add_batch, a, b, 24, a_inf, b_inf)
 
+    def _msm(self, fn, pts, width, inf, scalars):
+        pts, inf, n = self._pts(pts, width, inf)
+        k = np.ascontiguousarray(scalars, dtype=np.uint64).reshape(-1, 4)
+        if k.shape[0] != n:
+            raise ValueError("one 4-limb scalar per point expected")
+        out, oinf, st = np.zeros(width, np.uint64), np.zeros(1, np.uint8), np.zeros(1, np.uint8)
+        self._check(fn(self._ctx, _ptr(pts), _ptr(inf), _ptr(k), n, _ptr(out), _ptr(oinf), _ptr(st)))
+        return out, int(oinf[0]), int(st[0])
+
+    def g1_msm(self, points, scalars, inf=None):
+        """sum_i [k_i]P_i over caller-given G1 points (scalars: (n,4) little-endian u64, any 256-bit integer, not reduced
+        mod r; no subgroup check) -> (point (12,) uint64, is_infinity, status: 0 ok, 1 a point off the curve (ZKP_POINT_*))."""
+        return self._msm(self._lib.zkp_g1_msm, points, 12, inf, scalars)
+
+    def g2_msm(self, points, scalars, inf=None):
+        """sum_i [k_i]Q_i over caller-given G2 points -> (point (24,) uint64, is_infinity, status)."""
+        return self._msm(self._lib.zkp_g2_msm, points, 24, inf, scalars)
+
+    def g1_msm_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_g1_msm_scratch_bytes(n))
+
+    def g2_msm_scratch_bytes(self, n: int) -> int:
+        return int(self._lib.zkp_g2_msm_scratch_bytes(n))
+
+    def g1_msm_dev(self, d_points, d_scalars, n: int, d_out, d_out_inf, d_status, d_scratch, d_inf=None, err=None, stream: int = 0,
+                   dev: int = 0):
+        """Asynchronous form on device-resident torch tensors; d_scratch holds g1_msm_scratch_bytes(n) bytes, 16-byte
+        aligned; d_out takes 12 u64, d_out_inf and d_status one byte each."""
+        self._check(self._lib.zkp_g1_msm_dev(self._ctx, dev, _dptr(d_points), _dptr(d_inf), _dptr(d_scalars), n, _dptr(d_out),
+                                             _dptr(d_out_inf), _dptr(d_status), _dptr(err), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
+    def g2_msm_dev(self, d_points, d_scalars, n: int, d_out, d_out_inf, d_status, d_scratch, d_inf=None, err=None, stream: int = 0,
+                   dev: int = 0):
+        """The G2 form of g1_msm_dev (d_out takes 24 u64, d_scratch g2_msm_scratch_bytes(n) bytes)."""
+        self._check(self._lib.zkp_g2_msm_dev(self._ctx, dev, _dptr(d_points), _dptr(d_inf), _dptr(d_scalars), n, _dptr(d_out),
+                                             _dptr(d_out_inf), _dptr(d_status), _dptr(err), _dptr(d_scratch), ctypes.c_void_p(stream)))
+
     def pairing_dev(self, mode: int, out, g1=None, g2=None, g1_inf=None, g2_inf=None, in_fp12=None, n_checks=None,
                     pairs_per_check: int = 1, is_one=None, err=None, stream: int = 0, dev: int = 0):
         """Asynchronous launch on device-resident buffers (torch CUDA tensors).  ``stream`` is a raw
